@@ -4,6 +4,7 @@ throughput of the B200 hot path, with the reference's CPU path timed beside it.
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...  # reference arm (CPU oracle port)
+    python bench.py ... --dump-outputs DIR                   # + the last timed build's outputs as DIR/*.npy
 
 One step = one full index build of the workload text: byte histogram -> K1 suffix
 array -> K2 BWT -> K3 wavelet tree with rank/select directories and C[] -> sampled
@@ -58,7 +59,14 @@ def parse():
     ap.add_argument("--dist-bytes-per-rank", type=int, default=1_000_000_000)
     ap.add_argument("--no-c3", action="store_true", help="skip the C3 / C4 records (200 MB ENG96 text)")
     ap.add_argument("--no-queries", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed build computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------ clocks
@@ -397,6 +405,42 @@ def run_dist_build(args, world, rank, dev, barrier, max_over_ranks, sum_over_ran
     return out
 
 
+# ------------------------------------------------------------------ outputs of the timed build
+DUMP_ROWS = 1 << 19      # rows sampled from each length-n output: a dump stays below 40 MB at any text size
+DUMP_SEED = 7
+
+
+def dump_outputs(out_dir, idx):
+    """Writes what one build (a DeviceIndex) hands its caller to out_dir/<name>.npy, float64 for positions and
+    counts, float32 for symbols and bits, so that two builds of the project can be compared output for output.
+    Outputs of length n are read at one fixed, seeded sample of DUMP_ROWS rows (every row of a smaller text):
+      rows            the sampled rows, ascending
+      sa, bwt         the suffix array and the BWT at those rows
+      sa_via_samples  the suffix array at those rows recovered from the sampled suffix array (LF walks)
+      occ             wavelet-tree rank of bwt[row] before row: the Occ value a backward-search step reads
+      wt_level<l>     the bits of wavelet-tree level l at the sampled rows below that level's length
+      count           C[] as (byte, number of smaller symbols), one row per symbol of the text"""
+    import torch
+    n = idx.n
+    rows_np = (np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS
+               else np.arange(n))
+    rows = torch.from_numpy(rows_np.astype(np.int64)).to(idx.device)
+    bwt = idx.bwt[rows]
+    out = {"rows": rows_np.astype(np.float64),
+           "sa": idx.sa[rows].cpu().numpy().astype(np.float64),
+           "bwt": bwt.cpu().numpy().astype(np.float32),
+           "sa_via_samples": idx.locate_rows(rows.to(torch.int32), use_samples=True).cpu().numpy().astype(np.float64),
+           "occ": idx.wt.rank(bwt, rows).cpu().numpy().astype(np.float64)}
+    for level in range(idx.wt.levels):
+        m = idx.wt.level_len(level)
+        out[f"wt_level{level}"] = idx.wt.bv_bits(level, 0, m)[rows[rows < m]].cpu().numpy().astype(np.float32)
+    out["count"] = np.array([[ord(c), v] for c, v in idx.wt.count_table().items()], dtype=np.float64).reshape(-1, 2)
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------ our arm
 def run_ours(args):
     import torch
@@ -493,6 +537,8 @@ def run_ours(args):
     ms = max_over_ranks(float(np.mean(step_ms)))
     value = world * nbytes / 1e6 / (ms / 1e3)
     stats = idx.stats.sa
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, idx)
 
     # ---- e2e: host text -> H2D -> build -> D2H of the INDEX (wavelet-tree blob + sampled-SA blob: what a build
     #      produces and what save() / a serving process needs), every step.  The full suffix array (4n bytes) is an
