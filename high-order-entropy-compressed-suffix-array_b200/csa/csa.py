@@ -74,7 +74,8 @@ class CompressedSuffixArray:
         self._E = engine
         self.text = text
         self.epsilon = epsilon
-        self._smap = engine.SymbolMap(text, extra="$") if isinstance(text, str) else None
+        self._is_str = isinstance(text, str)
+        self._smap = engine.SymbolMap(text, extra="$") if self._is_str else None
         if self._smap is not None:
             d_text = engine.to_device_u8(self._smap.host_bytes(text), tail=self._smap.encode("$"))
             has_sentinel = "$" in text
@@ -100,6 +101,18 @@ class CompressedSuffixArray:
     @property
     def device_index(self):
         return self._idx
+
+    @property
+    def text(self):
+        """The text the index was built from.  An index opened with load() holds no copy: the first access extracts
+        it from the index."""
+        if self._text is None:
+            self._text = self.extract(0, self.n - 1)
+        return self._text
+
+    @text.setter
+    def text(self, value):
+        self._text = value
 
     def _pack(self, patterns):
         """Patterns -> device CSR; a str pattern with a symbol the text cannot hold becomes a pattern that misses."""
@@ -151,8 +164,63 @@ class CompressedSuffixArray:
         rep["coded_index_bits_per_symbol"] = rep["coded_level_bits_per_symbol"] + rep["sampled_sa_bits_per_symbol"]
         return rep
 
+    def extract(self, start, end):
+        """text[start:end] from the index alone (Python slice semantics on the text without the sentinel): a str for a
+        str text, bytes otherwise.  ValueError when the text held '$' in a way that keeps LF from inverting the suffix
+        order (the index then cannot give the text back)."""
+        return self.extract_batch([(start, end)])[0]
+
+    def extract_batch(self, pairs):
+        """[text[a:b] for (a, b) in pairs], every range extracted by one batched kernel call."""
+        import torch
+        m = self.n - 1
+        bounds = np.array([slice(a, b).indices(m)[:2] for a, b in pairs], dtype=np.int64).reshape(-1, 2)
+        bounds[:, 1] = np.maximum(bounds[:, 1], bounds[:, 0])           # a > b: the empty slice
+        d = torch.from_numpy(bounds).to(self._idx.device)
+        off, data = self._idx.extract_batch(d[:, 0], d[:, 1])
+        off, data = off.cpu().numpy(), self._E.to_host(data).tobytes()
+        if not self._is_str:
+            return [data[off[k]:off[k + 1]] for k in range(len(bounds))]
+        return [self._smap.decode(data[off[k]:off[k + 1]]) for k in range(len(bounds))]
+
     def save(self, path, compressed=True):
-        self._idx.save(path, compressed=compressed)
+        """The index (DeviceIndex.save) plus what load() needs to answer as this object does: n, the sampling rate,
+        epsilon, whether the sentinel was unique, str or bytes, the code points of a re-coded str alphabet and H_k."""
+        back = self._smap.back if self._smap is not None else None
+        meta = {"csa_meta": np.array([self.n, self.sa_sample_rate, int(self.sentinel_unique), int(self._is_str)],
+                                     dtype=np.int64),
+                "csa_epsilon": np.array([np.nan if self.epsilon is None else self.epsilon], dtype=np.float64),
+                "csa_symbols": np.array([ord(c) for c in back] if back else [], dtype=np.int32),
+                "csa_entropy": np.array(sorted(self.entropy.items()), dtype=np.float64).reshape(-1, 2)}
+        self._idx.save(path, compressed=compressed, extra=meta)
+
+    @classmethod
+    def load(cls, path):
+        """A query-only CompressedSuffixArray from a file save() wrote: count, locate, extract, space_report and
+        index_bytes work; ``text`` is extracted from the index on first access."""
+        from hkcsa import engine
+        with np.load(path) as z:
+            if "csa_meta" not in z.files:
+                raise ValueError(f"{path} was not written by CompressedSuffixArray.save")
+            n, rate, unique, is_str = (int(v) for v in z["csa_meta"])
+            epsilon = float(z["csa_epsilon"][0])
+            symbols = [chr(int(c)) for c in z["csa_symbols"]]
+            entropy = {int(k): float(v) for k, v in z["csa_entropy"]}
+        if not unique:
+            raise ValueError("the saved text held the sentinel '$': such an index locates through its full suffix "
+                             "array, which save() does not write")
+        self = cls.__new__(cls)
+        self._E = engine
+        self._text = None
+        self.epsilon = None if epsilon != epsilon else epsilon
+        self._is_str = bool(is_str)
+        self._smap = engine.SymbolMap.from_code_points(symbols) if self._is_str else None
+        self.sa_sample_rate = rate
+        self.sentinel_unique = True
+        self._idx = engine.DeviceIndex.load(path)
+        self.n = n
+        self.entropy = entropy
+        return self
 
     def index_bytes(self):
         """Device bytes held by the index (wavelet tree blob + sampled SA blob [+ the suffix array, kept only when

@@ -1,0 +1,356 @@
+// extract.cu -- K4c: text back out of the compressed index (the third self-index query next to count and locate).
+//
+// No reference counterpart: WaveletTree.decompress returns '' (csa/wavelet_tree.py:158-200).  Two kernels:
+//
+//  * inverse-SA samples: isa[k] = row of the suffix that starts at text position k * rate (k < S = ceil(n / rate)),
+//    isa[S] = isa[0].  Derived from the sampled SA alone -- every marked row j has slot r = rank1(marks, j) and
+//    samples[r] = SA[j] / rate -- so a loaded index (no text, no full SA) has them too.
+//  * batched extract: a request [begin, end) is cut at sample boundaries into segments
+//    [k * rate, (k + 1) * rate) & [begin, end); each segment is one independent walk that starts at row isa[k + 1]
+//    (the suffix just past the segment: its BWT symbol is the segment's last symbol) and emits text[p - 1],
+//    text[p - 2], ... by LF steps.  Whole-text extraction is n / rate walks of <= rate steps: a parallel BWT
+//    inversion.  Adjacent threads own adjacent segments, so the byte stores of a long range land close together.
+//    The LF step is the wavelet tree's access + rank descent, or the sampled Occ table's (layouts 0 and 1).
+#include "common.cuh"
+#include "prof.cuh"
+#include "wavelet.cuh"
+
+namespace hkcsa {
+
+constexpr int EXT_THREADS = 256;
+constexpr int SCAN_THREADS = 1024;
+
+// ---------------------------------------------------------------- inverse-SA samples
+// one thread per mark rank block: the marked rows of the block in order, their slots from the block's rank header
+__global__ void __launch_bounds__(256)
+isa_samples_kernel(BitVec marks, const uint32_t *__restrict__ samples, uint64_t n, uint64_t S, uint32_t *__restrict__ isa)
+{
+    const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g * HKCSA_BLOCK_BITS >= n) return;
+    const RankBlock b = load_block(marks.blocks + g);
+    uint64_t r = marks.super[g / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu);
+    const uint64_t row0 = g * HKCSA_BLOCK_BITS;
+#pragma unroll
+    for (int w = 0; w < 4; ++w) {
+        // payload bit o of the block is bit o + 32 of the 256: word 0 holds payload bits 0-31 in its high half
+        uint64_t m = (w == 0) ? (b.w[0] >> 32) : b.w[w];
+        const uint64_t base = row0 + (w == 0 ? 0u : 32u + 64u * (w - 1));
+        while (m) {
+            const uint64_t j = base + (uint64_t)(__ffsll((long long)m) - 1);
+            m &= m - 1;
+            if (j >= n) break;
+            const uint32_t s = samples[r++];
+            isa[s] = (uint32_t)j;
+            if (s == 0) isa[S] = (uint32_t)j;     // the walk of the text's last stretch starts at the row of suffix 0
+        }
+    }
+}
+
+// ---------------------------------------------------------------- segments of the requests
+// A request clamped to 0 <= b <= e <= n and to its own output slice: whatever the caller passes, the kernel never
+// writes outside out[out_off[q] .. out_off[q + 1]).
+struct ExtRange {
+    uint64_t b, e;
+};
+__device__ __forceinline__ ExtRange clamp_request(const int64_t *__restrict__ begin, const int64_t *__restrict__ end,
+                                               const int64_t *__restrict__ out_off, uint64_t q, uint64_t n)
+{
+    const int64_t room = max(out_off[q + 1] - out_off[q], (int64_t)0);
+    const int64_t b = min(max(begin[q], (int64_t)0), (int64_t)n);
+    const int64_t e = min(min(max(end[q], b), (int64_t)n), b + room);
+    return ExtRange{(uint64_t)b, (uint64_t)e};
+}
+__device__ __forceinline__ uint64_t segments_of(const ExtRange &r, uint32_t rate)
+{
+    return r.e > r.b ? (r.e - 1) / rate - r.b / rate + 1 : 0;
+}
+
+// seg_off[q] = segments of the requests before q; three passes (block sums, scan of the block sums, block scans)
+__device__ __forceinline__ uint64_t block_excl_sum(uint64_t v, uint64_t &total)
+{
+    __shared__ uint64_t s_warp[SCAN_THREADS / 32];
+    const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
+    uint64_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= (uint32_t)o) x += y;
+    }
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+        uint64_t w = (lane < blockDim.x / 32) ? s_warp[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint64_t y = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= (uint32_t)o) w += y;
+        }
+        s_warp[lane] = w;                          // inclusive prefix over the warps
+    }
+    __syncthreads();
+    total = s_warp[blockDim.x / 32 - 1];
+    const uint64_t ex = x - v + (warp ? s_warp[warp - 1] : 0);
+    __syncthreads();                               // s_warp is reused by the next call
+    return ex;
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+seg_block_sum_kernel(const int64_t *__restrict__ begin, const int64_t *__restrict__ end,
+                     const int64_t *__restrict__ out_off, uint64_t R, uint64_t n, uint32_t rate, uint64_t *__restrict__ bsum)
+{
+    const uint64_t q = (uint64_t)blockIdx.x * SCAN_THREADS + threadIdx.x;
+    const uint64_t v = q < R ? segments_of(clamp_request(begin, end, out_off, q, n), rate) : 0;
+    uint64_t total;
+    block_excl_sum(v, total);
+    if (threadIdx.x == 0) bsum[blockIdx.x] = total;
+}
+
+// one CTA: exclusive prefix of the block sums in place
+__global__ void __launch_bounds__(SCAN_THREADS) seg_scan_sums_kernel(uint64_t *__restrict__ bsum, uint64_t nb)
+{
+    uint64_t carry = 0;
+    for (uint64_t i0 = 0; i0 < nb; i0 += SCAN_THREADS) {
+        const uint64_t i = i0 + threadIdx.x;
+        const uint64_t v = i < nb ? bsum[i] : 0;
+        uint64_t total;
+        const uint64_t ex = block_excl_sum(v, total);
+        if (i < nb) bsum[i] = carry + ex;
+        carry += total;
+    }
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+seg_offsets_kernel(const int64_t *__restrict__ begin, const int64_t *__restrict__ end,
+                   const int64_t *__restrict__ out_off, uint64_t R, uint64_t n, uint32_t rate,
+                   const uint64_t *__restrict__ bsum, uint64_t *__restrict__ seg_off)
+{
+    const uint64_t q = (uint64_t)blockIdx.x * SCAN_THREADS + threadIdx.x;
+    const uint64_t v = q < R ? segments_of(clamp_request(begin, end, out_off, q, n), rate) : 0;
+    uint64_t total;
+    const uint64_t ex = block_excl_sum(v, total) + bsum[blockIdx.x];
+    if (q < R) seg_off[q] = ex;
+    if (q == R - 1) seg_off[R] = ex + v;
+}
+
+// ---------------------------------------------------------------- LF steps
+// The sampled Occ table (occ_table.cu): layout 0 rows of [2^SHIFT BWT bytes][sigma x u32 counts], or (SHIFT == 0)
+// layout 1 per-symbol entries {count, bitmap of 32 rows} followed by a copy of the BWT.
+struct ExtOccView {
+    const uint8_t *rows;
+    uint64_t stride;
+    const uint8_t *bwt;
+};
+// LF(j) from the Occ table; sym = bwt[j].  The same step as locate_rows_occ_kernel's, kept apart from it so that the
+// locate kernels' code does not change with this file.
+template <int SHIFT>
+__device__ __forceinline__ uint32_t occ_lf(const ExtOccView &o, const uint32_t *s_C, const uint16_t *s_code, uint32_t j,
+                                          uint32_t &sym)
+{
+    if constexpr (SHIFT == 0) {
+        const uint32_t ch = __ldg(o.bwt + j);
+        const uint32_t code = s_code[ch];
+        const uint2 e = __ldg(reinterpret_cast<const uint2 *>(o.rows) + (uint64_t)code * o.stride + (j >> 5));
+        sym = ch;
+        return s_C[code] + e.x + __popc(e.y & ((1u << (j & 31u)) - 1u));
+    } else {
+        constexpr uint32_t B = 1u << SHIFT;
+        const uint8_t *row = o.rows + (uint64_t)(j >> SHIFT) * o.stride;
+        const uint32_t t = j & (B - 1);
+        uint64_t x[B / 8];
+#pragma unroll
+        for (int v = 0; v < (int)B / 32; ++v) ld_nc_256(row + 32 * v, x[4 * v], x[4 * v + 1], x[4 * v + 2], x[4 * v + 3]);
+        const uint32_t ch = __ldg(row + t);         // same sector as the loads above
+        const uint32_t code = s_code[ch];
+        const uint32_t base = __ldg(reinterpret_cast<const uint32_t *>(row + B) + code);
+        const uint32_t ch4 = ch * 0x01010101u;
+        uint64_t bits = 0;
+#pragma unroll
+        for (int v = 0; v < (int)B / 8; ++v) {       // bit i = (byte i of the row == ch)
+            const uint32_t lo = __vcmpeq4((uint32_t)x[v], ch4) & 0x01010101u;
+            const uint32_t hi = __vcmpeq4((uint32_t)(x[v] >> 32), ch4) & 0x01010101u;
+            bits |= (uint64_t)(((lo * 0x01020408u) >> 24) | (((hi * 0x01020408u) >> 24) << 4)) << (8 * v);
+        }
+        sym = ch;
+        return s_C[code] + base + __popcll(bits & ((1ull << t) - 1ull));
+    }
+}
+
+// ---------------------------------------------------------------- extract
+// Segment t of the batch: request q = the last with seg_off[q] <= t (binary search; a warp's lanes mostly share q
+// and read the same offsets), k = its (t - seg_off[q])-th sample block.
+__device__ __forceinline__ uint64_t request_of(const uint64_t *__restrict__ seg_off, uint64_t R, uint64_t t)
+{
+    uint64_t lo = 0, hi = R;                       // seg_off[lo] <= t < seg_off[hi]
+    while (hi - lo > 1) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if (seg_off[mid] <= t) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+struct ExtractArgs {
+    const uint32_t *isa;
+    uint32_t rate;
+    uint64_t n;
+    const int64_t *begin, *end, *out_off;
+    uint64_t R;
+    const uint64_t *seg_off;
+    uint8_t *out;
+};
+
+// the walks of every segment, grid-strided; lf(j, sym) returns LF(j) and sets sym = bwt[j]
+template <typename LF>
+__device__ __forceinline__ void extract_walks(const ExtractArgs &a, LF lf)
+{
+    const uint64_t total = a.seg_off[a.R];
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += stride) {
+        const uint64_t q = request_of(a.seg_off, a.R, t);
+        const ExtRange r = clamp_request(a.begin, a.end, a.out_off, q, a.n);
+        const uint64_t k = r.b / a.rate + (t - a.seg_off[q]);
+        const uint64_t lo = max(r.b, k * a.rate);
+        const uint64_t hi = min(r.e, (k + 1) * a.rate);
+        uint64_t p = min((k + 1) * a.rate, a.n);   // the walk starts at the row of the suffix that begins at p
+        uint32_t j = __ldg(a.isa + k + 1);
+        uint8_t *dst = a.out + a.out_off[q];
+        while (p > lo) {
+            uint32_t sym;
+            j = lf(j, sym);
+            --p;                                   // sym = text[p]
+            if (p < hi) dst[p - r.b] = (uint8_t)sym;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(EXT_THREADS) extract_wt_kernel(WtDev wt, ExtractArgs a)
+{
+    __shared__ WtSmem s;
+    wt_smem_load(s, wt);
+    __syncthreads();
+    extract_walks(a, [&](uint32_t j, uint32_t &sym) {
+        uint32_t occ;
+        const uint32_t code = wt_access_rank(s, wt, j, occ);    // symbol and rank from one descent
+        sym = s.sym_of_code[code];
+        return s.C[code] + occ;
+    });
+}
+
+template <int SHIFT>
+__global__ void __launch_bounds__(EXT_THREADS) extract_occ_kernel(const WtTables *__restrict__ tab, ExtOccView occ, ExtractArgs a)
+{
+    __shared__ uint32_t s_C[260];
+    __shared__ uint16_t s_code[256];
+    for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s_C[i] = tab->C[i];
+    for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s_code[i] = tab->code_of_sym[i];
+    __syncthreads();
+    extract_walks(a, [&](uint32_t j, uint32_t &sym) { return occ_lf<SHIFT>(occ, s_C, s_code, j, sym); });
+}
+
+// the number of walks is known on the device only: a grid of exactly the resident CTAs strides over them
+template <typename K>
+int resident_grid(K kernel)
+{
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, EXT_THREADS, 0) != cudaSuccess || per_sm < 1)
+        per_sm = 1;
+    return per_sm * num_sms();
+}
+
+}  // namespace hkcsa
+
+using namespace hkcsa;
+
+static int ssa_plan_check(const hkcsa_ssa_plan *p)
+{
+    HK_REQUIRE(p->rate >= 1, HKCSA_EINVAL, "sampling rate must be >= 1");
+    HK_REQUIRE(p->n <= HKCSA_MAX_N, HKCSA_ERANGE, "n exceeds HKCSA_MAX_N");
+    HK_REQUIRE(p->n_samples == (p->n + p->rate - 1) / p->rate, HKCSA_EINVAL,
+               "inverse-SA samples need the sampled SA of a whole text (a slice plan samples a part of it)");
+    return HKCSA_OK;
+}
+
+extern "C" int hkcsa_isa_samples(const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa, uint32_t *d_isa, void *stream)
+{
+    HK_REQUIRE(d_ssa_blob && h_ssa && d_isa, HKCSA_EINVAL, "null pointer");
+    const int rc = ssa_plan_check(h_ssa);
+    if (rc != HKCSA_OK) return rc;
+    const uint64_t n = h_ssa->n, S = h_ssa->n_samples;
+    if (n == 0) return HKCSA_OK;
+    cudaStream_t st = as_stream(stream);
+    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
+    BitVec marks;
+    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
+    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
+    marks.len = n;
+    const uint64_t nblocks = (n + HKCSA_BLOCK_BITS - 1) / HKCSA_BLOCK_BITS;
+    // mark blocks and samples read once, S + 1 entries scattered
+    prof::Scope ps(st, prof::SSA_BUILD, nblocks * sizeof(RankBlock) + S * 4 + (S + 1) * 4);
+    isa_samples_kernel<<<(uint32_t)((nblocks + 255) / 256), 256, 0, st>>>(
+        marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), n, S, d_isa);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
+}
+
+static size_t extract_scratch(uint64_t R, uint64_t **seg_off, uint64_t **bsum, void *base)
+{
+    Carver c(base);
+    *seg_off = c.take<uint64_t>(R + 1);
+    *bsum = c.take<uint64_t>((R + SCAN_THREADS - 1) / SCAN_THREADS + 1);
+    return c.total();
+}
+
+extern "C" size_t hkcsa_extract_scratch_bytes(uint64_t R)
+{
+    uint64_t *a, *b;
+    return extract_scratch(R, &a, &b, nullptr);
+}
+
+extern "C" int hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan, const void *d_occ_blob,
+                             const hkcsa_occ_plan *h_occ_plan, const uint32_t *d_isa, uint32_t rate,
+                             const int64_t *d_begin, const int64_t *d_end, const int64_t *d_out_off, uint64_t R,
+                             uint8_t *d_out, void *d_scratch, size_t scratch_bytes, void *stream)
+{
+    HK_REQUIRE(d_wt_blob && h_wt_plan && d_isa, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE((d_occ_blob == nullptr) == (h_occ_plan == nullptr), HKCSA_EINVAL, "occ blob and plan go together");
+    HK_REQUIRE(rate >= 1, HKCSA_EINVAL, "sampling rate must be >= 1");
+    const uint64_t n = h_wt_plan->n;
+    HK_REQUIRE(n >= 1 && n <= HKCSA_MAX_N, HKCSA_EINVAL, "empty index or n beyond HKCSA_MAX_N");
+    if (h_occ_plan) {
+        HK_REQUIRE(h_occ_plan->n == n && h_occ_plan->sigma == h_wt_plan->sigma, HKCSA_EINVAL,
+                   "occ plan does not match the index");
+        HK_REQUIRE(h_occ_plan->layout == 1 ? h_occ_plan->shift == 5 : (h_occ_plan->shift == 5 || h_occ_plan->shift == 6),
+                   HKCSA_EINVAL, "unknown occ table layout");
+    }
+    if (R == 0) return HKCSA_OK;
+    HK_REQUIRE(d_begin && d_end && d_out_off && d_out && d_scratch, HKCSA_EINVAL, "null pointer");
+    uint64_t *seg_off, *bsum;
+    HK_REQUIRE(extract_scratch(R, &seg_off, &bsum, d_scratch) <= scratch_bytes, HKCSA_ESCRATCH, "extract scratch too small");
+    cudaStream_t st = as_stream(stream);
+
+    const uint32_t nb = (uint32_t)((R + SCAN_THREADS - 1) / SCAN_THREADS);
+    seg_block_sum_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum);
+    HK_LAUNCH_CHECK();
+    seg_scan_sums_kernel<<<1, SCAN_THREADS, 0, st>>>(bsum, nb);
+    HK_LAUNCH_CHECK();
+    seg_offsets_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum, seg_off);
+    HK_LAUNCH_CHECK();
+
+    ExtractArgs a{d_isa, rate, n, d_begin, d_end, d_out_off, R, seg_off, d_out};
+    prof::Scope ps(st, prof::LOCATE, 0);
+    if (!h_occ_plan) {
+        extract_wt_kernel<<<resident_grid(extract_wt_kernel), EXT_THREADS, 0, st>>>(make_wt_dev(d_wt_blob, h_wt_plan), a);
+    } else {
+        const WtTables *tab = reinterpret_cast<const WtTables *>(static_cast<const uint8_t *>(d_wt_blob) + h_wt_plan->off_tables);
+        const ExtOccView occ{static_cast<const uint8_t *>(d_occ_blob), h_occ_plan->stride,
+                          static_cast<const uint8_t *>(d_occ_blob) + h_occ_plan->off_bwt};
+        if (h_occ_plan->layout == 1)
+            extract_occ_kernel<0><<<resident_grid(extract_occ_kernel<0>), EXT_THREADS, 0, st>>>(tab, occ, a);
+        else if (h_occ_plan->shift == 5)
+            extract_occ_kernel<5><<<resident_grid(extract_occ_kernel<5>), EXT_THREADS, 0, st>>>(tab, occ, a);
+        else
+            extract_occ_kernel<6><<<resident_grid(extract_occ_kernel<6>), EXT_THREADS, 0, st>>>(tab, occ, a);
+    }
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
+}

@@ -201,6 +201,10 @@ SIGNATURES = {
     "hkcsa_ranges_unpack": (_i32, [_vp, _u64, _vp, _vp, _vp]),
     "hkcsa_locate_rows_occ": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(OccPlan), _vp, C.POINTER(SsaPlan), _vp,
                                      _u64, _vp, _vp]),
+    "hkcsa_isa_samples": (_i32, [_vp, C.POINTER(SsaPlan), _vp, _vp]),
+    "hkcsa_extract_scratch_bytes": (_sz, [_u64]),
+    "hkcsa_extract": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(OccPlan), _vp, _u32, _vp, _vp, _vp, _u64, _vp,
+                             _vp, _sz, _vp]),
     "hkcsa_kmer_k": (_u32, [_u32]),
     "hkcsa_kmer_entries": (_u64, [_u32, _u32]),
     "hkcsa_kmer_scratch_bytes": (_sz, [_u32, _u32]),

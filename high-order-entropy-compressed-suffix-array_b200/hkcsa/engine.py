@@ -80,6 +80,16 @@ class SymbolMap:
             self.back = cps
             self._fwd = {ord(c): i for i, c in enumerate(cps)}
 
+    @classmethod
+    def from_code_points(cls, back) -> "SymbolMap":
+        """The map whose byte i is back[i] (an empty list: the identity map) -- what a saved index records."""
+        self = cls.__new__(cls)
+        self._cache = None
+        self.back = list(back) or None
+        if self.back is not None:
+            self._fwd = {ord(c): i for i, c in enumerate(self.back)}
+        return self
+
     @property
     def identity(self) -> bool:
         return self.back is None
@@ -710,11 +720,12 @@ class DeviceIndex:
                 "levels_kept_plain": [l for l, (v, r) in enumerate(zip(coded, raw)) if v.coded_bits >= r],
                 "sampled_sa_bits_per_symbol": ssa_bits / n}
 
-    def save(self, path: str, compressed: bool = False) -> None:
+    def save(self, path: str, compressed: bool = False, extra: dict | None = None) -> None:
         """Write the query structures to one .npz file.  compressed=False: the wavelet-tree blob exactly as it lives
         in HBM (loading is a single host->device copy).  compressed=True: every level in the class/offset code
         (n*H_0 of the level + o(n) bits; over the levels of a BWT: n*H_k + o(n)); load() decodes the payload bits
-        in place and rebuilds the rank directories -- the restored blob is bit-identical."""
+        in place and rebuilds the rank directories -- the restored blob is bit-identical.  extra: more named arrays
+        for the same file (a caller's metadata); load() reads its own keys by name and ignores them."""
         parts = {"n": np.array([self.n], dtype=np.int64),
                  "wt_plan": np.frombuffer(bytes(self.wt.plan), dtype=np.uint8)}
         if compressed:
@@ -731,6 +742,10 @@ class DeviceIndex:
         if self.ssa is not None:
             parts["ssa_plan"] = np.frombuffer(bytes(self.ssa.plan), dtype=np.uint8)
             parts["ssa_blob"] = to_host(self.ssa.blob)
+        for key, arr in (extra or {}).items():
+            if key in parts:
+                raise ValueError(f"extra key {key!r} collides with an index array")
+            parts[key] = np.asarray(arr)
         with open(path, "wb") as f:
             np.savez(f, **parts)
 
@@ -895,6 +910,76 @@ class DeviceIndex:
         else:
             check(L.hkcsa_gather_u32(_ptr(self.sa), _ptr(rows), rows.numel(), _ptr(out), _stream()))
         return out
+
+    # extract (csrc/extract.cu): text[begin:end) from the index alone -- the reference's decompress returns ''
+    def isa_samples(self) -> torch.Tensor:
+        """int32[S + 1]: the row of the suffix at text position k * rate for k < S = ceil(n / rate), and [S] = [0].
+        Derived from the sampled suffix array (no text, no full SA: a loaded index has it too); built on first use."""
+        if getattr(self, "_isa", None) is None:
+            if self.ssa is None:
+                raise ValueError("index was built without a sampled suffix array")
+            out = _empty(int(self.ssa.plan.n_samples) + 1, torch.int32, self.device)
+            check(_lib.load().hkcsa_isa_samples(_ptr(self.ssa.blob), C.byref(self.ssa.plan), _ptr(out), _stream()))
+            self._isa = out
+        return self._isa
+
+    @property
+    def invertible(self) -> bool:
+        """Whether LF is the inverse of the suffix order on this index, i.e. whether extract gives back the text.  With
+        j0 = the row of suffix 0 and c = bwt[j0] (= text[n-1]), LF is right everywhere iff j0 is the first row whose BWT
+        symbol is c.  Always true with a unique sentinel; a text that holds the sentinel elsewhere may fail it."""
+        if getattr(self, "_invertible", None) is None:
+            if self.n == 0:
+                self._invertible = False
+            else:
+                j0 = self.isa_samples()[:1].to(torch.int64)
+                c = self.wt.access(j0)
+                self._invertible = int(self.wt.rank(c, j0).item()) == 0
+        return self._invertible
+
+    def extract_batch(self, begin: torch.Tensor, end: torch.Tensor, *, use_occ_table: bool | None = None):
+        """text[begin[q]:end[q]) for every q (int64 device tensors; 0 <= begin <= end <= n, sentinel included) ->
+        (out_off int64[R+1], bytes uint8[total]) on the device, request q at bytes[out_off[q]:out_off[q+1]].
+        use_occ_table: None = LF steps on the sampled Occ table when one was built (as locate_rows), else the tree."""
+        L = _lib.load()
+        begin = begin.to(device=self.device, dtype=torch.int64).contiguous()
+        end = end.to(device=self.device, dtype=torch.int64).contiguous()
+        if begin.shape != end.shape or begin.dim() != 1:
+            raise ValueError("begin and end must be 1-d tensors of the same length")
+        if not self.invertible:
+            raise ValueError("LF does not invert the suffix order on this index (its text holds the sentinel "
+                             "elsewhere too): extract cannot give the text back")
+        R = begin.numel()
+        out_off = torch.zeros(R + 1, dtype=torch.int64, device=self.device)
+        if R == 0:
+            return out_off, _empty(0, torch.uint8, self.device)
+        out_off[1:] = torch.cumsum(end - begin, 0)                          # plumbing: CSR offsets
+        bad = ((begin < 0) | (end < begin) | (end > self.n)).any()
+        total, bad = torch.stack([out_off[-1], bad.to(torch.int64)]).tolist()   # one read-back for both
+        if bad:
+            raise ValueError(f"extract ranges must satisfy 0 <= begin <= end <= n = {self.n}")
+        out = _empty(total, torch.uint8, self.device)
+        if total == 0:
+            return out_off, out
+        occ = getattr(self, "_occ", None)
+        if use_occ_table is None:
+            use_occ_table = occ is not None
+        if use_occ_table and occ is None:
+            raise ValueError("no sampled Occ table: call build_occ_table() first")
+        plan, blob = occ if use_occ_table else (None, None)
+        isa = self.isa_samples()
+        nbytes = L.hkcsa_extract_scratch_bytes(R)
+        scratch = _scratch(nbytes, self.device)
+        check(L.hkcsa_extract(_ptr(self.wt.blob), C.byref(self.wt.plan), _ptr(blob),
+                              C.byref(plan) if plan is not None else None, _ptr(isa), int(self.ssa.plan.rate),
+                              _ptr(begin), _ptr(end), _ptr(out_off), R, _ptr(out), _ptr(scratch), nbytes, _stream()))
+        return out_off, out
+
+    def extract(self, begin: int, end: int, *, use_occ_table: bool | None = None) -> torch.Tensor:
+        """text[begin:end) of the indexed text (sentinel included) as a uint8 device tensor."""
+        b = torch.tensor([begin], dtype=torch.int64, device=self.device)
+        e = torch.tensor([end], dtype=torch.int64, device=self.device)
+        return self.extract_batch(b, e, use_occ_table=use_occ_table)[1]
 
 
 # ------------------------------------------------------------------ measurement hook

@@ -547,6 +547,32 @@ int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan,
                           const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos, void *stream);
 
 /* ------------------------------------------------------------------------ */
+/* K4c extract: text[begin:end) back out of the index, without the text (no  */
+/* reference counterpart: WaveletTree.decompress returns '',                  */
+/* csa/wavelet_tree.py:158-200).                                              */
+/* hkcsa_isa_samples: isa[k] = row of the suffix at text position k * rate    */
+/* for k < S = h_ssa->n_samples, and isa[S] = isa[0]; derived from the        */
+/* sampled SA alone (works on a loaded index).  A slice plan                  */
+/* (hkcsa_ssa_plan_make_slice) is refused.  d_isa: uint32[S + 1].             */
+/* hkcsa_extract: R requests [d_begin[q], d_end[q]) over the indexed text     */
+/* (sentinel included), 0 <= begin <= end <= n; the bytes of request q go to  */
+/* d_out[d_out_off[q] .. d_out_off[q+1]) (the caller's exclusive prefix sum   */
+/* of end - begin).  Ranges are clamped on the device, so a bad one never     */
+/* writes outside its own slice.  Each request runs as one LF walk per        */
+/* sample block it touches, <= rate steps each.  d_occ_blob / h_occ_plan both */
+/* NULL: LF on the wavelet tree; otherwise on the sampled Occ table (layout 0 */
+/* or 1).  LF inverts the suffix order only when the text's sentinel is       */
+/* unique (more precisely: when occ(bwt[isa[0]], isa[0]) == 0); on any other  */
+/* index the bytes are not the text.                                          */
+/* ------------------------------------------------------------------------ */
+int    hkcsa_isa_samples(const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa, uint32_t *d_isa, void *stream);
+size_t hkcsa_extract_scratch_bytes(uint64_t R);
+int    hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan, const void *d_occ_blob,
+                     const hkcsa_occ_plan *h_occ_plan, const uint32_t *d_isa, uint32_t rate, const int64_t *d_begin,
+                     const int64_t *d_end, const int64_t *d_out_off, uint64_t R, uint8_t *d_out, void *d_scratch,
+                     size_t scratch_bytes, void *stream);
+
+/* ------------------------------------------------------------------------ */
 /* Host text in, index out: the reference's constructor takes a Python str   */
 /* (EnhancedFMIndex.__init__, csa/enhanced_fm_index.py:8-9; the corpus loader */
 /* returns one, utils/data_loader.py:4) whose bytes sit in PAGEABLE memory.   */
