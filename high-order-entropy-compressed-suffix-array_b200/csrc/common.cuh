@@ -195,6 +195,17 @@ __device__ __forceinline__ uint32_t block_bit(const RankBlock &b, uint32_t o)
     const uint32_t t = o + 32u;
     return (uint32_t)(b.w[t >> 6] >> (t & 63u)) & 1u;
 }
+// The exact LF step of locate: LF(j) = C[code] + lf_fix(occ(code, j), ...).  Row row0 holds suffix 0, whose BWT
+// symbol c0 = text[n-1] stands for the one-symbol suffix n-1: the first of the c0-suffixes.  When c0 also occurs
+// before row0 (a text that holds its last symbol elsewhere, e.g. a second '$'), occ alone ranks row0 after those
+// rows: the true step is C[c0] at row0 and one more than occ on every c0-row before it.  fix = occ(c0, row0) != 0;
+// with a unique sentinel it is 0 and the step is the plain one.
+__device__ __forceinline__ uint32_t lf_fix(uint32_t occ, uint32_t code, uint32_t j, uint32_t c0, uint32_t row0,
+                                           uint32_t fix)
+{
+    if (!fix || code != c0 || j > row0) return occ;
+    return j == row0 ? 0u : occ + 1u;
+}
 // one 256-bit read-only load (sm_100: LDG.E.256) of a 32-byte-aligned sector
 __device__ __forceinline__ void ld_nc_256(const void *p, uint64_t &w0, uint64_t &w1, uint64_t &w2, uint64_t &w3)
 {

@@ -200,11 +200,18 @@ __global__ void gather_u32_kernel(const uint32_t *__restrict__ src, const uint32
 // position of row j: walk LF until a marked row, pos = sample * rate + steps.
 // LF(j) = C[c] + occ(c, j) with c = bwt[j], both from one wavelet descent.
 __global__ void __launch_bounds__(256)
-locate_rows_kernel(WtDev wt, BitVec marks, const uint32_t *__restrict__ samples, uint32_t rate,
+locate_rows_kernel(WtDev wt, BitVec marks, const uint32_t *__restrict__ samples, uint32_t rate, uint32_t row0,
                    const uint32_t *__restrict__ rows, uint64_t m, uint32_t *__restrict__ out)
 {
     __shared__ WtSmem s;
+    __shared__ uint32_t s_c0, s_fix;
     wt_smem_load(s, wt);
+    __syncthreads();
+    if (threadIdx.x == 0) {             // c0 = bwt[row0] = text[n-1]; LF needs fixing iff c0 occurs before row0
+        uint32_t occ0;
+        s_c0 = wt_access_rank(s, wt, row0, occ0);
+        s_fix = occ0 != 0;
+    }
     __syncthreads();
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= m) return;
@@ -219,12 +226,12 @@ locate_rows_kernel(WtDev wt, BitVec marks, const uint32_t *__restrict__ samples,
             out[q] = samples[r] * rate + steps;
             return;
         }
-        // a sampled row is at most rate-1 LF steps away when the sentinel is unique; on a text that already holds
-        // the sentinel LF is a permutation whose cycles may miss every mark: stop, report HKCSA_NO_POSITION
+        // with the exact LF step below a walk meets a marked row within rate-1 steps on every text; the bound only
+        // keeps a walk over a corrupt index from spinning
         if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }
         uint32_t occ;
         const uint32_t code = wt_access_rank(s, wt, j, occ);
-        j = s.C[code] + occ;
+        j = s.C[code] + lf_fix(occ, code, j, s_c0, row0, s_fix);
         ++steps;
     }
 }
@@ -466,11 +473,13 @@ extern "C" int hkcsa_gather_u32(const uint32_t *d_src, const uint32_t *d_rows, u
 }
 
 extern "C" int hkcsa_locate_rows(const void *d_wt_blob, const hkcsa_wt_plan *h_plan, const void *d_ssa_blob,
-                                 const hkcsa_ssa_plan *h_ssa, const uint32_t *d_rows, uint64_t m,
+                                 const hkcsa_ssa_plan *h_ssa, uint32_t row0, const uint32_t *d_rows, uint64_t m,
                                  uint32_t *d_out_pos, void *stream)
 {
     if (m == 0) return HKCSA_OK;
     HK_REQUIRE(d_wt_blob && h_plan && d_ssa_blob && h_ssa && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(h_ssa->n == h_plan->n, HKCSA_EINVAL, "plans do not match");
+    HK_REQUIRE(row0 < h_plan->n, HKCSA_EINVAL, "row0 (the row of suffix 0) out of range");
     cudaStream_t st = as_stream(stream);
     WtDev wt = make_wt_dev(d_wt_blob, h_plan);
     const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
@@ -480,7 +489,8 @@ extern "C" int hkcsa_locate_rows(const void *d_wt_blob, const hkcsa_wt_plan *h_p
     marks.len = h_ssa->n;
     prof::Scope ps(st, prof::LOCATE, 0);
     locate_rows_kernel<<<(uint32_t)((m + 255) / 256), 256, 0, st>>>(
-        wt, marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), h_ssa->rate, d_rows, m, d_out_pos);
+        wt, marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), h_ssa->rate, row0, d_rows, m,
+        d_out_pos);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }

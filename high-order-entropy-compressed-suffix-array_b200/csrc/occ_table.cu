@@ -290,18 +290,44 @@ fm_count_occ_kernel(OccDev occ, const WtTables *__restrict__ tab, const uint8_t 
     }
 }
 
+// occ(bwt[j], j) from the Occ table, and the symbol's code
+template <int SHIFT>
+__device__ __forceinline__ uint32_t occ_step(const OccDev &occ, const uint16_t *s_code, uint32_t j, uint32_t &code)
+{
+    constexpr uint32_t B = 1u << SHIFT;
+    if (SHIFT == 0) {
+        const uint32_t ch = __ldg(occ.bwt + j);
+        code = s_code[ch];
+        const uint2 e = __ldg(reinterpret_cast<const uint2 *>(occ.rows) + (uint64_t)code * occ.stride + (j >> 5));
+        return e.x + __popc(e.y & ((1u << (j & 31u)) - 1u));
+    } else {
+        const uint32_t t = j & (B - 1);
+        const uint8_t *row = occ_sym_ptr(occ, j >> SHIFT);
+        const uint32_t ch = __ldg(row + t);
+        code = s_code[ch];
+        return __ldg(occ_cnt_ptr(row, code, B)) + occ_count<(SHIFT ? SHIFT : 5)>(row, ch * 0x01010101u, t);
+    }
+}
+
 // position of row j: LF walk until a marked row (locate_rows_kernel of fm_search.cu with the LF step read from
 // the Occ table: the symbol bwt[j] and its count before j come from the same row -- two sectors per step)
 template <int SHIFT>
 __global__ void __launch_bounds__(256)
 locate_rows_occ_kernel(OccDev occ, const WtTables *__restrict__ tab, BitVec marks, const uint32_t *__restrict__ samples,
-                       uint32_t rate, const uint32_t *__restrict__ rows, uint64_t m, uint32_t *__restrict__ out)
+                       uint32_t rate, uint32_t row0, const uint32_t *__restrict__ rows, uint64_t m,
+                       uint32_t *__restrict__ out)
 {
-    constexpr uint32_t B = 1u << SHIFT;
     __shared__ uint32_t s_C[260];
     __shared__ uint16_t s_code[256];
+    __shared__ uint32_t s_c0, s_fix;
     for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s_C[i] = tab->C[i];
     for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s_code[i] = tab->code_of_sym[i];
+    __syncthreads();
+    if (threadIdx.x == 0) {             // c0 = bwt[row0]; the LF step needs lf_fix iff c0 occurs before row0
+        uint32_t c0;
+        s_fix = occ_step<SHIFT>(occ, s_code, row0, c0) != 0;
+        s_c0 = c0;
+    }
     __syncthreads();
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= m) return;
@@ -316,20 +342,10 @@ locate_rows_occ_kernel(OccDev occ, const WtTables *__restrict__ tab, BitVec mark
             out[q] = samples[r] * rate + steps;
             return;
         }
-        if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }   // sentinel not unique: see locate_rows_kernel
-        const uint32_t t = j & (B - 1);
-        if (SHIFT == 0) {
-            const uint32_t ch = __ldg(occ.bwt + j);
-            const uint32_t code = s_code[ch];
-            const uint2 e = __ldg(reinterpret_cast<const uint2 *>(occ.rows) + (uint64_t)code * occ.stride + (j >> 5));
-            j = s_C[code] + e.x + __popc(e.y & ((1u << (j & 31u)) - 1u));
-        } else {
-            const uint8_t *row = occ_sym_ptr(occ, j >> SHIFT);
-            const uint32_t ch = __ldg(row + t);
-            const uint32_t code = s_code[ch];
-            const uint32_t base = __ldg(occ_cnt_ptr(row, code, B));
-            j = s_C[code] + base + occ_count<(SHIFT ? SHIFT : 5)>(row, ch * 0x01010101u, t);
-        }
+        if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }   // corrupt index only: see locate_rows_kernel
+        uint32_t code;
+        const uint32_t cnt = occ_step<SHIFT>(occ, s_code, j, code);
+        j = s_C[code] + lf_fix(cnt, code, j, s_c0, row0, s_fix);
         ++steps;
     }
 }
@@ -487,11 +503,13 @@ extern "C" int hkcsa_count_batch_peers(const void *d_wt_blob, const hkcsa_wt_pla
 
 extern "C" int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
                                      const hkcsa_occ_plan *p, const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa,
-                                     const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos, void *stream)
+                                     uint32_t row0, const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos,
+                                     void *stream)
 {
     if (m == 0) return HKCSA_OK;
     HK_REQUIRE(d_wt_blob && h_wt && d_occ_blob && p && d_ssa_blob && h_ssa && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
     HK_REQUIRE(p->n == h_wt->n && p->sigma == h_wt->sigma && h_ssa->n == p->n, HKCSA_EINVAL, "plans do not match");
+    HK_REQUIRE(row0 < p->n, HKCSA_EINVAL, "row0 (the row of suffix 0) out of range");
     cudaStream_t st = as_stream(stream);
     const WtTables *d_tab = reinterpret_cast<const WtTables *>(static_cast<const uint8_t *>(d_wt_blob) + h_wt->off_tables);
     OccDev occ;
@@ -509,11 +527,14 @@ extern "C" int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan 
     const uint32_t grid = (uint32_t)((m + 255) / 256);
     prof::Scope ps(st, prof::LOCATE, 0);
     if (p->layout == 1)
-        locate_rows_occ_kernel<0><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, d_rows, m, d_out_pos);
+        locate_rows_occ_kernel<0><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
+                                                            d_out_pos);
     else if (p->shift == 5)
-        locate_rows_occ_kernel<5><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, d_rows, m, d_out_pos);
+        locate_rows_occ_kernel<5><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
+                                                            d_out_pos);
     else
-        locate_rows_occ_kernel<6><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, d_rows, m, d_out_pos);
+        locate_rows_occ_kernel<6><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
+                                                            d_out_pos);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }

@@ -199,8 +199,8 @@ SIGNATURES = {
                                        _u32, C.POINTER(_u64), C.POINTER(_u64), _vp]),
     "hkcsa_ranges_push_peers": (_i32, [_vp, _vp, _u64, _u64, _u32, C.POINTER(_u64), _u64, _vp]),
     "hkcsa_ranges_unpack": (_i32, [_vp, _u64, _vp, _vp, _vp]),
-    "hkcsa_locate_rows_occ": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(OccPlan), _vp, C.POINTER(SsaPlan), _vp,
-                                     _u64, _vp, _vp]),
+    "hkcsa_locate_rows_occ": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(OccPlan), _vp, C.POINTER(SsaPlan), _u32,
+                                     _vp, _u64, _vp, _vp]),
     "hkcsa_isa_samples": (_i32, [_vp, C.POINTER(SsaPlan), _vp, _vp]),
     "hkcsa_extract_scratch_bytes": (_sz, [_u64]),
     "hkcsa_extract": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(OccPlan), _vp, _u32, _vp, _vp, _vp, _u64, _vp,
@@ -220,7 +220,7 @@ SIGNATURES = {
     "hkcsa_multi_locate_rows": (_i32, [_vp, _vp, _u64, _vp, _vp]),
     "hkcsa_expand_ranges": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp]),
     "hkcsa_gather_u32": (_i32, [_vp, _vp, _u64, _vp, _vp]),
-    "hkcsa_locate_rows": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(SsaPlan), _vp, _u64, _vp, _vp]),
+    "hkcsa_locate_rows": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(SsaPlan), _u32, _vp, _u64, _vp, _vp]),
     "hkcsa_symbol_positions_scratch_bytes": (_sz, [_u64]),
     "hkcsa_symbol_positions": (_i32, [_vp, _u64, _vp, _vp, _vp, _sz, _vp]),
     "hkcsa_rrr_tables_bytes": (_sz, []),

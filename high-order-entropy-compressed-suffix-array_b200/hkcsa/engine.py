@@ -899,14 +899,17 @@ class DeviceIndex:
         if use_samples:
             if self.ssa is None:
                 raise ValueError("index was built without a sampled suffix array")
+            if rows.numel() == 0:
+                return out
+            row0 = self.row_of_suffix0()
             occ = getattr(self, "_occ", None)
             if occ is not None:      # LF steps from the sampled Occ table: two sectors instead of one per level
                 check(L.hkcsa_locate_rows_occ(_ptr(self.wt.blob), C.byref(self.wt.plan), _ptr(occ[1]), C.byref(occ[0]),
-                                              _ptr(self.ssa.blob), C.byref(self.ssa.plan), _ptr(rows), rows.numel(),
-                                              _ptr(out), _stream()))
+                                              _ptr(self.ssa.blob), C.byref(self.ssa.plan), row0, _ptr(rows),
+                                              rows.numel(), _ptr(out), _stream()))
                 return out
             check(L.hkcsa_locate_rows(_ptr(self.wt.blob), C.byref(self.wt.plan), _ptr(self.ssa.blob),
-                                      C.byref(self.ssa.plan), _ptr(rows), rows.numel(), _ptr(out), _stream()))
+                                      C.byref(self.ssa.plan), row0, _ptr(rows), rows.numel(), _ptr(out), _stream()))
         else:
             check(L.hkcsa_gather_u32(_ptr(self.sa), _ptr(rows), rows.numel(), _ptr(out), _stream()))
         return out
@@ -922,6 +925,13 @@ class DeviceIndex:
             check(_lib.load().hkcsa_isa_samples(_ptr(self.ssa.blob), C.byref(self.ssa.plan), _ptr(out), _stream()))
             self._isa = out
         return self._isa
+
+    def row_of_suffix0(self) -> int:
+        """The row of suffix 0 (isa_samples()[0]): the LF step of a sampled locate needs it to be exact on a text that
+        holds its last symbol elsewhere too.  Read back once per sampled suffix array."""
+        if getattr(self, "_row0", None) is None or self._row0[0] is not self.ssa:
+            self._row0 = (self.ssa, int(self.isa_samples()[0].item()))
+        return self._row0[1]
 
     @property
     def invertible(self) -> bool:

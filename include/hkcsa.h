@@ -357,13 +357,15 @@ int hkcsa_expand_ranges(const int64_t *d_lo, const int64_t *d_hi, const int64_t 
 /* csa/enhanced_fm_index.py:19): out[q] = SA[rows[q]], SA order preserved.       */
 int hkcsa_gather_u32(const uint32_t *d_src, const uint32_t *d_rows, uint64_t m, uint32_t *d_out,
                      void *stream);
-/* locate, step 2b: positions by LF walk to the next sampled row.  With a unique */
-/* sentinel a walk takes at most rate-1 steps; a walk that exceeds them (text    */
-/* that already contains the sentinel: LF is then not the inverse of the suffix  */
-/* order) stops and writes HKCSA_NO_POSITION instead of spinning.                */
+/* locate, step 2b: positions by LF walk to the next sampled row.  row0 = the   */
+/* row of suffix 0 (hkcsa_isa_samples()[0]).  The LF step is exact on every text */
+/* (also one that holds its last symbol elsewhere, e.g. a second '$': occ alone  */
+/* would misrank row0 there), so a walk meets a marked row within rate-1 steps; */
+/* a walk that exceeds them (only on a corrupt index) stops and writes          */
+/* HKCSA_NO_POSITION instead of spinning.                                        */
 #define HKCSA_NO_POSITION 0xFFFFFFFFu
 int hkcsa_locate_rows(const void *d_wt_blob, const hkcsa_wt_plan *h_plan, const void *d_ssa_blob,
-                      const hkcsa_ssa_plan *h_ssa, const uint32_t *d_rows, uint64_t m,
+                      const hkcsa_ssa_plan *h_ssa, uint32_t row0, const uint32_t *d_rows, uint64_t m,
                       uint32_t *d_out_pos, void *stream);
 
 /* ------------------------------------------------------------------------ */
@@ -544,7 +546,7 @@ int hkcsa_ranges_unpack(const uint64_t *d_packed, uint64_t P, int64_t *d_lo, int
 /* hkcsa_locate_rows with the LF step (symbol + its count) read from the Occ table; same positions. */
 int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan, const void *d_occ_blob,
                           const hkcsa_occ_plan *h_plan, const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa,
-                          const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos, void *stream);
+                          uint32_t row0, const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos, void *stream);
 
 /* ------------------------------------------------------------------------ */
 /* K4c extract: text[begin:end) back out of the index, without the text (no  */

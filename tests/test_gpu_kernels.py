@@ -860,3 +860,28 @@ def test_psi_is_the_inverse_of_lf(E, name):
     assert np.array_equal(sa[psi], (sa + 1) % n)
     w_pos, _ = O.symbol_positions(host(idx.bwt))
     assert np.array_equal(psi.astype(np.uint32), w_pos)
+
+
+@pytest.mark.parametrize("mode", ["wt", "occ0_shift5", "occ0_shift6", "occ1"])
+@pytest.mark.parametrize("text,rate", [(b"ab$ab$", 6), (b"a$b$a$", 2), (b"mississippi$" * 400 + b"$", 32),
+                                       (b"mississippi$" * 40 + b"$", 5), (b"banana$", 3)])
+def test_sampled_locate_is_exact_when_the_last_symbol_occurs_earlier(E, text, rate, mode):
+    """A text that holds its last symbol elsewhere too (a second '$'): occ alone ranks the row of suffix 0 after the
+    other rows holding that symbol, so a plain LF step goes wrong there -- on "mississippi$" * 400 + "$" at rate 32,
+    600 of 4801 walks reported a position 12 too far and 3000 none.  The locate kernels take the exact step (row0
+    from the inverse samples): every row gives the position its suffix-array entry holds, on the tree and on every
+    Occ-table layout, also from an index that keeps no suffix array."""
+    n = len(text)
+    sa = O.build_suffix_array(text).astype(np.int64)
+    idx = E.DeviceIndex(dev(E, text), sa_sample_rate=rate, keep_sa=False)
+    if mode != "wt":
+        layout, shift = (1, 5) if mode == "occ1" else (0, int(mode[-1]))
+        idx.build_occ_table(shift, layout=layout)
+    assert idx.row_of_suffix0() == int(np.flatnonzero(sa == 0)[0])
+    rows = torch.arange(n, dtype=torch.int32, device="cuda")
+    got = idx.locate_rows(rows).cpu().numpy().astype(np.int64)       # no suffix array: the samples are used
+    assert np.array_equal(got, sa)
+    o, p = idx.locate_batch(*E.pack_patterns([b"ss", b"$", b"i$", b"a"]))
+    o, p = o.cpu().numpy(), p.cpu().numpy()
+    for k, pat in enumerate([b"ss", b"$", b"i$", b"a"]):
+        assert sorted(p[o[k]:o[k + 1]].tolist()) == [m for m in range(n) if text.startswith(pat, m)], pat
