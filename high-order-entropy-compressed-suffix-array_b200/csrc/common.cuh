@@ -206,6 +206,13 @@ __device__ __forceinline__ uint32_t lf_fix(uint32_t occ, uint32_t code, uint32_t
     if (!fix || code != c0 || j > row0) return occ;
     return j == row0 ? 0u : occ + 1u;
 }
+// the same step over 64-bit rows (the sliced index of the distributed build, csrc/multi_slice.cu)
+__device__ __forceinline__ uint64_t lf_fix(uint64_t occ, uint32_t code, uint64_t j, uint32_t c0, uint64_t row0,
+                                           uint32_t fix)
+{
+    if (!fix || code != c0 || j > row0) return occ;
+    return j == row0 ? 0ull : occ + 1ull;
+}
 // one 256-bit read-only load (sm_100: LDG.E.256) of a 32-byte-aligned sector
 __device__ __forceinline__ void ld_nc_256(const void *p, uint64_t &w0, uint64_t &w1, uint64_t &w2, uint64_t &w3)
 {

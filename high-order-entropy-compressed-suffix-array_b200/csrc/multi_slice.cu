@@ -20,6 +20,7 @@ struct MultiDesc {
     uint32_t S;
     uint32_t rate;                             // 0 = no sampled SA
     uint64_t n;
+    uint64_t row0;                             // global row of suffix 0 (UINT64_MAX: no sampled SA)
 };
 
 __device__ __forceinline__ uint32_t ms_slice_of(const MultiDesc *d, uint64_t i)
@@ -99,11 +100,27 @@ __device__ __forceinline__ uint32_t ms_access_rank(const WtDev &w, uint32_t i, u
     return lo;
 }
 
-// text position of global row j: LF walk across slices until a marked row
+// text position of global row j: LF walk across slices until a marked row.  The step is the exact one of
+// locate_rows_kernel (lf_fix, csrc/common.cuh) on global rows and byte symbols: slices number their codes apart.
 __global__ void __launch_bounds__(256)
 ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ rows, uint64_t m,
                  uint64_t *__restrict__ out)
 {
+    __shared__ uint32_t s_c0, s_fix;
+    const uint64_t row0 = d->row0;
+    if (threadIdx.x == 0) {             // c0 = bwt[row0] = text[n-1]; LF needs fixing iff c0 occurs before row0
+        s_c0 = 0;
+        s_fix = 0;
+        if (row0 < d->n) {
+            const uint32_t s = ms_slice_of(d, row0);
+            const WtDev &w = d->slice[s];
+            uint32_t occ0;
+            const uint32_t code = ms_access_rank(w, (uint32_t)(row0 - d->start[s]), occ0);
+            s_c0 = w.tab->sym_of_code[code];
+            s_fix = (d->cum[s][s_c0] + occ0) != 0;
+        }
+    }
+    __syncthreads();
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= m) return;
     uint64_t j = rows[q];
@@ -120,12 +137,14 @@ ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ r
             out[q] = (uint64_t)d->samples[s][r] * d->rate + steps;
             return;
         }
-        if (steps >= d->rate) { out[q] = ~0ull; return; }       // sentinel not unique: see locate_rows_kernel
+        // with the exact step a walk meets a marked row within rate-1 steps on every text; the bound only keeps a
+        // walk over a corrupt index from spinning
+        if (steps >= d->rate) { out[q] = HKCSA_NO_POSITION64; return; }
         const WtDev &w = d->slice[s];
         uint32_t occ;
         const uint32_t code = ms_access_rank(w, lj, occ);
         const uint32_t byte = w.tab->sym_of_code[code];
-        j = d->C[byte] + d->cum[s][byte] + occ;
+        j = d->C[byte] + lf_fix(d->cum[s][byte] + occ, byte, j, s_c0, row0, s_fix);
         ++steps;
     }
 }
@@ -137,10 +156,12 @@ using namespace hkcsa;
 extern "C" size_t hkcsa_multi_desc_bytes(void) { return sizeof(MultiDesc); }
 
 // h_starts: uint64[S+1] global first row of every slice (h_starts[S] = n).  d_ssa_blobs / h_ssa_plans may be
-// NULL (no locate).  Builds the descriptor on the host and copies it into d_desc (hkcsa_multi_desc_bytes()).  syncs.
+// NULL (no locate); row0 = the global row of suffix 0 (< n), UINT64_MAX without them.  Builds the descriptor on the
+// host and copies it into d_desc (hkcsa_multi_desc_bytes()).  syncs.
 extern "C" int hkcsa_multi_desc_build(uint32_t S, const void *const *d_wt_blobs, const hkcsa_wt_plan *const *h_plans,
                                       const uint64_t *h_starts, const void *const *d_ssa_blobs,
-                                      const hkcsa_ssa_plan *const *h_ssa_plans, void *d_desc, void *stream)
+                                      const hkcsa_ssa_plan *const *h_ssa_plans, uint64_t row0, void *d_desc,
+                                      void *stream)
 {
     HK_REQUIRE(S >= 1 && S <= HKCSA_MAX_SLICES, HKCSA_EINVAL, "1..HKCSA_MAX_SLICES slices");
     HK_REQUIRE(d_wt_blobs && h_plans && h_starts && d_desc, HKCSA_EINVAL, "null pointer");
@@ -175,6 +196,9 @@ extern "C" int hkcsa_multi_desc_build(uint32_t S, const void *const *d_wt_blobs,
         run += tot[c];
     }
     HK_REQUIRE(run == D.n, HKCSA_EINVAL, "slice symbol counts do not add up to n");
+    HK_REQUIRE(row0 < D.n || (row0 == UINT64_MAX && D.rate == 0), HKCSA_EINVAL,
+               "row0 (the row of suffix 0) out of range");
+    D.row0 = row0;
     cudaStream_t st = as_stream(stream);
     HK_CUDA(cudaMemcpyAsync(d_desc, &D, sizeof(D), cudaMemcpyHostToDevice, st));
     HK_CUDA(cudaStreamSynchronize(st));

@@ -215,7 +215,7 @@ SIGNATURES = {
     "hkcsa_ssa_plan_make_slice": (_i32, [_u64, _u32, _u64, C.POINTER(SsaPlan)]),
     "hkcsa_multi_desc_bytes": (_sz, []),
     "hkcsa_multi_desc_build": (_i32, [_u32, C.POINTER(_vp), C.POINTER(C.POINTER(WtPlan)), C.POINTER(_u64),
-                                      C.POINTER(_vp), C.POINTER(C.POINTER(SsaPlan)), _vp, _vp]),
+                                      C.POINTER(_vp), C.POINTER(C.POINTER(SsaPlan)), _u64, _vp, _vp]),
     "hkcsa_multi_count_batch": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),
     "hkcsa_multi_locate_rows": (_i32, [_vp, _vp, _u64, _vp, _vp]),
     "hkcsa_expand_ranges": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp]),

@@ -457,19 +457,23 @@ class MultiSliceIndex:
     build), so count / locate run locally and the pattern batch can be sharded exactly as for one index."""
 
     def __init__(self, n: int, slices, sa_sample_rate: int = 0):
-        """slices: list of dicts with 'bwt' (uint8 tensor) and, for locate, 'sa' (uint32-as-int32 tensor), in
-        rank order.  Builds the per-slice structures with libhkcsa K3 / the sampled-SA kernels."""
+        """slices: list of dicts with 'bwt' (uint8 tensor) and, for locate, 'sa' (uint32-as-int32 or int64 tensor),
+        in rank order.  Builds the per-slice structures with libhkcsa K3 / the sampled-SA kernels."""
         from .engine import DeviceWaveletTree
         self.n = n
         self.device = slices[0]["bwt"].device
         self.wts, self.ssas = [], []
+        self.row0 = -1
         starts = [0]
         for sl in slices:
             bw = sl["bwt"]
             self.wts.append(DeviceWaveletTree(bw))
-            starts.append(starts[-1] + bw.numel())
             if sa_sample_rate > 0:
                 self.ssas.append(_sampled_sa_slice(sl["sa"], sa_sample_rate))
+                hit = (sl["sa"] == 0).nonzero()                   # plumbing: where suffix 0 is
+                if hit.numel():
+                    self.row0 = starts[-1] + int(hit[0, 0])
+            starts.append(starts[-1] + bw.numel())
         if starts[-1] != n:
             raise ValueError("slice lengths do not add up to n")
         self.starts = starts
@@ -477,11 +481,12 @@ class MultiSliceIndex:
         self._assemble()
 
     @classmethod
-    def from_parts(cls, n, starts, wt_parts, ssa_parts, rate):
-        """wt_parts: [(WtPlan, blob tensor)], ssa_parts: [(SsaPlan, blob tensor)] or [] -- replicas."""
+    def from_parts(cls, n, starts, wt_parts, ssa_parts, rate, row0):
+        """wt_parts: [(WtPlan, blob tensor)], ssa_parts: [(SsaPlan, blob tensor)] or [] -- replicas.  row0: the
+        global row of suffix 0 (-1 without ssa_parts); the exact LF step of locate needs it."""
         from .engine import DeviceWaveletTree, SampledSA
         self = cls.__new__(cls)
-        self.n, self.starts, self.rate = n, list(starts), rate
+        self.n, self.starts, self.rate, self.row0 = n, list(starts), rate, int(row0)
         self.device = wt_parts[0][1].device
         self.wts = []
         for plan, blob in wt_parts:
@@ -506,7 +511,8 @@ class MultiSliceIndex:
             splans = (C.POINTER(_lib.SsaPlan) * S)(*[C.pointer(s.plan) for s in self.ssas])
         else:
             sblobs, splans = None, None
-        check(L.hkcsa_multi_desc_build(S, blobs, plans, starts, sblobs, splans, _ptr(self.desc), _stream()))
+        row0 = self.row0 if self.row0 >= 0 else (1 << 64) - 1
+        check(L.hkcsa_multi_desc_build(S, blobs, plans, starts, sblobs, splans, row0, _ptr(self.desc), _stream()))
 
     def count_batch(self, pat: torch.Tensor, off: torch.Tensor):
         P = off.numel() - 1
@@ -528,9 +534,17 @@ class MultiSliceIndex:
         total = int(out_off[-1].item()) if P else 0
         rows = _empty(total, torch.int64, self.device)
         check(L.hkcsa_expand_ranges64(_ptr(lo), _ptr(hi), _ptr(out_off), P, _ptr(rows), _stream()))
-        out = _empty(total, torch.int64, self.device)
-        check(L.hkcsa_multi_locate_rows(_ptr(self.desc), _ptr(rows), total, _ptr(out), _stream()))
-        return out_off, out
+        return out_off, self.locate_rows(rows)
+
+    def locate_rows(self, rows: torch.Tensor) -> torch.Tensor:
+        """int64 global rows -> int64 text positions (SA[row]) through LF walks across slices; -1 only for a walk
+        over a corrupt index."""
+        if not self.ssas:
+            raise ValueError("index was built without a sampled suffix array")
+        rows = rows.to(device=self.device, dtype=torch.int64).contiguous()
+        out = _empty(rows.numel(), torch.int64, self.device)
+        check(_lib.load().hkcsa_multi_locate_rows(_ptr(self.desc), _ptr(rows), rows.numel(), _ptr(out), _stream()))
+        return out
 
 
 def _sampled_sa_slice(sa_slice: torch.Tensor, rate: int):
@@ -560,16 +574,21 @@ def replicate_sliced_index(sl: SuffixArraySlice, sa_sample_rate: int = 32, group
     wt = DeviceWaveletTree(sl.bwt)
     ssa = _sampled_sa_slice(sl.sa, sa_sample_rate) if sa_sample_rate > 0 else None
     wsz, ssz = C.sizeof(_lib.WtPlan), C.sizeof(_lib.SsaPlan)
-    head = torch.zeros(24 + wsz + ssz, dtype=torch.uint8)
-    head[:24] = torch.from_numpy(np.array([sl.sa.numel(), wt.blob.numel(), ssa.blob.numel() if ssa is not None else 0],
-                                          dtype=np.int64).view(np.uint8))
-    head[24:24 + wsz] = torch.frombuffer(bytearray(bytes(wt.plan)), dtype=torch.uint8)
+    mine0 = -1                                               # my global row of suffix 0, or -1
     if ssa is not None:
-        head[24 + wsz:] = torch.frombuffer(bytearray(bytes(ssa.plan)), dtype=torch.uint8)
+        hit = (sl.sa == 0).nonzero()
+        mine0 = sl.offset + int(hit[0, 0]) if hit.numel() else -1
+    H = 32
+    head = torch.zeros(H + wsz + ssz, dtype=torch.uint8)
+    head[:H] = torch.from_numpy(np.array([sl.sa.numel(), wt.blob.numel(), ssa.blob.numel() if ssa is not None else 0,
+                                          mine0], dtype=np.int64).view(np.uint8))
+    head[H:H + wsz] = torch.frombuffer(bytearray(bytes(wt.plan)), dtype=torch.uint8)
+    if ssa is not None:
+        head[H + wsz:] = torch.frombuffer(bytearray(bytes(ssa.plan)), dtype=torch.uint8)
     heads = torch.empty((world, head.numel()), dtype=torch.uint8, device=dev)
     dist.all_gather_into_tensor(heads, head.to(dev), group=group)
     heads = heads.cpu().numpy()
-    meta = [heads[r, :24].view(np.int64).tolist() for r in range(world)]
+    meta = [heads[r, :H].view(np.int64).tolist() for r in range(world)]
     starts = [0]
     for r in range(world):
         starts.append(starts[-1] + meta[r][0])
@@ -584,9 +603,10 @@ def replicate_sliced_index(sl: SuffixArraySlice, sa_sample_rate: int = 32, group
         return [allb[r, : sizes[r]] for r in range(world)]
 
     wt_blobs = gather_blobs(wt.blob, [m[1] for m in meta])
-    wt_parts = [(_lib.WtPlan.from_buffer_copy(heads[r, 24:24 + wsz].tobytes()), wt_blobs[r]) for r in range(world)]
+    wt_parts = [(_lib.WtPlan.from_buffer_copy(heads[r, H:H + wsz].tobytes()), wt_blobs[r]) for r in range(world)]
     ssa_parts = []
     if sa_sample_rate > 0:
         ssa_blobs = gather_blobs(ssa.blob, [m[2] for m in meta])
-        ssa_parts = [(_lib.SsaPlan.from_buffer_copy(heads[r, 24 + wsz:].tobytes()), ssa_blobs[r]) for r in range(world)]
-    return MultiSliceIndex.from_parts(sl.n, starts, wt_parts, ssa_parts, sa_sample_rate)
+        ssa_parts = [(_lib.SsaPlan.from_buffer_copy(heads[r, H + wsz:].tobytes()), ssa_blobs[r]) for r in range(world)]
+    row0 = max(m[3] for m in meta)
+    return MultiSliceIndex.from_parts(sl.n, starts, wt_parts, ssa_parts, sa_sample_rate, row0)

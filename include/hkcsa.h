@@ -400,14 +400,18 @@ int hkcsa_expand_ranges64(const int64_t *d_lo, const int64_t *d_hi, const int64_
 /* [h_starts[s], h_starts[s+1]) with its own wavelet-tree blob / plan (hkcsa_wt_build over its BWT slice) and, */
 /* optionally, its own sampled SA.  The descriptor lives in device memory (hkcsa_multi_desc_bytes()).          */
 /* Same recurrences and miss conventions as hkcsa_count_batch; rows and positions are global (n <= 2^40).      */
+/* row0 = the global row of suffix 0 (< n), UINT64_MAX when there is no sampled SA: the LF step of locate is   */
+/* the exact one of hkcsa_locate_rows, also on a text that holds its last symbol elsewhere.                    */
 #define HKCSA_MAX_SLICES 8
 size_t hkcsa_multi_desc_bytes(void);
 int hkcsa_multi_desc_build(uint32_t S, const void *const *d_wt_blobs, const hkcsa_wt_plan *const *h_plans,
                            const uint64_t *h_starts, const void *const *d_ssa_blobs,
-                           const hkcsa_ssa_plan *const *h_ssa_plans, void *d_desc, void *stream);
+                           const hkcsa_ssa_plan *const *h_ssa_plans, uint64_t row0, void *d_desc, void *stream);
 int hkcsa_multi_count_batch(const void *d_desc, const uint8_t *d_pat, const int64_t *d_off, uint64_t P,
                             int64_t *d_lo, int64_t *d_hi, void *stream);
-/* rows and positions are 64-bit (the sliced index may exceed 2^32 rows): use hkcsa_expand_ranges64 */
+/* rows and positions are 64-bit (the sliced index may exceed 2^32 rows): use hkcsa_expand_ranges64.  A walk  */
+/* longer than rate steps (a corrupt index only) writes HKCSA_NO_POSITION64 (-1 as int64).                    */
+#define HKCSA_NO_POSITION64 0xFFFFFFFFFFFFFFFFull
 int hkcsa_multi_locate_rows(const void *d_desc, const uint64_t *d_rows, uint64_t m, uint64_t *d_out_pos,
                             void *stream);
 

@@ -4,7 +4,9 @@ The CPU oracle sorts suffixes by comparison, which is too slow at n = 2^30 and o
 are linear or n log n, run on CPU tensors as well as CUDA tensors, and are pinned to the oracle on small inputs by
 tests/test_device_reference.py.  Every function works in chunks: at n = 2^30 its peak beside its inputs stays within
 about 16 GB (check_suffix_array: the int32 ISA + ~1 GB; symbol_positions: int32[n] + ~1 GB), except entropy_hk, whose
-torch.unique over n packed int64 windows takes about 3 x 8 B x n (26 GB at 2^30).
+torch.unique over n packed int64 windows takes about 3 x 8 B x n (26 GB at 2^30).  Past 2^31 - 1 symbols (the
+distributed build) rows and suffix ids no longer fit int32: the ISA and the row lists are int64 there (about 17 GB
++ ~1 GB each at 2^31), and `wide=True` forces that form at any size.  Suffix arrays may be int32 or int64.
 
 Conventions are those of the package: suffixes compare as byte strings and a proper prefix sorts first; ranges are
 inclusive (lo, hi) with (-1, -1) for a miss and (0, n-1) for the empty pattern; rank(p) counts ones in [0, p);
@@ -23,23 +25,34 @@ def _chunks(n: int, chunk: int = CHUNK):
 
 
 # ------------------------------------------------------------------ suffix array
-def check_suffix_array(text: torch.Tensor, sa: torch.Tensor, chunk: int = CHUNK) -> torch.Tensor:
+INT32_MAX = (1 << 31) - 1
+
+
+def _row_dtype(n: int, wide: bool | None) -> torch.dtype:
+    """int32 while every row and suffix id < n fits it, else (or with wide=True) int64."""
+    return torch.int64 if wide or n > INT32_MAX else torch.int32
+
+
+def check_suffix_array(text: torch.Tensor, sa: torch.Tensor, chunk: int = CHUNK, *, wide: bool | None = None
+                       ) -> torch.Tensor:
     """The O(n) checker of Burkhardt and Kaerkkaeinen.  `sa` is the suffix array of `text` iff it is a permutation of
     [0, n) and, with R[j] = ISA[j] for j < n and R[n] = -1, every row i has
         (text[sa[i]], R[sa[i] + 1]) < (text[sa[i+1]], R[sa[i+1] + 1])   (strictly).
-    Raises AssertionError naming the first bad row; returns the ISA (int32[n])."""
+    Raises AssertionError naming the first bad row; returns the ISA (int32[n], int64[n] past 2^31 - 1 or with
+    wide=True)."""
     n = text.numel()
     assert sa.numel() == n, f"suffix array has {sa.numel()} entries for a text of {n}"
     dev = sa.device
+    dt = _row_dtype(n, wide)
     if n == 0:
-        return torch.empty(0, dtype=torch.int32, device=dev)
+        return torch.empty(0, dtype=dt, device=dev)
     lo, hi = int(sa.min()), int(sa.max())
     assert 0 <= lo and hi < n, f"suffix array entries out of [0, {n}): min {lo}, max {hi}"
-    isa = torch.empty(n, dtype=torch.int32, device=dev)
+    isa = torch.empty(n, dtype=dt, device=dev)
     for a, b in _chunks(n, chunk):
-        isa[sa[a:b].long()] = torch.arange(a, b, dtype=torch.int32, device=dev)
+        isa[sa[a:b].long()] = torch.arange(a, b, dtype=dt, device=dev)
     for a, b in _chunks(n, chunk):             # a duplicate leaves one of its rows overwritten by the other
-        bad = isa[sa[a:b].long()] != torch.arange(a, b, dtype=torch.int32, device=dev)
+        bad = isa[sa[a:b].long()] != torch.arange(a, b, dtype=dt, device=dev)
         if bool(bad.any()):
             i = a + int(bad.nonzero()[0, 0])
             raise AssertionError(f"suffix array is not a permutation: row {i} holds {int(sa[i])}, "
@@ -68,9 +81,10 @@ def bwt_of(text: torch.Tensor, sa: torch.Tensor, chunk: int = CHUNK) -> torch.Te
 
 
 # ------------------------------------------------------------------ rank over the BWT
-def symbol_positions(bwt: torch.Tensor, chunk: int = 1 << 25):
+def symbol_positions(bwt: torch.Tensor, chunk: int = 1 << 25, *, wide: bool | None = None):
     """(pos int32[n], start int64[257]): the rows of every byte value in ascending order, values in byte order;
-    the rows holding byte c are pos[start[c]:start[c+1]].  j = C[c] + occ(c, pos[j]) for every such row."""
+    the rows holding byte c are pos[start[c]:start[c+1]].  j = C[c] + occ(c, pos[j]) for every such row.  pos is
+    int64 past 2^31 - 1 rows or with wide=True."""
     n = bwt.numel()
     dev = bwt.device
     cnt = torch.zeros(256, dtype=torch.int64, device=dev)
@@ -79,14 +93,14 @@ def symbol_positions(bwt: torch.Tensor, chunk: int = 1 << 25):
     start = torch.zeros(257, dtype=torch.int64, device=dev)
     start[1:] = torch.cumsum(cnt, 0)
     base = start[:256].clone()
-    pos = torch.empty(n, dtype=torch.int32, device=dev)
+    pos = torch.empty(n, dtype=_row_dtype(n, wide), device=dev)
     for a, b in _chunks(n, chunk):
         vals, order = torch.sort(bwt[a:b], stable=True)
         cc = torch.bincount(vals.long(), minlength=256)
         cstart = torch.cumsum(cc, 0) - cc
         v = vals.long()
         dest = base[v] + torch.arange(b - a, device=dev) - cstart[v]
-        pos[dest] = (order + a).to(torch.int32)
+        pos[dest] = (order + a).to(pos.dtype)
         base += cc
     return pos, start
 

@@ -264,6 +264,59 @@ def test_distributed_build_plan_is_host_only():
     assert L.hkcsa_entropy_from_sa(None, 3, None, 5, out, None, 0, None) == 0 and list(out) == [0.0] * 5   # n <= k -> 0
 
 
+def test_distributed_plan_id_width_and_size_limit():
+    """Suffix ids stay 32-bit up to 2^32 - 2 symbols (one id value is kept free) and widen at 2^32 - 1; the build
+    takes texts up to 2^40 symbols and refuses one more with ERANGE."""
+    from hkcsa import _lib
+    L = _lib.load()
+    h = np.zeros(256, dtype=np.uint64)
+    h[97] = 10
+
+    def make(n):
+        p = _lib.DsaPlan()
+        return L.hkcsa_dsa_plan_make(h.ctypes.data_as(C.POINTER(C.c_uint64)), n, 0, C.byref(p)), p
+
+    assert _lib.DSA_MAX_N32 == (1 << 32) - 2
+    for n, rc, wide in (((1 << 32) - 2, 0, 0), ((1 << 32) - 1, 0, 1), (1 << 40, 0, 1)):
+        got_rc, p = make(n)
+        assert (got_rc, p.wide, p.n) == (rc, wide, n), n
+    assert make((1 << 40) + 1)[0] == _lib.ERANGE and b"2^40" in L.hkcsa_last_error()
+
+
+def test_multi_slice_descriptor_argument_checks_without_gpu():
+    """hkcsa_multi_desc_build refuses a bad slice count, n > 2^40, slice lengths that differ from their plans and a row
+    of suffix 0 outside [0, n) -- each before any CUDA call (none of the pointers is a device address)."""
+    from hkcsa import _lib
+    L = _lib.load()
+    parts = [b"banana", b"$abc"]
+    plans = [_plan(x) for x in parts]
+    ssa = []
+    for x in parts:
+        sp = _lib.SsaPlan()
+        assert L.hkcsa_ssa_plan_make_slice(len(x), 4, 1, C.byref(sp)) == 0
+        ssa.append(sp)
+    n = sum(len(x) for x in parts)
+    fake = [0x1000, 0x2000]
+
+    def build(S, starts, with_ssa=True, row0=0, plan_list=plans):
+        k = max(S, 1)
+        blobs = (C.c_void_p * k)(*(fake * k)[:k])
+        pl = (C.POINTER(_lib.WtPlan) * k)(*[C.pointer(plan_list[i % 2]) for i in range(k)])
+        st = (C.c_uint64 * len(starts))(*starts)
+        sb = (C.c_void_p * k)(*(fake * k)[:k]) if with_ssa else None
+        sp = (C.POINTER(_lib.SsaPlan) * k)(*[C.pointer(ssa[i % 2]) for i in range(k)]) if with_ssa else None
+        return L.hkcsa_multi_desc_build(S, blobs, pl, st, sb, sp, row0, C.c_void_p(0x3000), None)
+
+    assert build(0, [0]) == _lib.EINVAL
+    assert build(9, [0] + [n] * 9) == _lib.EINVAL and b"slices" in L.hkcsa_last_error()
+    assert build(2, [0, 6, (1 << 40) + 1]) == _lib.ERANGE and b"2^40" in L.hkcsa_last_error()
+    assert build(2, [0, 5, n]) == _lib.EINVAL and b"plan length" in L.hkcsa_last_error()
+    assert build(2, [0, 6, n], plan_list=plans[::-1]) == _lib.EINVAL
+    for row0 in (n, n + 1, (1 << 64) - 1):
+        assert build(2, [0, 6, n], row0=row0) == _lib.EINVAL and b"row0" in L.hkcsa_last_error(), row0
+    assert build(2, [0, 6, n], with_ssa=False, row0=n) == _lib.EINVAL and b"row0" in L.hkcsa_last_error()
+
+
 def test_pack_patterns_host_fast_and_slow_paths_agree():
     """One join + one encode for a list of latin-1 str patterns; bytes / mixed lists pattern by pattern: same CSR."""
     from hkcsa import engine

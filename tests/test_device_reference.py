@@ -118,6 +118,71 @@ def test_references_agree_with_the_oracle(name):
     assert R.lf_invertible(bwt, isa) == (inv.astype(np.uint8).tobytes() == text)
 
 
+# ------------------------------------------------------------------ the int64 forms (texts past 2^31 - 1 symbols)
+def test_row_dtype_switches_past_int32():
+    assert R._row_dtype(R.INT32_MAX, None) == torch.int32 and R._row_dtype(R.INT32_MAX + 1, None) == torch.int64
+    assert R._row_dtype(5, True) == torch.int64 and R._row_dtype(5, False) == torch.int32
+
+
+@pytest.mark.parametrize("name", golden_case_names())
+def test_int64_checker_accepts_golden_suffix_arrays(golden, name):
+    text = golden.text(name)
+    sa = torch.from_numpy(golden.get(f"{name}/sa").astype(np.int64))
+    isa = R.check_suffix_array(_t(text), sa, wide=True)
+    assert isa.dtype == torch.int64
+    if len(text):
+        assert np.array_equal(isa.numpy()[sa.numpy()], np.arange(len(text)))
+        assert R.bwt_of(_t(text), sa).numpy().tobytes() == golden.get(f"{name}/bwt").tobytes()
+
+
+@pytest.mark.parametrize("name", list(TEXTS))
+def test_int64_references_agree_with_the_oracle(name):
+    """An int64 suffix array through every reference, with the int64 ISA and row lists forced: the same answers as the
+    int32 forms and the oracle."""
+    text = TEXTS[name]()
+    n = len(text)
+    t, sa32 = _t(text), _sa(text)
+    sa = sa32.long()
+    isa = R.check_suffix_array(t, sa, chunk=777, wide=True)
+    assert isa.dtype == torch.int64 and torch.equal(isa, R.check_suffix_array(t, sa32).long())
+    bwt = R.bwt_of(t, sa, chunk=1000)
+    want_bwt = O.bwt_transform(text, sa32.numpy().astype(np.uint32))
+    assert np.array_equal(bwt.numpy(), want_bwt)
+    groups = R.symbol_positions(bwt, chunk=999, wide=True)
+    opos, ostart = O.symbol_positions(want_bwt)
+    assert groups[0].dtype == torch.int64
+    assert np.array_equal(groups[0].numpy(), opos.astype(np.int64)) and np.array_equal(groups[1].numpy(), ostart)
+    present = np.flatnonzero(np.bincount(want_bwt, minlength=256))
+    rng = np.random.RandomState(2)
+    sym = rng.choice(present, 3000).astype(np.uint8)
+    pos = rng.randint(0, n + 1, 3000)
+    got = R.occ_at(bwt, torch.from_numpy(sym), torch.from_numpy(pos), groups).numpy()
+    fm = O.FM(want_bwt)
+    assert all(got[q] == fm.rank(int(sym[q]), int(pos[q])) for q in range(3000))
+    pats, off = O.gen_patterns(6, 300, np.frombuffer(text[:-1] or b"a", dtype=np.uint8), 1, 64)
+    lo, hi = R.sa_range(t, sa, torch.from_numpy(pats), torch.from_numpy(off))
+    lo32, hi32 = R.sa_range(t, sa32, torch.from_numpy(pats), torch.from_numpy(off))
+    assert torch.equal(lo, lo32) and torch.equal(hi, hi32)
+    keep = [q for q in range(len(off) - 1) if b"$" not in pats[off[q]:off[q + 1] - 1].tobytes()]
+    w_lo, w_hi = fm.find_range_batch(pats, off)
+    assert np.array_equal(lo.numpy()[keep], w_lo[keep]) and np.array_equal(hi.numpy()[keep], w_hi[keep])
+    assert R.lf_invertible(bwt, isa) == R.lf_invertible(bwt, isa.int())
+
+
+def test_int64_references_see_a_flipped_row():
+    """The int64 row lists and occ reject what the int32 ones reject: a row moved to another symbol's list."""
+    text = MUT_TEXT
+    t, sa = _t(text), _sa(text).long()
+    bwt = R.bwt_of(t, sa)
+    pos, start = R.symbol_positions(bwt, wide=True)
+    bad = bwt.clone()
+    bad[1234] = bwt[1235] if bwt[1235] != bwt[1234] else bwt[0]
+    assert not torch.equal(R.symbol_positions(bad, wide=True)[0], pos)
+    q = torch.arange(len(text) + 1)
+    c = torch.full_like(q, int(bwt[1234])).to(torch.uint8)
+    assert not torch.equal(R.occ_at(bad, c, q), R.occ_at(bwt, c, q, (pos, start)))
+
+
 def _golden_hk_cases():
     with open(os.path.join(ROOT, "tests", "golden", "golden_hk.json")) as f:
         d = json.load(f)
@@ -198,8 +263,12 @@ MUT_TEXT = O.gen_text(O.ENG96, 12, 5000).tobytes() + b"$"
 
 
 def _reject(text: bytes, sa: np.ndarray, match: str):
+    """Both forms of the checker: an int32 suffix array with the int32 ISA, and an int64 one with the int64 ISA that
+    texts past 2^31 - 1 symbols take."""
     with pytest.raises(AssertionError, match=match):
         R.check_suffix_array(_t(text), torch.from_numpy(sa.astype(np.int32)), chunk=701)
+    with pytest.raises(AssertionError, match=match):
+        R.check_suffix_array(_t(text), torch.from_numpy(sa.astype(np.int64)), chunk=701, wide=True)
 
 
 def test_checker_rejects_two_adjacent_rows_with_equal_first_symbol_swapped():
