@@ -241,4 +241,16 @@ __device__ __forceinline__ uint64_t bv_rank(const BitVec &v, uint64_t i)
     return v.super[blk / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu) + block_rank(b, o);
 }
 
+// The mark test of a locate walk: is row j marked in the sampled SA, and if so slot = rank1(marks, j), the index of
+// its sample.
+__device__ __forceinline__ bool marked_slot(const BitVec &marks, uint32_t j, uint64_t &slot)
+{
+    const uint64_t g = j / HKCSA_BLOCK_BITS;
+    const uint32_t o = j - (uint32_t)g * HKCSA_BLOCK_BITS;
+    const RankBlock b = load_block(marks.blocks + g);
+    if (!block_bit(b, o)) return false;
+    slot = marks.super[g / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu) + block_rank(b, o);
+    return true;
+}
+
 }  // namespace hkcsa

@@ -12,6 +12,7 @@
 //    inversion.  Adjacent threads own adjacent segments, so the byte stores of a long range land close together.
 //    The LF step is the wavelet tree's access + rank descent, or the sampled Occ table's (layouts 0 and 1).
 #include "common.cuh"
+#include "occ.cuh"
 #include "prof.cuh"
 #include "wavelet.cuh"
 
@@ -132,49 +133,6 @@ seg_offsets_kernel(const int64_t *__restrict__ begin, const int64_t *__restrict_
     if (q == R - 1) seg_off[R] = ex + v;
 }
 
-// ---------------------------------------------------------------- LF steps
-// The sampled Occ table (occ_table.cu): layout 0 rows of [2^SHIFT BWT bytes][sigma x u32 counts], or (SHIFT == 0)
-// layout 1 per-symbol entries {count, bitmap of 32 rows} followed by a copy of the BWT.
-struct ExtOccView {
-    const uint8_t *rows;
-    uint64_t stride;
-    const uint8_t *bwt;
-};
-// LF(j) from the Occ table; sym = bwt[j].  The same step as locate_rows_occ_kernel's, kept apart from it so that the
-// locate kernels' code does not change with this file.
-template <int SHIFT>
-__device__ __forceinline__ uint32_t occ_lf(const ExtOccView &o, const uint32_t *s_C, const uint16_t *s_code, uint32_t j,
-                                          uint32_t &sym)
-{
-    if constexpr (SHIFT == 0) {
-        const uint32_t ch = __ldg(o.bwt + j);
-        const uint32_t code = s_code[ch];
-        const uint2 e = __ldg(reinterpret_cast<const uint2 *>(o.rows) + (uint64_t)code * o.stride + (j >> 5));
-        sym = ch;
-        return s_C[code] + e.x + __popc(e.y & ((1u << (j & 31u)) - 1u));
-    } else {
-        constexpr uint32_t B = 1u << SHIFT;
-        const uint8_t *row = o.rows + (uint64_t)(j >> SHIFT) * o.stride;
-        const uint32_t t = j & (B - 1);
-        uint64_t x[B / 8];
-#pragma unroll
-        for (int v = 0; v < (int)B / 32; ++v) ld_nc_256(row + 32 * v, x[4 * v], x[4 * v + 1], x[4 * v + 2], x[4 * v + 3]);
-        const uint32_t ch = __ldg(row + t);         // same sector as the loads above
-        const uint32_t code = s_code[ch];
-        const uint32_t base = __ldg(reinterpret_cast<const uint32_t *>(row + B) + code);
-        const uint32_t ch4 = ch * 0x01010101u;
-        uint64_t bits = 0;
-#pragma unroll
-        for (int v = 0; v < (int)B / 8; ++v) {       // bit i = (byte i of the row == ch)
-            const uint32_t lo = __vcmpeq4((uint32_t)x[v], ch4) & 0x01010101u;
-            const uint32_t hi = __vcmpeq4((uint32_t)(x[v] >> 32), ch4) & 0x01010101u;
-            bits |= (uint64_t)(((lo * 0x01020408u) >> 24) | (((hi * 0x01020408u) >> 24) << 4)) << (8 * v);
-        }
-        sym = ch;
-        return s_C[code] + base + __popcll(bits & ((1ull << t) - 1ull));
-    }
-}
-
 // ---------------------------------------------------------------- extract
 // Segment t of the batch: request q = the last with seg_off[q] <= t (binary search; a warp's lanes mostly share q
 // and read the same offsets), k = its (t - seg_off[q])-th sample block.
@@ -199,10 +157,14 @@ struct ExtractArgs {
     uint8_t *out;
 };
 
-// the walks of every segment, grid-strided; lf(j, sym) returns LF(j) and sets sym = bwt[j]
-template <typename LF>
-__device__ __forceinline__ void extract_walks(const ExtractArgs &a, LF lf)
+// the walks of every segment, grid-strided; each LF step of the rank source (WtDev or OccDev<SHIFT>, occ.cuh) gives
+// LF(j) and the symbol bwt[j]
+template <typename Src>
+__global__ void __launch_bounds__(EXT_THREADS) extract_kernel(Src src, ExtractArgs a)
 {
+    __shared__ typename Src::Smem s;
+    src.load(s);
+    __syncthreads();
     const uint64_t total = a.seg_off[a.R];
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += stride) {
@@ -215,36 +177,12 @@ __device__ __forceinline__ void extract_walks(const ExtractArgs &a, LF lf)
         uint32_t j = __ldg(a.isa + k + 1);
         uint8_t *dst = a.out + a.out_off[q];
         while (p > lo) {
-            uint32_t sym;
-            j = lf(j, sym);
-            --p;                                   // sym = text[p]
-            if (p < hi) dst[p - r.b] = (uint8_t)sym;
+            const LfStep st = src.step(s, j);
+            j = s.C[st.code] + st.occ;
+            --p;                                   // st.sym = text[p]
+            if (p < hi) dst[p - r.b] = (uint8_t)st.sym;
         }
     }
-}
-
-__global__ void __launch_bounds__(EXT_THREADS) extract_wt_kernel(WtDev wt, ExtractArgs a)
-{
-    __shared__ WtSmem s;
-    wt_smem_load(s, wt);
-    __syncthreads();
-    extract_walks(a, [&](uint32_t j, uint32_t &sym) {
-        uint32_t occ;
-        const uint32_t code = wt_access_rank(s, wt, j, occ);    // symbol and rank from one descent
-        sym = s.sym_of_code[code];
-        return s.C[code] + occ;
-    });
-}
-
-template <int SHIFT>
-__global__ void __launch_bounds__(EXT_THREADS) extract_occ_kernel(const WtTables *__restrict__ tab, ExtOccView occ, ExtractArgs a)
-{
-    __shared__ uint32_t s_C[260];
-    __shared__ uint16_t s_code[256];
-    for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s_C[i] = tab->C[i];
-    for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s_code[i] = tab->code_of_sym[i];
-    __syncthreads();
-    extract_walks(a, [&](uint32_t j, uint32_t &sym) { return occ_lf<SHIFT>(occ, s_C, s_code, j, sym); });
 }
 
 // the number of walks is known on the device only: a grid of exactly the resident CTAs strides over them
@@ -338,19 +276,11 @@ extern "C" int hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_pl
 
     ExtractArgs a{d_isa, rate, n, d_begin, d_end, d_out_off, R, seg_off, d_out};
     prof::Scope ps(st, prof::LOCATE, 0);
-    if (!h_occ_plan) {
-        extract_wt_kernel<<<resident_grid(extract_wt_kernel), EXT_THREADS, 0, st>>>(make_wt_dev(d_wt_blob, h_wt_plan), a);
-    } else {
-        const WtTables *tab = reinterpret_cast<const WtTables *>(static_cast<const uint8_t *>(d_wt_blob) + h_wt_plan->off_tables);
-        const ExtOccView occ{static_cast<const uint8_t *>(d_occ_blob), h_occ_plan->stride,
-                          static_cast<const uint8_t *>(d_occ_blob) + h_occ_plan->off_bwt};
-        if (h_occ_plan->layout == 1)
-            extract_occ_kernel<0><<<resident_grid(extract_occ_kernel<0>), EXT_THREADS, 0, st>>>(tab, occ, a);
-        else if (h_occ_plan->shift == 5)
-            extract_occ_kernel<5><<<resident_grid(extract_occ_kernel<5>), EXT_THREADS, 0, st>>>(tab, occ, a);
-        else
-            extract_occ_kernel<6><<<resident_grid(extract_occ_kernel<6>), EXT_THREADS, 0, st>>>(tab, occ, a);
-    }
-    HK_LAUNCH_CHECK();
-    return HKCSA_OK;
+    const auto launch = [&](auto src) {
+        extract_kernel<<<resident_grid(extract_kernel<decltype(src)>), EXT_THREADS, 0, st>>>(src, a);
+        HK_LAUNCH_CHECK();
+        return HKCSA_OK;
+    };
+    if (!h_occ_plan) return launch(make_wt_dev(d_wt_blob, h_wt_plan));
+    return with_occ_source(d_wt_blob, h_wt_plan, d_occ_blob, h_occ_plan, launch);
 }

@@ -2,9 +2,11 @@
 //
 // Replaces EnhancedFMIndex.find_range / .rank / .find (reference
 // csa/enhanced_fm_index.py:15-40).  occ[c][i] of build_occ (utils/utils.py:
-// 26-32) is answered by a rank walk over the wavelet tree; C[] and the node
-// tables live in shared memory; every rank step reads one 32-byte block.
+// 26-32) is answered by a rank source: the wavelet tree (WtDev, a rank walk that
+// reads one 32-byte block per level) or the sampled Occ table (OccDev, occ.cuh);
+// C[] and the source's tables live in shared memory.
 #include "common.cuh"
+#include "occ.cuh"
 #include "prof.cuh"
 #include "radix_sort.cuh"
 #include "wavelet.cuh"
@@ -24,20 +26,20 @@ constexpr int COUNT_THREADS = 256;
 // One lane per pattern.  A warp owns a contiguous chunk of the batch and refills a lane as soon as
 // its pattern ends (last symbol consumed or range empty), so ragged lengths (8-64) and early misses do
 // not idle the warp: every iteration each busy lane consumes ONE symbol -- both boundaries of the SA
-// range walk the wavelet tree together.  find_range (csa/enhanced_fm_index.py:21-32) in half-open form:
+// range take the rank step of the source together (Src: WtDev or OccDev<SHIFT>, occ.cuh).  find_range
+// (csa/enhanced_fm_index.py:21-32) in half-open form:
 //   l = 0, r = n;  per symbol from the end: l = C[c] + occ(c, l), r = C[c] + occ(c, r);
 //   l >= r -> (-1, -1).  Result (l, r-1).
-template <bool PEERS>
-__global__ void __launch_bounds__(COUNT_THREADS)
-fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__restrict__ off, uint64_t P,
+template <typename Src, int MIN_CTAS, bool PEERS>
+__global__ void __launch_bounds__(COUNT_THREADS, MIN_CTAS)
+fm_count_kernel(Src src, const uint8_t *__restrict__ pat, const int64_t *__restrict__ off, uint64_t P,
                 int64_t *__restrict__ out_lo, int64_t *__restrict__ out_hi, const uint2 *__restrict__ kmer, uint32_t kk,
                 PeerOut po)
 {
-    __shared__ WtSmem s;
-    wt_smem_load(s, wt);
+    __shared__ typename Src::Smem s;
+    src.load(s);
     __syncthreads();
-    const uint32_t lane = lane_id();
-    const uint32_t n = (uint32_t)wt.n;
+    const uint32_t n = (uint32_t)src.n;
     const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
     const uint64_t chunk = (P + nwarps - 1) / nwarps;
@@ -47,6 +49,7 @@ fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__rest
     int64_t p = -1;            // pattern owned by this lane, -1 = idle
     int64_t k = 0, b = 0;      // next symbol to consume, first symbol of the pattern
     uint32_t l = 0, r = 0;
+    uint32_t ch_next = 0;      // pat[k], loaded one step ahead so the step's rank loads do not wait for it
     while (true) {
         // ---- refill idle lanes with the next patterns of the chunk, in lane order
         const uint32_t idle = __ballot_sync(0xffffffffu, p < 0);
@@ -66,7 +69,7 @@ fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__rest
                     for (uint32_t t = 0; t < kk; ++t) {
                         const uint32_t code = s.code_of_sym[pat[k - kk + 1 + t]];
                         known = known && code != 0xFFFFu;
-                        id = id * wt.sigma + (known ? code : 0u);
+                        id = id * src.sigma + (known ? code : 0u);
                     }
                     if (known) {
                         const uint2 e2 = __ldg(kmer + id);
@@ -76,6 +79,7 @@ fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__rest
                         if (l >= r) { l = 1; r = 0; k = b - 1; }   // finishes below as a miss
                     }
                 }
+                if (k >= b) ch_next = pat[k];
             }
             next += __popc(idle);
             if (idle == 0xffffffffu && __ballot_sync(0xffffffffu, p >= 0) == 0) break;
@@ -84,10 +88,12 @@ fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__rest
         // ---- one backward-search step (or finish an exhausted / empty pattern)
         bool done = k < b, miss = l >= r;
         if (!done) {
-            const uint32_t code = s.code_of_sym[pat[k]];
+            const uint32_t ch = ch_next;
+            if (k > b) ch_next = pat[k - 1];
+            const uint32_t code = s.code_of_sym[ch];
             if (code == 0xFFFFu) { miss = true; }          // symbol absent: rank 0, C 0 -> empty range
             else {
-                if (wt.sigma > 1) wt_rank_code2(s, wt, code, l, r);
+                src.rank2(s, code, ch, l, r);
                 const uint32_t c0 = s.C[code];
                 l += c0;
                 r += c0;
@@ -103,9 +109,10 @@ fm_count_kernel(WtDev wt, const uint8_t *__restrict__ pat, const int64_t *__rest
     }
 }
 
-// rows[off[p] + k] = lo[p] + k: one warp per pattern
+// rows[off[p] + k] = lo[p] + k: one warp per pattern; Row = uint64_t for indexes beyond 2^32 rows
+template <typename Row>
 __global__ void expand_ranges_kernel(const int64_t *__restrict__ lo, const int64_t *__restrict__ hi,
-                                     const int64_t *__restrict__ out_off, uint64_t P, uint32_t *__restrict__ rows)
+                                     const int64_t *__restrict__ out_off, uint64_t P, Row *__restrict__ rows)
 {
     const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = lane_id();
@@ -113,21 +120,7 @@ __global__ void expand_ranges_kernel(const int64_t *__restrict__ lo, const int64
         const int64_t l = lo[p], h = hi[p];
         if (l < 0) continue;
         const int64_t o = out_off[p];
-        for (int64_t k = lane; k <= h - l; k += 32) rows[o + k] = (uint32_t)(l + k);
-    }
-}
-
-// 64-bit rows for indexes beyond 2^32 rows
-__global__ void expand_ranges64_kernel(const int64_t *__restrict__ lo, const int64_t *__restrict__ hi,
-                                       const int64_t *__restrict__ out_off, uint64_t P, uint64_t *__restrict__ rows)
-{
-    const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint32_t lane = lane_id();
-    for (uint64_t p = warp; p < P; p += ((uint64_t)gridDim.x * blockDim.x) >> 5) {
-        const int64_t l = lo[p], h = hi[p];
-        if (l < 0) continue;
-        const int64_t o = out_off[p];
-        for (int64_t k = lane; k <= h - l; k += 32) rows[o + k] = (uint64_t)(l + k);
+        for (int64_t k = lane; k <= h - l; k += 32) rows[o + k] = (Row)(l + k);
     }
 }
 
@@ -198,19 +191,20 @@ __global__ void gather_u32_kernel(const uint32_t *__restrict__ src, const uint32
 }
 
 // position of row j: walk LF until a marked row, pos = sample * rate + steps.
-// LF(j) = C[c] + occ(c, j) with c = bwt[j], both from one wavelet descent.
+// LF(j) = C[c] + occ(c, j) with c = bwt[j], both from one access + rank step of the source.
+template <typename Src>
 __global__ void __launch_bounds__(256)
-locate_rows_kernel(WtDev wt, BitVec marks, const uint32_t *__restrict__ samples, uint32_t rate, uint32_t row0,
+locate_rows_kernel(Src src, BitVec marks, const uint32_t *__restrict__ samples, uint32_t rate, uint32_t row0,
                    const uint32_t *__restrict__ rows, uint64_t m, uint32_t *__restrict__ out)
 {
-    __shared__ WtSmem s;
+    __shared__ typename Src::Smem s;
     __shared__ uint32_t s_c0, s_fix;
-    wt_smem_load(s, wt);
+    src.load(s);
     __syncthreads();
     if (threadIdx.x == 0) {             // c0 = bwt[row0] = text[n-1]; LF needs fixing iff c0 occurs before row0
-        uint32_t occ0;
-        s_c0 = wt_access_rank(s, wt, row0, occ0);
-        s_fix = occ0 != 0;
+        const LfStep t = src.step(s, row0);
+        s_c0 = t.code;
+        s_fix = t.occ != 0;
     }
     __syncthreads();
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -218,20 +212,16 @@ locate_rows_kernel(WtDev wt, BitVec marks, const uint32_t *__restrict__ samples,
     uint32_t j = rows[q];
     uint32_t steps = 0;
     while (true) {
-        const uint64_t g = j / HKCSA_BLOCK_BITS;
-        const uint32_t o = j - (uint32_t)g * HKCSA_BLOCK_BITS;
-        const RankBlock b = load_block(marks.blocks + g);
-        if (block_bit(b, o)) {
-            const uint64_t r = marks.super[g / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu) + block_rank(b, o);
-            out[q] = samples[r] * rate + steps;
+        uint64_t slot;
+        if (marked_slot(marks, j, slot)) {
+            out[q] = samples[slot] * rate + steps;
             return;
         }
         // with the exact LF step below a walk meets a marked row within rate-1 steps on every text; the bound only
         // keeps a walk over a corrupt index from spinning
         if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }
-        uint32_t occ;
-        const uint32_t code = wt_access_rank(s, wt, j, occ);
-        j = s.C[code] + lf_fix(occ, code, j, s_c0, row0, s_fix);
+        const LfStep t = src.step(s, j);
+        j = s.C[t.code] + lf_fix(t.occ, t.code, j, s_c0, row0, s_fix);
         ++steps;
     }
 }
@@ -335,6 +325,41 @@ extern "C" int hkcsa_kmer_table_build(const void *d_blob, const hkcsa_wt_plan *h
     return HKCSA_OK;
 }
 
+// The count kernel of rank source Src at MIN_CTAS CTAs per SM (0: no minimum), over a grid of twice the CTAs an SM
+// holds (4 when the kernel sets no minimum).
+template <typename Src, int MIN_CTAS>
+static int count_launch(const Src &src, const uint2 *kmer, uint32_t k, const uint8_t *d_pat, const int64_t *d_off,
+                        uint64_t P, int64_t *d_lo, int64_t *d_hi, const PeerOut &po, cudaStream_t st)
+{
+    const uint64_t per_sm = 2 * (MIN_CTAS ? MIN_CTAS : 4);
+    const int blocks = (int)std::min<uint64_t>((P + COUNT_THREADS - 1) / COUNT_THREADS, (uint64_t)num_sms() * per_sm);
+    const uint32_t kk = kmer ? k : 0u;
+    prof::Scope ps(st, prof::COUNT, 0);
+    if (po.n) fm_count_kernel<Src, MIN_CTAS, true><<<blocks, COUNT_THREADS, 0, st>>>(src, d_pat, d_off, P, d_lo, d_hi, kmer, kk, po);
+    else fm_count_kernel<Src, MIN_CTAS, false><<<blocks, COUNT_THREADS, 0, st>>>(src, d_pat, d_off, P, d_lo, d_hi, kmer, kk, po);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
+}
+
+// count over the sampled Occ table of plan p
+static int count_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob, const hkcsa_occ_plan *p,
+                     const void *d_kmer_table, uint32_t k, const uint8_t *d_pat, const int64_t *d_off, uint64_t P,
+                     int64_t *d_lo, int64_t *d_hi, const PeerOut &po, cudaStream_t st)
+{
+    HK_REQUIRE(p->n == h_wt->n && p->sigma == h_wt->sigma && p->n >= 1, HKCSA_EINVAL, "occ plan does not match the index");
+    const uint2 *kmer = static_cast<const uint2 *>(d_kmer_table);
+    return with_occ_source(d_wt_blob, h_wt, d_occ_blob, p, [&](auto occ) {
+        using Src = decltype(occ);
+        // 4 CTAs/SM (at most 48 registers for layout 1 and for 32 rows per entry, 63 for 64): measured best of 4 / 5 / 6
+        // / 8 on the 2.8 GB table (more lanes in flight were slower).  Layout 1: DRAM-resident tables run best at 4 CTAs/SM,
+        // tables near the L2 size at 6 (measured: 1.42 vs 1.34 G patterns/s on the 4.8 GB table of the 200 MB text,
+        // 3.4 vs 4.0 on the 225 MB DNA table)
+        if constexpr (std::is_same_v<Src, OccDev<0>>)
+            if (p->blob_bytes <= (1ull << 30)) return count_launch<Src, 6>(occ, kmer, k, d_pat, d_off, P, d_lo, d_hi, po, st);
+        return count_launch<Src, 4>(occ, kmer, k, d_pat, d_off, P, d_lo, d_hi, po, st);
+    });
+}
+
 extern "C" int hkcsa_count_batch_kmer(const void *d_blob, const hkcsa_wt_plan *h_plan, const void *d_kmer_table,
                                       uint32_t k, const uint8_t *d_pat, const int64_t *d_off, uint64_t P,
                                       int64_t *d_lo, int64_t *d_hi, void *stream)
@@ -345,19 +370,48 @@ extern "C" int hkcsa_count_batch_kmer(const void *d_blob, const hkcsa_wt_plan *h
     HK_REQUIRE(h_plan->n >= 1, HKCSA_EINVAL, "empty index");
     PeerOut po;
     memset(&po, 0, sizeof(po));
-    return count_wt_launch(make_wt_dev(d_blob, h_plan), static_cast<const uint2 *>(d_kmer_table), k, d_pat, d_off, P,
-                           d_lo, d_hi, po, as_stream(stream));
+    return count_launch<WtDev, 0>(make_wt_dev(d_blob, h_plan), static_cast<const uint2 *>(d_kmer_table), k, d_pat, d_off,
+                                  P, d_lo, d_hi, po, as_stream(stream));
 }
 
-int hkcsa::count_wt_launch(const WtDev &wt, const uint2 *kmer, uint32_t k, const uint8_t *d_pat, const int64_t *d_off,
-                           uint64_t P, int64_t *d_lo, int64_t *d_hi, const PeerOut &po, cudaStream_t st)
+extern "C" int hkcsa_count_batch_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
+                                     const hkcsa_occ_plan *p, const void *d_kmer_table, uint32_t k,
+                                     const uint8_t *d_pat, const int64_t *d_off, uint64_t P, int64_t *d_lo,
+                                     int64_t *d_hi, void *stream)
 {
-    const int blocks = (int)std::min<uint64_t>((P + COUNT_THREADS - 1) / COUNT_THREADS, (uint64_t)num_sms() * 8);
-    prof::Scope ps(st, prof::COUNT, 0);
-    if (po.n) fm_count_kernel<true><<<blocks, COUNT_THREADS, 0, st>>>(wt, d_pat, d_off, P, d_lo, d_hi, kmer, kmer ? k : 0u, po);
-    else fm_count_kernel<false><<<blocks, COUNT_THREADS, 0, st>>>(wt, d_pat, d_off, P, d_lo, d_hi, kmer, kmer ? k : 0u, po);
-    HK_LAUNCH_CHECK();
-    return HKCSA_OK;
+    HK_REQUIRE(d_wt_blob && h_wt && d_occ_blob && p, HKCSA_EINVAL, "null pointer");
+    if (P == 0) return HKCSA_OK;
+    HK_REQUIRE(d_off && d_lo && d_hi, HKCSA_EINVAL, "null pointer");
+    PeerOut po;
+    memset(&po, 0, sizeof(po));
+    return count_occ(d_wt_blob, h_wt, d_occ_blob, p, d_kmer_table, k, d_pat, d_off, P, d_lo, d_hi, po, as_stream(stream));
+}
+
+extern "C" int hkcsa_count_batch_peers(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
+                                       const hkcsa_occ_plan *h_occ, const void *d_kmer_table, uint32_t k,
+                                       const uint8_t *d_pat, const int64_t *d_off, uint64_t P, uint64_t out_base,
+                                       uint32_t n_peers, const uint64_t *h_peer_lo, const uint64_t *h_peer_hi, void *stream)
+{
+    HK_REQUIRE(d_wt_blob && h_wt && h_peer_lo && h_peer_hi, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(n_peers >= 1 && n_peers <= HKCSA_MAX_PEERS, HKCSA_EINVAL, "n_peers must be in [1, HKCSA_MAX_PEERS]");
+    HK_REQUIRE((d_occ_blob == nullptr) == (h_occ == nullptr), HKCSA_EINVAL, "occ blob and plan go together");
+    if (P == 0) return HKCSA_OK;
+    HK_REQUIRE(d_off != nullptr, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(h_wt->n >= 1, HKCSA_EINVAL, "empty index");
+    PeerOut po;
+    memset(&po, 0, sizeof(po));
+    po.n = n_peers;
+    po.base = out_base;
+    for (uint32_t r = 0; r < n_peers; ++r) {
+        HK_REQUIRE(h_peer_lo[r] && h_peer_hi[r], HKCSA_EINVAL, "null peer pointer");
+        po.lo[r] = reinterpret_cast<int64_t *>(static_cast<uintptr_t>(h_peer_lo[r]));
+        po.hi[r] = reinterpret_cast<int64_t *>(static_cast<uintptr_t>(h_peer_hi[r]));
+    }
+    cudaStream_t st = as_stream(stream);
+    if (d_occ_blob)
+        return count_occ(d_wt_blob, h_wt, d_occ_blob, h_occ, d_kmer_table, k, d_pat, d_off, P, nullptr, nullptr, po, st);
+    return count_launch<WtDev, 0>(make_wt_dev(d_wt_blob, h_wt), static_cast<const uint2 *>(d_kmer_table), k, d_pat, d_off,
+                                  P, nullptr, nullptr, po, st);
 }
 
 extern "C" int hkcsa_ssa_plan_make(uint64_t n, uint32_t rate, hkcsa_ssa_plan *p)
@@ -446,7 +500,7 @@ extern "C" int hkcsa_expand_ranges(const int64_t *d_lo, const int64_t *d_hi, con
     if (P == 0) return HKCSA_OK;
     HK_REQUIRE(d_lo && d_hi && d_out_off, HKCSA_EINVAL, "null pointer");
     const int blocks = (int)std::min<uint64_t>((P * 32 + 255) / 256, (uint64_t)num_sms() * 16);
-    expand_ranges_kernel<<<blocks, 256, 0, as_stream(stream)>>>(d_lo, d_hi, d_out_off, P, d_rows);
+    expand_ranges_kernel<uint32_t><<<blocks, 256, 0, as_stream(stream)>>>(d_lo, d_hi, d_out_off, P, d_rows);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }
@@ -457,7 +511,7 @@ extern "C" int hkcsa_expand_ranges64(const int64_t *d_lo, const int64_t *d_hi, c
     if (P == 0) return HKCSA_OK;
     HK_REQUIRE(d_lo && d_hi && d_out_off, HKCSA_EINVAL, "null pointer");
     const int blocks = (int)std::min<uint64_t>((P * 32 + 255) / 256, (uint64_t)num_sms() * 16);
-    expand_ranges64_kernel<<<blocks, 256, 0, as_stream(stream)>>>(d_lo, d_hi, d_out_off, P, d_rows);
+    expand_ranges_kernel<uint64_t><<<blocks, 256, 0, as_stream(stream)>>>(d_lo, d_hi, d_out_off, P, d_rows);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }
@@ -472,6 +526,23 @@ extern "C" int hkcsa_gather_u32(const uint32_t *d_src, const uint32_t *d_rows, u
     return HKCSA_OK;
 }
 
+template <typename Src>
+static int locate_launch(const Src &src, const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa, uint32_t row0,
+                         const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos, cudaStream_t st)
+{
+    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
+    BitVec marks;
+    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
+    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
+    marks.len = h_ssa->n;
+    prof::Scope ps(st, prof::LOCATE, 0);
+    locate_rows_kernel<Src><<<(uint32_t)((m + 255) / 256), 256, 0, st>>>(
+        src, marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), h_ssa->rate, row0, d_rows, m,
+        d_out_pos);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
+}
+
 extern "C" int hkcsa_locate_rows(const void *d_wt_blob, const hkcsa_wt_plan *h_plan, const void *d_ssa_blob,
                                  const hkcsa_ssa_plan *h_ssa, uint32_t row0, const uint32_t *d_rows, uint64_t m,
                                  uint32_t *d_out_pos, void *stream)
@@ -480,19 +551,22 @@ extern "C" int hkcsa_locate_rows(const void *d_wt_blob, const hkcsa_wt_plan *h_p
     HK_REQUIRE(d_wt_blob && h_plan && d_ssa_blob && h_ssa && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
     HK_REQUIRE(h_ssa->n == h_plan->n, HKCSA_EINVAL, "plans do not match");
     HK_REQUIRE(row0 < h_plan->n, HKCSA_EINVAL, "row0 (the row of suffix 0) out of range");
-    cudaStream_t st = as_stream(stream);
-    WtDev wt = make_wt_dev(d_wt_blob, h_plan);
-    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
-    BitVec marks;
-    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
-    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
-    marks.len = h_ssa->n;
-    prof::Scope ps(st, prof::LOCATE, 0);
-    locate_rows_kernel<<<(uint32_t)((m + 255) / 256), 256, 0, st>>>(
-        wt, marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), h_ssa->rate, row0, d_rows, m,
-        d_out_pos);
-    HK_LAUNCH_CHECK();
-    return HKCSA_OK;
+    return locate_launch(make_wt_dev(d_wt_blob, h_plan), d_ssa_blob, h_ssa, row0, d_rows, m, d_out_pos,
+                         as_stream(stream));
+}
+
+extern "C" int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
+                                     const hkcsa_occ_plan *p, const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa,
+                                     uint32_t row0, const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos,
+                                     void *stream)
+{
+    if (m == 0) return HKCSA_OK;
+    HK_REQUIRE(d_wt_blob && h_wt && d_occ_blob && p && d_ssa_blob && h_ssa && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(p->n == h_wt->n && p->sigma == h_wt->sigma && h_ssa->n == p->n, HKCSA_EINVAL, "plans do not match");
+    HK_REQUIRE(row0 < p->n, HKCSA_EINVAL, "row0 (the row of suffix 0) out of range");
+    return with_occ_source(d_wt_blob, h_wt, d_occ_blob, p, [&](auto occ) {
+        return locate_launch(occ, d_ssa_blob, h_ssa, row0, d_rows, m, d_out_pos, as_stream(stream));
+    });
 }
 
 extern "C" int hkcsa_symbol_positions(const uint8_t *d_bwt, uint64_t n, uint32_t *d_pos, uint64_t *d_start,

@@ -30,20 +30,6 @@ __device__ __forceinline__ uint32_t ms_slice_of(const MultiDesc *d, uint64_t i)
     return s;
 }
 
-// rank walk with the node tables read from global memory (they are a few KB per slice and stay in L1/L2)
-__device__ __forceinline__ uint32_t ms_rank_local(const WtDev &w, uint32_t code, uint32_t p)
-{
-    const WtTables *t = w.tab;
-    const uint32_t dep = t->depth[code];
-    for (uint32_t l = 0; l < dep; ++l) {
-        const uint32_t ns = __ldg(&t->node_start[l][code]);
-        const uint32_t start = ns & NODE_START_MASK;
-        const uint32_t r1 = (uint32_t)bv_rank(w.level[l], (uint64_t)start + p) - __ldg(&t->node_ones[l][code]);
-        p = (ns & NODE_BIT_FLAG) ? r1 : (p - r1);
-    }
-    return p;
-}
-
 // occurrences of `byte` in global rows [0, i)
 __device__ __forceinline__ uint64_t ms_rank(const MultiDesc *d, uint32_t byte, uint64_t i)
 {
@@ -53,7 +39,7 @@ __device__ __forceinline__ uint64_t ms_rank(const MultiDesc *d, uint32_t byte, u
     uint32_t local = 0;
     if (code != 0xFFFFu) {
         const uint32_t p = (uint32_t)(i - d->start[s]);
-        local = (w.sigma == 1) ? p : ms_rank_local(w, code, p);
+        local = (w.sigma == 1) ? p : wt_rank_code(*w.tab, w, code, p);   // node tables from global memory
     }
     return d->cum[s][byte] + local;
 }
@@ -78,30 +64,10 @@ ms_count_kernel(const MultiDesc *__restrict__ d, const uint8_t *__restrict__ pat
     out_hi[p] = miss ? -1 : (int64_t)r - 1;
 }
 
-// access + rank inside one slice, tables from global memory
-__device__ __forceinline__ uint32_t ms_access_rank(const WtDev &w, uint32_t i, uint32_t &occ)
-{
-    const WtTables *t = w.tab;
-    uint32_t lo = 0, hi = w.sigma, p = i;
-    for (uint32_t l = 0; hi - lo > 1; ++l) {
-        const uint32_t mid = lo + (hi - lo) / 2;
-        const uint32_t start = __ldg(&t->node_start[l][lo]) & NODE_START_MASK;
-        const BitVec &v = w.level[l];
-        const uint64_t ia = (uint64_t)start + p;
-        const uint64_t ba = ia / HKCSA_BLOCK_BITS;
-        const uint32_t o = (uint32_t)(ia - ba * HKCSA_BLOCK_BITS);
-        const RankBlock q = load_block(v.blocks + ba);
-        const uint32_t r1 = (uint32_t)(v.super[ba / HKCSA_SUPER_BLOCKS] + (uint32_t)(q.w[0] & 0xFFFFFFFFu) +
-                                       block_rank(q, o)) - __ldg(&t->node_ones[l][lo]);
-        if (block_bit(q, o)) { p = r1; lo = mid; }
-        else { p -= r1; hi = mid; }
-    }
-    occ = p;
-    return lo;
-}
-
 // text position of global row j: LF walk across slices until a marked row.  The step is the exact one of
 // locate_rows_kernel (lf_fix, csrc/common.cuh) on global rows and byte symbols: slices number their codes apart.
+// Kept apart from locate_rows_kernel (fm_search.cu): one slice lookup per step serves both the mark test and the LF
+// step, and rows, C[] and positions are 64-bit.
 __global__ void __launch_bounds__(256)
 ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ rows, uint64_t m,
                  uint64_t *__restrict__ out)
@@ -115,7 +81,7 @@ ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ r
             const uint32_t s = ms_slice_of(d, row0);
             const WtDev &w = d->slice[s];
             uint32_t occ0;
-            const uint32_t code = ms_access_rank(w, (uint32_t)(row0 - d->start[s]), occ0);
+            const uint32_t code = wt_access_rank(*w.tab, w, (uint32_t)(row0 - d->start[s]), occ0);
             s_c0 = w.tab->sym_of_code[code];
             s_fix = (d->cum[s][s_c0] + occ0) != 0;
         }
@@ -128,13 +94,9 @@ ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ r
     while (true) {
         const uint32_t s = ms_slice_of(d, j);
         const uint32_t lj = (uint32_t)(j - d->start[s]);
-        const BitVec &mk = d->marks[s];
-        const uint64_t g = lj / HKCSA_BLOCK_BITS;
-        const uint32_t o = lj - (uint32_t)g * HKCSA_BLOCK_BITS;
-        const RankBlock b = load_block(mk.blocks + g);
-        if (block_bit(b, o)) {
-            const uint64_t r = mk.super[g / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu) + block_rank(b, o);
-            out[q] = (uint64_t)d->samples[s][r] * d->rate + steps;
+        uint64_t slot;
+        if (marked_slot(d->marks[s], lj, slot)) {
+            out[q] = (uint64_t)d->samples[s][slot] * d->rate + steps;
             return;
         }
         // with the exact step a walk meets a marked row within rate-1 steps on every text; the bound only keeps a
@@ -142,7 +104,7 @@ ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ r
         if (steps >= d->rate) { out[q] = HKCSA_NO_POSITION64; return; }
         const WtDev &w = d->slice[s];
         uint32_t occ;
-        const uint32_t code = ms_access_rank(w, lj, occ);
+        const uint32_t code = wt_access_rank(*w.tab, w, lj, occ);
         const uint32_t byte = w.tab->sym_of_code[code];
         j = d->C[byte] + lf_fix(d->cum[s][byte] + occ, byte, j, s_c0, row0, s_fix);
         ++steps;

@@ -20,6 +20,9 @@
 // search is bound by the rate of random requests, not by their size: tools/probes/sector_probe.cu).  Costs
 // 8 sigma bytes per 32 rows (24 B per symbol for the 97-symbol text); the blob ends with a copy of the BWT for
 // the LF steps of locate.
+//
+// This file builds the table; the rank and LF steps that read it are OccDev (occ.cuh), the rank source the query
+// kernels of fm_search.cu and extract.cu are instantiated with.
 #include "common.cuh"
 #include "prof.cuh"
 #include "wavelet.cuh"
@@ -29,24 +32,6 @@ namespace hkcsa {
 
 constexpr int OCC_THREADS = 256;
 constexpr int OCC_SUB = 32;           // blocks per sub-chunk of a tile (4 per warp)
-
-struct OccDev {
-    const uint8_t *rows;
-    uint64_t stride;      // layout 0: bytes per row; layout 1: entries per code
-    const uint8_t *bwt;   // layout 1: the BWT copy at the end of the blob
-    uint32_t sigma;
-    uint32_t n;
-};
-
-// where the symbols / the counter of `code` live inside a row (B = symbols per row)
-__device__ __forceinline__ const uint8_t *occ_sym_ptr(const OccDev &o, uint32_t row)
-{
-    return o.rows + (uint64_t)row * o.stride;
-}
-__device__ __forceinline__ const uint32_t *occ_cnt_ptr(const uint8_t *sym, uint32_t code, uint32_t B)
-{
-    return reinterpret_cast<const uint32_t *>(sym + B) + code;
-}
 
 // ---------------------------------------------------------------- build
 // One CTA per WTL_TILE rows.  gpre[code][tile] (wt_tile_hist + wt_tile_scan) = occurrences before the tile.
@@ -103,57 +88,6 @@ occ_fill_kernel(const uint8_t *__restrict__ bwt, uint64_t n, const WtTables *__r
     }
 }
 
-// ---------------------------------------------------------------- rank
-// bit j of the result = (byte j of the block == ch), for the 2^SHIFT bytes held in x[]
-template <int SHIFT>
-__device__ __forceinline__ uint64_t occ_match_bits(const uint64_t (&x)[(1 << SHIFT) / 8], uint32_t ch4)
-{
-    uint64_t bits = 0;
-#pragma unroll
-    for (int v = 0; v < (1 << SHIFT) / 8; ++v) {
-        const uint32_t lo = __vcmpeq4((uint32_t)x[v], ch4) & 0x01010101u;           // 1 per equal byte
-        const uint32_t hi = __vcmpeq4((uint32_t)(x[v] >> 32), ch4) & 0x01010101u;
-        const uint32_t byte = ((lo * 0x01020408u) >> 24) | (((hi * 0x01020408u) >> 24) << 4);   // byte i -> bit i
-        bits |= (uint64_t)byte << (8 * v);
-    }
-    return bits;
-}
-// the row's symbols: one 256-bit load per 32 bytes (LDG.E.256).  (L1::no_allocate was measured: same L2 and DRAM
-// traffic, 60 % slower on the 2.8 GB table -- fewer requests in flight on that path.)
-template <int SHIFT>
-__device__ __forceinline__ void occ_load_row(const uint8_t *sym, uint64_t (&x)[(1 << SHIFT) / 8])
-{
-#pragma unroll
-    for (int v = 0; v < (1 << SHIFT) / 32; ++v) ld_nc_256(sym + 32 * v, x[4 * v], x[4 * v + 1], x[4 * v + 2], x[4 * v + 3]);
-}
-// occurrences of `ch` among the first t bytes (t < 2^SHIFT) of the row whose symbols start at `sym`
-template <int SHIFT>
-__device__ __forceinline__ uint32_t occ_count(const uint8_t *sym, uint32_t ch4, uint32_t t)
-{
-    uint64_t x[(1 << SHIFT) / 8];
-    occ_load_row<SHIFT>(sym, x);
-    return __popcll(occ_match_bits<SHIFT>(x, ch4) & ((1ull << t) - 1ull));
-}
-
-// both boundaries of a backward-search step: a <- occ(code, a), b <- occ(code, b).  The four loads (two
-// counters, two symbol blocks) are issued together whether or not the boundaries share a row: no divergent
-// paths inside the warp, one memory round trip per step (a shared row is served by the same sectors).
-template <int SHIFT>
-__device__ __forceinline__ void occ_rank2(const OccDev &o, uint32_t code, uint32_t ch, uint32_t &a, uint32_t &b)
-{
-    constexpr uint32_t B = 1u << SHIFT;
-    const uint32_t ch4 = ch * 0x01010101u;
-    const uint8_t *pa = occ_sym_ptr(o, a >> SHIFT);
-    const uint8_t *pb = occ_sym_ptr(o, b >> SHIFT);
-    const uint32_t base_a = __ldg(occ_cnt_ptr(pa, code, B));
-    const uint32_t base_b = __ldg(occ_cnt_ptr(pb, code, B));
-    uint64_t xa[B / 8], xb[B / 8];
-    occ_load_row<SHIFT>(pa, xa);
-    occ_load_row<SHIFT>(pb, xb);
-    a = base_a + __popcll(occ_match_bits<SHIFT>(xa, ch4) & ((1ull << (a & (B - 1))) - 1ull));
-    b = base_b + __popcll(occ_match_bits<SHIFT>(xb, ch4) & ((1ull << (b & (B - 1))) - 1ull));
-}
-
 // ---------------------------------------------------------------- layout 1: per-symbol bitmaps
 __global__ void __launch_bounds__(OCC_THREADS)
 occ_bitmap_fill_kernel(const uint8_t *__restrict__ bwt, uint64_t n, const WtTables *__restrict__ tab,
@@ -197,156 +131,6 @@ occ_bitmap_fill_kernel(const uint8_t *__restrict__ bwt, uint64_t n, const WtTabl
             if (lane == 0) s_base[c] = base + total;
         }
         __syncthreads();
-    }
-}
-
-// SHIFT = 0 selects the bitmap layout in the search kernels
-template <>
-__device__ __forceinline__ void occ_rank2<0>(const OccDev &o, uint32_t code, uint32_t ch, uint32_t &a, uint32_t &b)
-{
-    const uint2 *e = reinterpret_cast<const uint2 *>(o.rows) + (uint64_t)code * o.stride;
-    const uint2 ea = __ldg(e + (a >> 5));
-    const uint2 eb = __ldg(e + (b >> 5));           // the same entry once the range is narrow (merged in L1)
-    a = ea.x + __popc(ea.y & ((1u << (a & 31u)) - 1u));
-    b = eb.x + __popc(eb.y & ((1u << (b & 31u)) - 1u));
-}
-
-// Same search as fm_count_kernel (fm_search.cu): one lane per pattern, lanes refilled as patterns end;
-// find_range (csa/enhanced_fm_index.py:21-32) in half-open form.  Only the rank primitive differs.
-template <int SHIFT, int MIN_CTAS, bool PEERS>
-__global__ void __launch_bounds__(OCC_THREADS, MIN_CTAS)
-fm_count_occ_kernel(OccDev occ, const WtTables *__restrict__ tab, const uint8_t *__restrict__ pat,
-                    const int64_t *__restrict__ off, uint64_t P, int64_t *__restrict__ out_lo,
-                    int64_t *__restrict__ out_hi, const uint2 *__restrict__ kmer, uint32_t kk, PeerOut po)
-{
-    __shared__ uint32_t s_C[260];
-    __shared__ uint16_t s_code[256];
-    for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s_C[i] = tab->C[i];
-    for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s_code[i] = tab->code_of_sym[i];
-    __syncthreads();
-    const uint32_t n = occ.n;
-    const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
-    const uint64_t chunk = (P + nwarps - 1) / nwarps;
-    uint64_t next = min(P, warp * chunk);
-    const uint64_t end = min(P, next + chunk);
-
-    int64_t p = -1;
-    int64_t k = 0, b = 0;
-    uint32_t l = 0, r = 0;
-    uint32_t ch_next = 0;      // pat[k], loaded one step ahead so the step's rank loads do not wait for it
-    while (true) {
-        const uint32_t idle = __ballot_sync(0xffffffffu, p < 0);
-        if (idle) {
-            const uint64_t mine = next + __popc(idle & lanemask_lt());
-            if (p < 0 && mine < end) {
-                p = (int64_t)mine;
-                b = off[mine];
-                k = off[mine + 1] - 1;
-                l = 0;
-                r = n;
-                if (kmer != nullptr && k - b + 1 >= (int64_t)kk) {
-                    uint32_t id = 0;
-                    bool known = true;
-                    for (uint32_t t = 0; t < kk; ++t) {
-                        const uint32_t code = s_code[pat[k - kk + 1 + t]];
-                        known = known && code != 0xFFFFu;
-                        id = id * occ.sigma + (known ? code : 0u);
-                    }
-                    if (known) {
-                        const uint2 e2 = __ldg(kmer + id);
-                        l = e2.x;
-                        r = e2.y;
-                        k -= kk;
-                        if (l >= r) { l = 1; r = 0; k = b - 1; }
-                    }
-                }
-                if (k >= b) ch_next = pat[k];
-            }
-            next += __popc(idle);
-            if (idle == 0xffffffffu && __ballot_sync(0xffffffffu, p >= 0) == 0) break;
-        }
-        if (p < 0) continue;
-        bool done = k < b, miss = l >= r;
-        if (!done) {
-            const uint32_t ch = ch_next;
-            if (k > b) ch_next = pat[k - 1];
-            const uint32_t code = s_code[ch];
-            if (code == 0xFFFFu) { miss = true; }
-            else {
-                occ_rank2<SHIFT>(occ, code, ch, l, r);
-                const uint32_t c0 = s_C[code];
-                l += c0;
-                r += c0;
-                miss = l >= r;
-            }
-            --k;
-            done = miss || k < b;
-        }
-        if (done) {
-            put_range<PEERS>(po, out_lo, out_hi, p, miss ? -1 : (int64_t)l, miss ? -1 : (int64_t)r - 1);
-            p = -1;
-        }
-    }
-}
-
-// occ(bwt[j], j) from the Occ table, and the symbol's code
-template <int SHIFT>
-__device__ __forceinline__ uint32_t occ_step(const OccDev &occ, const uint16_t *s_code, uint32_t j, uint32_t &code)
-{
-    constexpr uint32_t B = 1u << SHIFT;
-    if (SHIFT == 0) {
-        const uint32_t ch = __ldg(occ.bwt + j);
-        code = s_code[ch];
-        const uint2 e = __ldg(reinterpret_cast<const uint2 *>(occ.rows) + (uint64_t)code * occ.stride + (j >> 5));
-        return e.x + __popc(e.y & ((1u << (j & 31u)) - 1u));
-    } else {
-        const uint32_t t = j & (B - 1);
-        const uint8_t *row = occ_sym_ptr(occ, j >> SHIFT);
-        const uint32_t ch = __ldg(row + t);
-        code = s_code[ch];
-        return __ldg(occ_cnt_ptr(row, code, B)) + occ_count<(SHIFT ? SHIFT : 5)>(row, ch * 0x01010101u, t);
-    }
-}
-
-// position of row j: LF walk until a marked row (locate_rows_kernel of fm_search.cu with the LF step read from
-// the Occ table: the symbol bwt[j] and its count before j come from the same row -- two sectors per step)
-template <int SHIFT>
-__global__ void __launch_bounds__(256)
-locate_rows_occ_kernel(OccDev occ, const WtTables *__restrict__ tab, BitVec marks, const uint32_t *__restrict__ samples,
-                       uint32_t rate, uint32_t row0, const uint32_t *__restrict__ rows, uint64_t m,
-                       uint32_t *__restrict__ out)
-{
-    __shared__ uint32_t s_C[260];
-    __shared__ uint16_t s_code[256];
-    __shared__ uint32_t s_c0, s_fix;
-    for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s_C[i] = tab->C[i];
-    for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s_code[i] = tab->code_of_sym[i];
-    __syncthreads();
-    if (threadIdx.x == 0) {             // c0 = bwt[row0]; the LF step needs lf_fix iff c0 occurs before row0
-        uint32_t c0;
-        s_fix = occ_step<SHIFT>(occ, s_code, row0, c0) != 0;
-        s_c0 = c0;
-    }
-    __syncthreads();
-    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= m) return;
-    uint32_t j = rows[q];
-    uint32_t steps = 0;
-    while (true) {
-        const uint64_t g = j / HKCSA_BLOCK_BITS;
-        const uint32_t o = j - (uint32_t)g * HKCSA_BLOCK_BITS;
-        const RankBlock b = load_block(marks.blocks + g);
-        if (block_bit(b, o)) {
-            const uint64_t r = marks.super[g / HKCSA_SUPER_BLOCKS] + (uint32_t)(b.w[0] & 0xFFFFFFFFu) + block_rank(b, o);
-            out[q] = samples[r] * rate + steps;
-            return;
-        }
-        if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }   // corrupt index only: see locate_rows_kernel
-        uint32_t code;
-        const uint32_t cnt = occ_step<SHIFT>(occ, s_code, j, code);
-        j = s_C[code] + lf_fix(cnt, code, j, s_c0, row0, s_fix);
-        ++steps;
     }
 }
 
@@ -417,124 +201,6 @@ extern "C" int hkcsa_occ_build(const void *d_wt_blob, const hkcsa_wt_plan *h_wt,
         occ_fill_kernel<5><<<grid, OCC_THREADS, smem, st>>>(d_bwt, n, d_tab, d_gcnt, tiles, p->sigma, p->stride, rows, p->rows);
     else
         occ_fill_kernel<6><<<grid, OCC_THREADS, smem, st>>>(d_bwt, n, d_tab, d_gcnt, tiles, p->sigma, p->stride, rows, p->rows);
-    HK_LAUNCH_CHECK();
-    return HKCSA_OK;
-}
-
-static int count_occ_launch(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
-                            const hkcsa_occ_plan *p, const void *d_kmer_table, uint32_t k, const uint8_t *d_pat,
-                            const int64_t *d_off, uint64_t P, int64_t *d_lo, int64_t *d_hi, const PeerOut &po,
-                            cudaStream_t st)
-{
-    HK_REQUIRE(p->n == h_wt->n && p->sigma == h_wt->sigma && p->n >= 1, HKCSA_EINVAL, "occ plan does not match the index");
-    const WtTables *d_tab = reinterpret_cast<const WtTables *>(static_cast<const uint8_t *>(d_wt_blob) + h_wt->off_tables);
-    OccDev occ;
-    occ.rows = static_cast<const uint8_t *>(d_occ_blob);
-    occ.stride = p->stride;
-    occ.bwt = occ.rows + p->off_bwt;
-    occ.sigma = p->sigma;
-    occ.n = (uint32_t)p->n;
-    const uint2 *kmer = static_cast<const uint2 *>(d_kmer_table);
-    const uint32_t kk = kmer ? k : 0u;
-    prof::Scope ps(st, prof::COUNT, 0);
-    // 4 CTAs/SM (53 registers): measured best of 4 / 5 / 6 / 8 on the 2.8 GB table (more lanes in flight were slower)
-    const int blocks = (int)std::min<uint64_t>((P + OCC_THREADS - 1) / OCC_THREADS, (uint64_t)num_sms() * 8);
-#define OCC_COUNT(SH, MC, GRID)                                                                                         \
-    do {                                                                                                                \
-        if (po.n) fm_count_occ_kernel<SH, MC, true><<<GRID, OCC_THREADS, 0, st>>>(occ, d_tab, d_pat, d_off, P, d_lo, d_hi, kmer, kk, po);  \
-        else fm_count_occ_kernel<SH, MC, false><<<GRID, OCC_THREADS, 0, st>>>(occ, d_tab, d_pat, d_off, P, d_lo, d_hi, kmer, kk, po);      \
-    } while (0)
-    if (p->layout == 1) {
-        // lanes in flight: DRAM-resident tables run best at 4 CTAs/SM, tables near the L2 size at 6 (measured:
-        // 1.42 vs 1.34 G patterns/s on the 4.8 GB table of the 200 MB text, 3.4 vs 4.0 on the 225 MB DNA table)
-        const int ctas = (p->blob_bytes > (1ull << 30)) ? 4 : 6;
-        const int blocks1 = (int)std::min<uint64_t>((P + OCC_THREADS - 1) / OCC_THREADS, (uint64_t)num_sms() * 2 * ctas);
-        if (ctas == 6) OCC_COUNT(0, 6, blocks1);
-        else OCC_COUNT(0, 4, blocks1);
-    } else if (p->shift == 5) {
-        OCC_COUNT(5, 4, blocks);
-    } else {
-        OCC_COUNT(6, 4, blocks);
-    }
-#undef OCC_COUNT
-    HK_LAUNCH_CHECK();
-    return HKCSA_OK;
-}
-
-extern "C" int hkcsa_count_batch_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
-                                     const hkcsa_occ_plan *p, const void *d_kmer_table, uint32_t k,
-                                     const uint8_t *d_pat, const int64_t *d_off, uint64_t P, int64_t *d_lo,
-                                     int64_t *d_hi, void *stream)
-{
-    HK_REQUIRE(d_wt_blob && h_wt && d_occ_blob && p, HKCSA_EINVAL, "null pointer");
-    if (P == 0) return HKCSA_OK;
-    HK_REQUIRE(d_off && d_lo && d_hi, HKCSA_EINVAL, "null pointer");
-    PeerOut po;
-    memset(&po, 0, sizeof(po));
-    return count_occ_launch(d_wt_blob, h_wt, d_occ_blob, p, d_kmer_table, k, d_pat, d_off, P, d_lo, d_hi, po, as_stream(stream));
-}
-
-extern "C" int hkcsa_count_batch_peers(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
-                                       const hkcsa_occ_plan *h_occ, const void *d_kmer_table, uint32_t k,
-                                       const uint8_t *d_pat, const int64_t *d_off, uint64_t P, uint64_t out_base,
-                                       uint32_t n_peers, const uint64_t *h_peer_lo, const uint64_t *h_peer_hi, void *stream)
-{
-    HK_REQUIRE(d_wt_blob && h_wt && h_peer_lo && h_peer_hi, HKCSA_EINVAL, "null pointer");
-    HK_REQUIRE(n_peers >= 1 && n_peers <= HKCSA_MAX_PEERS, HKCSA_EINVAL, "n_peers must be in [1, HKCSA_MAX_PEERS]");
-    HK_REQUIRE((d_occ_blob == nullptr) == (h_occ == nullptr), HKCSA_EINVAL, "occ blob and plan go together");
-    if (P == 0) return HKCSA_OK;
-    HK_REQUIRE(d_off != nullptr, HKCSA_EINVAL, "null pointer");
-    HK_REQUIRE(h_wt->n >= 1, HKCSA_EINVAL, "empty index");
-    PeerOut po;
-    memset(&po, 0, sizeof(po));
-    po.n = n_peers;
-    po.base = out_base;
-    for (uint32_t r = 0; r < n_peers; ++r) {
-        HK_REQUIRE(h_peer_lo[r] && h_peer_hi[r], HKCSA_EINVAL, "null peer pointer");
-        po.lo[r] = reinterpret_cast<int64_t *>(static_cast<uintptr_t>(h_peer_lo[r]));
-        po.hi[r] = reinterpret_cast<int64_t *>(static_cast<uintptr_t>(h_peer_hi[r]));
-    }
-    cudaStream_t st = as_stream(stream);
-    if (d_occ_blob)
-        return count_occ_launch(d_wt_blob, h_wt, d_occ_blob, h_occ, d_kmer_table, k, d_pat, d_off, P, nullptr, nullptr, po, st);
-    return count_wt_launch(make_wt_dev(d_wt_blob, h_wt), static_cast<const uint2 *>(d_kmer_table), k, d_pat, d_off, P,
-                           nullptr, nullptr, po, st);
-}
-
-extern "C" int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan *h_wt, const void *d_occ_blob,
-                                     const hkcsa_occ_plan *p, const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa,
-                                     uint32_t row0, const uint32_t *d_rows, uint64_t m, uint32_t *d_out_pos,
-                                     void *stream)
-{
-    if (m == 0) return HKCSA_OK;
-    HK_REQUIRE(d_wt_blob && h_wt && d_occ_blob && p && d_ssa_blob && h_ssa && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
-    HK_REQUIRE(p->n == h_wt->n && p->sigma == h_wt->sigma && h_ssa->n == p->n, HKCSA_EINVAL, "plans do not match");
-    HK_REQUIRE(row0 < p->n, HKCSA_EINVAL, "row0 (the row of suffix 0) out of range");
-    cudaStream_t st = as_stream(stream);
-    const WtTables *d_tab = reinterpret_cast<const WtTables *>(static_cast<const uint8_t *>(d_wt_blob) + h_wt->off_tables);
-    OccDev occ;
-    occ.rows = static_cast<const uint8_t *>(d_occ_blob);
-    occ.stride = p->stride;
-    occ.bwt = occ.rows + p->off_bwt;
-    occ.sigma = p->sigma;
-    occ.n = (uint32_t)p->n;
-    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
-    BitVec marks;
-    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
-    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
-    marks.len = h_ssa->n;
-    const uint32_t *samples = reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples);
-    const uint32_t grid = (uint32_t)((m + 255) / 256);
-    prof::Scope ps(st, prof::LOCATE, 0);
-    if (p->layout == 1)
-        locate_rows_occ_kernel<0><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
-                                                            d_out_pos);
-    else if (p->shift == 5)
-        locate_rows_occ_kernel<5><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
-                                                            d_out_pos);
-    else
-        locate_rows_occ_kernel<6><<<grid, 256, 0, st>>>(occ, d_tab, marks, samples, h_ssa->rate, row0, d_rows, m,
-                                                            d_out_pos);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }

@@ -2,6 +2,7 @@
 // the build kernels (wavelet.cu) and the FM search kernels (fm_search.cu).
 #pragma once
 #include "common.cuh"
+#include <type_traits>
 
 namespace hkcsa {
 
@@ -30,12 +31,34 @@ struct WtTables {
     uint16_t code_of_path[256];                 // 0xFFFF: no symbol has this path
 };
 
+// What one LF step reads at row j of a rank source: the code of bwt[j], its byte, and occ(code, j).
+struct LfStep {
+    uint32_t code, sym, occ;
+};
+
+// Shared-memory copy of what a symbol-rank walk needs ("C[] held in shared memory").
+struct WtSmem {
+    uint32_t node_start[HKCSA_MAX_LEVELS][256];
+    uint32_t node_ones[HKCSA_MAX_LEVELS][256];
+    uint32_t C[260];
+    uint16_t code_of_sym[256];
+    uint8_t depth[256];
+    uint8_t sym_of_code[256];
+};
+
+// The tree as seen by device code; also the wavelet-tree rank source of the query kernels (fm_search.cu, extract.cu),
+// which use load / rank2 / step with the tables in shared memory.
 struct WtDev {
     const WtTables *tab;
     BitVec level[HKCSA_MAX_LEVELS];
     uint32_t levels;
     uint32_t sigma;
     uint64_t n;
+
+    using Smem = WtSmem;
+    __device__ void load(WtSmem &s) const;
+    __device__ void rank2(const WtSmem &s, uint32_t code, uint32_t ch, uint32_t &a, uint32_t &b) const;
+    __device__ LfStep step(const WtSmem &s, uint32_t j) const;
 };
 
 static inline uint64_t rank_blocks_for(uint64_t bits) { return bits / HKCSA_BLOCK_BITS + 1; }
@@ -89,18 +112,6 @@ __device__ __forceinline__ void put_range(const PeerOut &po, int64_t *out_lo, in
         }
     }
 }
-int count_wt_launch(const WtDev &wt, const uint2 *kmer, uint32_t k, const uint8_t *d_pat, const int64_t *d_off, uint64_t P,
-                    int64_t *d_lo, int64_t *d_hi, const PeerOut &po, cudaStream_t st);
-
-// Shared-memory copy of what a symbol-rank walk needs ("C[] held in shared memory").
-struct WtSmem {
-    uint32_t node_start[HKCSA_MAX_LEVELS][256];
-    uint32_t node_ones[HKCSA_MAX_LEVELS][256];
-    uint32_t C[260];
-    uint16_t code_of_sym[256];
-    uint8_t depth[256];
-    uint8_t sym_of_code[256];
-};
 
 __device__ __forceinline__ void wt_smem_load(WtSmem &s, const WtDev &wt)
 {
@@ -117,15 +128,25 @@ __device__ __forceinline__ void wt_smem_load(WtSmem &s, const WtDev &wt)
     }
 }
 
+// Reads of the descent tables: WtSmem is in shared memory; WtTables is the copy in global memory (the sliced index
+// of multi_slice.cu), read through the read-only path.
+template <typename Tab, typename T>
+__device__ __forceinline__ T wt_ld(const T &x)
+{
+    if constexpr (std::is_same_v<Tab, WtTables>) return __ldg(&x);
+    else return x;
+}
+
 // occ(code, i) = occurrences of `code` in the sequence before position i.
-__device__ __forceinline__ uint32_t wt_rank_code(const WtSmem &s, const WtDev &wt, uint32_t code, uint32_t i)
+template <typename Tab>
+__device__ __forceinline__ uint32_t wt_rank_code(const Tab &t, const WtDev &wt, uint32_t code, uint32_t i)
 {
     uint32_t p = i;
-    const uint32_t dep = s.depth[code];
+    const uint32_t dep = t.depth[code];
     for (uint32_t l = 0; l < dep; ++l) {
-        const uint32_t ns = s.node_start[l][code];
+        const uint32_t ns = wt_ld<Tab>(t.node_start[l][code]);
         const uint32_t start = ns & NODE_START_MASK;
-        const uint32_t r1 = (uint32_t)bv_rank(wt.level[l], (uint64_t)start + p) - s.node_ones[l][code];
+        const uint32_t r1 = (uint32_t)bv_rank(wt.level[l], (uint64_t)start + p) - wt_ld<Tab>(t.node_ones[l][code]);
         p = (ns & NODE_BIT_FLAG) ? r1 : (p - r1);
     }
     return p;
@@ -157,24 +178,39 @@ __device__ __forceinline__ void wt_rank_code2(const WtSmem &s, const WtDev &wt, 
 }
 
 // access + rank in one descent: code at position i and occ(code, i).
-__device__ __forceinline__ uint32_t wt_access_rank(const WtSmem &s, const WtDev &wt, uint32_t i, uint32_t &occ)
+template <typename Tab>
+__device__ __forceinline__ uint32_t wt_access_rank(const Tab &t, const WtDev &wt, uint32_t i, uint32_t &occ)
 {
     uint32_t lo = 0, hi = wt.sigma, p = i;
     for (uint32_t l = 0; hi - lo > 1; ++l) {
         const uint32_t mid = lo + (hi - lo) / 2;
-        const uint32_t start = s.node_start[l][lo] & NODE_START_MASK;
+        const uint32_t start = wt_ld<Tab>(t.node_start[l][lo]) & NODE_START_MASK;
         const BitVec &v = wt.level[l];
         const uint64_t ia = (uint64_t)start + p;
         const uint64_t ba = ia / HKCSA_BLOCK_BITS;
         const uint32_t o = (uint32_t)(ia - ba * HKCSA_BLOCK_BITS);
         const RankBlock q = load_block(v.blocks + ba);
         const uint32_t r1 = (uint32_t)(v.super[ba / HKCSA_SUPER_BLOCKS] + (uint32_t)(q.w[0] & 0xFFFFFFFFu) +
-                                       block_rank(q, o)) - s.node_ones[l][lo];
+                                       block_rank(q, o)) - wt_ld<Tab>(t.node_ones[l][lo]);
         if (block_bit(q, o)) { p = r1; lo = mid; }
         else { p -= r1; hi = mid; }
     }
     occ = p;
     return lo;
+}
+
+__device__ __forceinline__ void WtDev::load(WtSmem &s) const { wt_smem_load(s, *this); }
+// with one symbol the depth is 0: the descent keeps both boundaries
+__device__ __forceinline__ void WtDev::rank2(const WtSmem &s, uint32_t code, uint32_t, uint32_t &a, uint32_t &b) const
+{
+    wt_rank_code2(s, *this, code, a, b);
+}
+__device__ __forceinline__ LfStep WtDev::step(const WtSmem &s, uint32_t j) const
+{
+    LfStep t;
+    t.code = wt_access_rank(s, *this, j, t.occ);
+    t.sym = s.sym_of_code[t.code];
+    return t;
 }
 
 }  // namespace hkcsa
