@@ -53,20 +53,16 @@ __device__ __forceinline__ uint32_t dsa_dest_of(const uint32_t *cuts, uint32_t w
 // MODE 1: (key, id) of every suffix of [begin, end) stored into the receive arrays of the rank owning its bucket.
 // MODE 2: suffixes of [begin, end) per destination rank (counters[d]): the exact region sizes of the exchange when
 //         the cut points came from a sampled histogram.
-// Keys are produced exactly as in sa_pack0_kernel (code words of the tile in one shared bit stream, key = the
-// 64-bit window at the symbol's bit offset), so both modes and the single-GPU builder agree on every key.
+// Keys come from the same key source as the single-GPU builder's (AlphaKeys), so every mode and both builders agree on
+// every key.
 template <int MODE, bool WIDE>
 __global__ void __launch_bounds__(PACK_THREADS, 4)
-dsa_pack_kernel(const uint8_t *__restrict__ text, uint64_t n, uint64_t begin, uint64_t end, AlphaCode ac, int bits,
+dsa_pack_kernel(const uint8_t *__restrict__ text, uint64_t n, uint64_t begin, uint64_t end, AlphaKeys src, int bits,
                 DsaDest dd, unsigned long long *__restrict__ counters, unsigned long long *__restrict__ bucket_hist,
                 uint32_t tile_stride, int xbits = 0)
 {
     using IdT = typename std::conditional<WIDE, uint64_t, uint32_t>::type;
-    __shared__ __align__(16) uint16_t s_off[PACK_TILE];
-    __shared__ uint32_t s_stream[PACK_STREAM_WORDS];
-    __shared__ uint32_t s_tab[257];
-    __shared__ uint32_t s_tot[PACK_VT + 24];
-    __shared__ __align__(16) uint16_t s_off_look[PACK_IPT];
+    __shared__ AlphaKeys::Smem s;
     __shared__ uint32_t s_cnt[DSA_MAX_WORLD], s_first[DSA_MAX_WORLD + 1], s_cuts[DSA_MAX_WORLD + 1];
     __shared__ uint64_t s_gbase[DSA_MAX_WORLD];
     __shared__ uint64_t *s_kptr[DSA_MAX_WORLD];
@@ -74,9 +70,7 @@ dsa_pack_kernel(const uint8_t *__restrict__ text, uint64_t n, uint64_t begin, ui
     __shared__ __align__(16) uint64_t s_keys[MODE == 1 ? PACK_TILE : 1];
     __shared__ __align__(16) IdT s_ids[MODE == 1 ? PACK_TILE : 1];
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    for (uint32_t i = tid; i < 257; i += PACK_THREADS) s_tab[i] = (ac.code[i] << 8) | ac.len[i];
-    for (uint32_t i = tid; i < PACK_STREAM_WORDS; i += PACK_THREADS) s_stream[i] = 0;
-    if (tid < 24) s_tot[PACK_VT + tid] = 0;
+    src.setup(s);
     if (tid < DSA_MAX_WORLD) {
         s_cnt[tid] = 0;
         s_kptr[tid] = dd.keys[tid];
@@ -86,24 +80,7 @@ dsa_pack_kernel(const uint8_t *__restrict__ text, uint64_t n, uint64_t begin, ui
     __syncthreads();
     const uint64_t base = begin + (uint64_t)blockIdx.x * tile_stride * PACK_TILE;
     const bool aligned8 = (reinterpret_cast<uintptr_t>(text + base) & 7) == 0;
-    uint32_t cl[PACK_IPT], cl2[PACK_IPT];
-    s_tot[tid] = pack_load8(text, n, base + (uint64_t)tid * PACK_IPT, aligned8, s_tab, cl);
-    if (tid < PACK_LOOK / PACK_IPT)
-        s_tot[PACK_THREADS + tid] = pack_load8(text, n, base + PACK_TILE + (uint64_t)tid * PACK_IPT, aligned8, s_tab, cl2);
-    __syncthreads();
-    if (warp == 0) {                                            // exclusive scan of the 264 group lengths
-        uint32_t v[9], sum = 0;
-#pragma unroll
-        for (int q = 0; q < 9; ++q) { v[q] = s_tot[lane * 9 + q]; sum += v[q]; }
-        uint32_t total;
-        uint32_t run = warp_excl_sum(sum, total);
-#pragma unroll
-        for (int q = 0; q < 9; ++q) { s_tot[lane * 9 + q] = run; run += v[q]; }
-    }
-    __syncthreads();
-    pack_emit8(s_stream, s_off + tid * PACK_IPT, s_tot[tid], cl);
-    if (tid < PACK_LOOK / PACK_IPT) pack_emit8(s_stream, s_off_look, s_tot[PACK_THREADS + tid], cl2);
-    __syncthreads();
+    src.fill(s, text, n, base, aligned8);
     uint64_t key[PACK_IPT];
     uint32_t ds[PACK_IPT];            // MODE 1: destination << 16 | slot among the tile's elements for that destination
     uint16_t xk[MODE == 1 && WIDE ? PACK_IPT : 1];      // the WIDE_X_BITS code-stream bits that follow the key
@@ -112,20 +89,12 @@ dsa_pack_kernel(const uint8_t *__restrict__ text, uint64_t n, uint64_t begin, ui
     for (int e = 0; e < PACK_IPT; ++e) {
         const uint32_t j = warp * (32u * PACK_IPT) + e * 32u + lane;
         const uint64_t g = base + j;
-        const uint32_t o = s_off[j];
-        const uint32_t wi = o >> 5, sh = o & 31u;
-        const uint32_t w0 = s_stream[wi], w1 = s_stream[wi + 1], w2 = s_stream[wi + 2];
-        const uint32_t hi = __funnelshift_l(w1, w0, sh), lo = __funnelshift_l(w2, w1, sh);
-        key[e] = (((uint64_t)hi << 32) | lo) >> (64 - bits);
-        if (MODE == 1 && WIDE) {
-            // 64-bit ids leave room: the next 16 bits of the same code stream travel in the id word, so the group
-            // round tells most tied suffixes apart without touching the text (xbits = 0: the look-ahead of the
-            // stream does not reach that far for 1-bit code words -- the field stays zero, everything ties)
-            const uint32_t ex = __funnelshift_l(s_stream[wi + 3], w2, sh);
-            const uint64_t rest = bits < 64 ? ((((uint64_t)hi << 32) | lo) << bits) | (((uint64_t)ex << 32) >> (64 - bits))
-                                            : ((uint64_t)ex << 32);
-            xk[e] = xbits ? (uint16_t)(rest >> (64 - WIDE_X_BITS)) : (uint16_t)0;
-        }
+        // 64-bit ids leave room: the next 16 bits of the same code stream travel in the id word, so the group round
+        // tells most tied suffixes apart without touching the text (xbits = 0: the look-ahead of the stream does not
+        // reach that far for 1-bit code words -- the field stays zero, everything ties)
+        uint16_t x = 0;
+        key[e] = src.window(s, j, bits, MODE == 1 && WIDE ? &x : nullptr) >> (64 - bits);
+        if (MODE == 1 && WIDE) xk[e] = xbits ? x : (uint16_t)0;
         const bool valid = g < end;
         const uint32_t bucket = (uint32_t)(key[e] >> (bits - DSA_BUCKET_BITS));
         if (MODE == 0) {
@@ -260,12 +229,9 @@ __device__ __forceinline__ bool suffix_less(const uint8_t *__restrict__ text, ui
 // comparison is decided by the symbols before that depth whatever member sits in the slot.
 template <bool WIDE>
 __device__ uint64_t dsa_remote_rank(const DsaPeers &pp, const uint8_t *__restrict__ text, uint64_t n, uint64_t t,
-                                    const uint32_t *s_code, const uint8_t *s_len)
+                                    const AlphaKeys::Tab &s_tab)
 {
-    const uint32_t bucket = (uint32_t)alpha_pack(s_code, s_len, DSA_BUCKET_BITS, [&](int q) {
-        const uint64_t g = t + q;
-        return g < n ? (uint32_t)text[g] : 256u;
-    });
+    const uint32_t bucket = (uint32_t)AlphaKeys::at(s_tab, text, n, t, DSA_BUCKET_BITS);
     const uint32_t r = dsa_dest_of(pp.cuts, pp.world, bucket);
     const uint32_t *sa = pp.sa[r];
     uint64_t lo = 0, hi = pp.slice_off[r + 1] - pp.slice_off[r];
@@ -288,9 +254,8 @@ dsa_keybuild_dbl_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__res
                         uint32_t *__restrict__ ghist)
 {
     __shared__ uint32_t s_hist[8 * RADIX];
-    __shared__ uint32_t s_code[257];
-    __shared__ uint8_t s_len[257];
-    for (uint32_t i = threadIdx.x; i < 257; i += blockDim.x) { s_code[i] = ac.code[i]; s_len[i] = ac.len[i]; }
+    __shared__ AlphaKeys::Tab s_tab;
+    s_tab.load(ac);
     hist_zero(s_hist, passes);
     __syncthreads();
     for (uint64_t base = (uint64_t)blockIdx.x * blockDim.x; base < m; base += (uint64_t)gridDim.x * blockDim.x) {
@@ -304,7 +269,7 @@ dsa_keybuild_dbl_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__res
             if (t < n) {
                 const uint64_t owner = t / pp.blk;
                 const IsaT v = ld_sys(static_cast<const IsaT *>(pp.isa[owner]) + (t - owner * pp.blk));
-                k2 = (v == (IsaT)~(IsaT)0 ? dsa_remote_rank<WIDE>(pp, text, n, t, s_code, s_len) : (uint64_t)v) + 1ull;
+                k2 = (v == (IsaT)~(IsaT)0 ? dsa_remote_rank<WIDE>(pp, text, n, t, s_tab) : (uint64_t)v) + 1ull;
             }
             key = ((uint64_t)cgrp[j] << b2) | k2;
             keys[j] = key;
@@ -517,7 +482,7 @@ extern "C" int hkcsa_dsa_plan_make(const uint64_t *h_byte_hist, uint64_t n, int 
     HK_REQUIRE(n <= (1ull << 40), HKCSA_ERANGE, "n exceeds 2^40");
     memset(p, 0, sizeof(*p));
     static thread_local Round0Plan r0;
-    make_round0_plan(h_byte_hist, r0);
+    if (int rc = plan_round0(h_byte_hist, r0)) return rc;
     p->n = n;
     p->sigma = r0.sigma;
     p->bits0 = (uint32_t)r0.bits0;
@@ -539,6 +504,14 @@ static void plan_codes(const hkcsa_dsa_plan *p, AlphaCode &ac, CodeMap *map)
     if (map) memcpy(map->code, p->fixed_code, sizeof(map->code));
 }
 
+// the round-0 key source of plan p.  max_len = PACK_MAX_LEN: a tile clears its whole stream, because the key
+// extension bits read the stream words behind the last code word.
+static void plan_keys(const hkcsa_dsa_plan *p, AlphaKeys &src)
+{
+    plan_codes(p, src.code, nullptr);
+    src.max_len = PACK_MAX_LEN;
+}
+
 // tile_stride > 1: only every tile_stride-th tile of 2048 positions is counted (cut points from a sample; the exact
 // region sizes then come from hkcsa_dsa_dest_counts)
 extern "C" int hkcsa_dsa_bucket_hist_sampled(const uint8_t *d_text, const hkcsa_dsa_plan *p, uint64_t begin, uint64_t end,
@@ -549,15 +522,15 @@ extern "C" int hkcsa_dsa_bucket_hist_sampled(const uint8_t *d_text, const hkcsa_
     cudaStream_t st = as_stream(stream);
     HK_CUDA(cudaMemsetAsync(d_hist, 0, (size_t)HKCSA_DSA_BUCKETS * sizeof(uint64_t), st));
     if (begin == end) return HKCSA_OK;
-    static thread_local AlphaCode ac;
-    plan_codes(p, ac, nullptr);
+    static thread_local AlphaKeys src;
+    plan_keys(p, src);
     DsaDest dd;
     memset(&dd, 0, sizeof(dd));
     const uint64_t tiles = (end - begin + PACK_TILE - 1) / PACK_TILE;
     const uint64_t blocks = (tiles + tile_stride - 1) / tile_stride;
     HK_REQUIRE(blocks <= 0x7FFFFFFFull, HKCSA_ERANGE, "block of positions too large for one launch");
     prof::Scope ps(st, prof::SA_PACK0, (end - begin) / tile_stride);
-    dsa_pack_kernel<0, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, ac, (int)p->bits0, dd,
+    dsa_pack_kernel<0, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, src, (int)p->bits0, dd,
                                                                        nullptr,
                                                                        reinterpret_cast<unsigned long long *>(d_hist),
                                                                        tile_stride);
@@ -582,8 +555,8 @@ extern "C" int hkcsa_dsa_dest_counts(const uint8_t *d_text, const hkcsa_dsa_plan
     cudaStream_t st = as_stream(stream);
     HK_CUDA(cudaMemsetAsync(d_counts, 0, DSA_MAX_WORLD * sizeof(uint64_t), st));
     if (begin == end) return HKCSA_OK;
-    static thread_local AlphaCode ac;
-    plan_codes(p, ac, nullptr);
+    static thread_local AlphaKeys src;
+    plan_keys(p, src);
     DsaDest dd;
     memset(&dd, 0, sizeof(dd));
     for (uint32_t r = 0; r <= world; ++r) dd.cuts[r] = h_cuts[r];
@@ -591,7 +564,7 @@ extern "C" int hkcsa_dsa_dest_counts(const uint8_t *d_text, const hkcsa_dsa_plan
     const uint64_t blocks = (end - begin + PACK_TILE - 1) / PACK_TILE;
     HK_REQUIRE(blocks <= 0x7FFFFFFFull, HKCSA_ERANGE, "block of positions too large for one launch");
     prof::Scope ps(st, prof::SA_PACK0, end - begin);
-    dsa_pack_kernel<2, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, ac, (int)p->bits0, dd,
+    dsa_pack_kernel<2, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, src, (int)p->bits0, dd,
                                                                        reinterpret_cast<unsigned long long *>(d_counts),
                                                                        nullptr, 1);
     HK_LAUNCH_CHECK();
@@ -610,8 +583,8 @@ extern "C" int hkcsa_dsa_pack_exchange(const uint8_t *d_text, const hkcsa_dsa_pl
     cudaStream_t st = as_stream(stream);
     HK_CUDA(cudaMemsetAsync(d_counters, 0, DSA_MAX_WORLD * sizeof(uint64_t), st));
     if (begin == end) return HKCSA_OK;
-    static thread_local AlphaCode ac;
-    plan_codes(p, ac, nullptr);
+    static thread_local AlphaKeys src;
+    plan_keys(p, src);
     DsaDest dd;
     memset(&dd, 0, sizeof(dd));
     for (uint32_t r = 0; r < world; ++r) {
@@ -629,13 +602,13 @@ extern "C" int hkcsa_dsa_pack_exchange(const uint8_t *d_text, const hkcsa_dsa_pl
     unsigned long long *cnt = reinterpret_cast<unsigned long long *>(d_counters);
     // the stream of a tile reaches PACK_LOOK positions beyond it: 64 + WIDE_X_BITS bits exist for every position when
     // no code word is shorter than two bits
-    int min_len = ac.len[256];                                  // past the end, then the bytes that occur
-    for (int c = 0; c < 256; ++c) if (p->fixed_code[c] && ac.len[c] < min_len) min_len = ac.len[c];
+    int min_len = src.code.len[256];                            // past the end, then the bytes that occur
+    for (int c = 0; c < 256; ++c) if (p->fixed_code[c] && src.code.len[c] < min_len) min_len = src.code.len[c];
     const int xbits = (min_len >= 2 && !getenv("HKCSA_DSA_NO_XBITS")) ? WIDE_X_BITS : 0;
     if (p->wide)
-        dsa_pack_kernel<1, true><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, ac, (int)p->bits0, dd, cnt, nullptr, 1, xbits);
+        dsa_pack_kernel<1, true><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, src, (int)p->bits0, dd, cnt, nullptr, 1, xbits);
     else
-        dsa_pack_kernel<1, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, ac, (int)p->bits0, dd, cnt, nullptr, 1);
+        dsa_pack_kernel<1, false><<<(uint32_t)blocks, PACK_THREADS, 0, st>>>(d_text, p->n, begin, end, src, (int)p->bits0, dd, cnt, nullptr, 1);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }

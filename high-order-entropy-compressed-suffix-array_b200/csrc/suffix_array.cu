@@ -65,41 +65,6 @@ bool build_alpha_code(const uint64_t *h_hist, AlphaCode &ac, double &avg_len, in
     return true;
 }
 
-void make_round0_plan(const uint64_t *h_hist, Round0Plan &p, bool want_carry)
-{
-    uint32_t sigma = 0;
-    for (int ch = 0; ch < 256; ++ch)
-        if (h_hist[ch]) ++sigma;
-    const int b = std::max(1, (int)bits_for(sigma));   // fixed-width code size, for reference
-    // round-0 keys: the first bits0 bits of the alphabetic code stream; as many symbols on average as a
-    // fixed-width packing of 64 / b symbols would hold, in fewer bits when the symbol distribution allows
-    AlphaCode &ac = p.ac;
-    double avg_len = b;
-    int max_len = b;
-    if (!build_alpha_code(h_hist, ac, avg_len, max_len)) {
-        uint32_t code = 0;                               // degenerate distribution: fixed-width codes
-        ac.code[256] = 0; ac.len[256] = (uint8_t)b;
-        for (int ch = 0; ch < 256; ++ch)
-            if (h_hist[ch]) { ac.code[ch] = ++code; ac.len[ch] = (uint8_t)b; }
-        avg_len = max_len = b;
-    }
-    const int k_target = 64 / b;
-    int bits0 = 8 * (int)ceil(k_target * avg_len / 8.0 - 1e-9);
-    bits0 = std::max(16, std::min(64, bits0));
-    // HKCSA_CARRY56=1: a 64-bit plan settles for 56 bits so that the BWT symbol can ride in the top byte -- one radix
-    // pass less and no gather afterwards, but more survivors in round 1.  Measured on the 200 MB English-like text
-    // (C3): 21.4 M survivors instead of 5.1 M, 17.2 ms instead of 16.4 ms -- so it is off unless asked for.
-    const char *c56 = getenv("HKCSA_CARRY56");
-    if (want_carry && bits0 > 56 && c56 && atoi(c56)) bits0 = 56;
-    if (const char *e = getenv("HKCSA_BITS0")) bits0 = std::max(16, std::min(64, 8 * (atoi(e) / 8)));   // tuning knob
-    p.sigma = sigma;
-    p.b = b;
-    p.max_len = max_len;
-    p.bits0 = bits0;
-    p.k0 = std::max(1, bits0 / max_len);         // symbols every key is guaranteed to cover
-    p.passes0 = bits0 / 8;
-}
-
 // ---------------------------------------------------------------- byte histogram
 __global__ void byte_hist_kernel(const uint8_t *__restrict__ text, uint64_t n, unsigned long long *__restrict__ ghist)
 {
@@ -146,116 +111,6 @@ cudaError_t byte_hist(const uint8_t *d_text, uint64_t n, uint64_t *d_hist, cudaS
     return cudaGetLastError();
 }
 
-// ---------------------------------------------------------------- round 0: pack
-// key[i] = the first `bits` bits of code(T[i]) code(T[i+1]) ... (the last code word truncated).
-//
-// The CTA writes the code words of its 2048 positions + 64 look-ahead positions into ONE bit stream in shared
-// memory (each thread owns 8 consecutive symbols: it sums their code lengths, a block scan gives its bit
-// offset, and it ORs its bits in 32-bit pieces); the key of a position is then the 64-bit window of the stream
-// at that position's bit offset -- three shared loads and two funnel shifts, whatever the number of symbols
-// the key covers.  Keys are produced warp-striped so the stores are fully coalesced.  The suffix ids are not
-// written at all: the first radix pass takes "value = index" (radix_sort_pairs_u64, identity_vals).
-// PASSES = radix passes of round 0 = key bits / 8, a template parameter: the key shift and the digit histogram of
-// every pass (the bulk of the kernel's instructions: one shared atomic per key and pass) are straight-line code.
-// CARRY: the symbol before the suffix (its BWT symbol, csa/bwt.py:6-11) rides in the top byte of the key, above
-// the sorted bits (keys of at most 56 bits): the sort delivers the BWT in suffix-array order and nobody has to gather
-// text[SA[i] - 1] at random afterwards.
-template <int PASSES, bool CARRY>
-__global__ void __launch_bounds__(PACK_THREADS, 6)
-sa_pack0_kernel(const uint8_t *__restrict__ text, uint32_t n, AlphaCode ac, uint32_t max_len,
-                uint64_t *__restrict__ keys, uint32_t *__restrict__ ghist)
-{
-    static_assert(!CARRY || PASSES <= 7, "the carried symbol needs the top byte of the key");
-    constexpr int bits = 8 * PASSES, passes = PASSES;
-    __shared__ __align__(16) uint16_t s_off[PACK_TILE];
-    __shared__ uint32_t s_stream[PACK_STREAM_WORDS];
-    __shared__ uint32_t s_hist[8 * RADIX];
-    __shared__ uint32_t s_tab[257];
-    __shared__ uint32_t s_tot[PACK_VT + 24];                    // 288 = 32 lanes x 9
-    __shared__ __align__(16) uint16_t s_off_look[PACK_IPT];     // offsets of a look-ahead group: written, never read
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    for (uint32_t i = tid; i < 257; i += PACK_THREADS) s_tab[i] = (ac.code[i] << 8) | ac.len[i];
-    if (tid < 24) s_tot[PACK_VT + tid] = 0;
-    hist_zero(s_hist, passes);
-    const bool aligned8 = (reinterpret_cast<uintptr_t>(text) & 7) == 0;
-    // the stream words a tile can touch: (tile + look-ahead) symbols of at most max_len bits
-    const uint32_t stream_words = min((uint32_t)PACK_STREAM_WORDS, ((PACK_TILE + PACK_LOOK) * max_len + 31u) / 32u + 4u);
-    // a CTA takes every gridDim.x-th tile: the digit histograms leave shared memory once per CTA, not once per tile
-    // (1536 global atomics per 2048 keys otherwise: 0.55 -> 0.48 ms at C2), and the code table is set up once
-    const uint32_t tiles = (n + PACK_TILE - 1) / PACK_TILE;
-    for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    for (uint32_t i = tid; i < stream_words; i += PACK_THREADS) s_stream[i] = 0;
-    __syncthreads();
-    const uint64_t base = (uint64_t)tile * PACK_TILE;
-    uint32_t cl[PACK_IPT], cl2[PACK_IPT];
-    s_tot[tid] = pack_load8(text, n, base + (uint64_t)tid * PACK_IPT, aligned8, s_tab, cl);
-    if (tid < PACK_LOOK / PACK_IPT)
-        s_tot[PACK_THREADS + tid] = pack_load8(text, n, base + PACK_TILE + (uint64_t)tid * PACK_IPT, aligned8, s_tab, cl2);
-    __syncthreads();
-    if (warp == 0) {                                            // exclusive scan of the 264 group lengths
-        uint32_t v[9], sum = 0;
-#pragma unroll
-        for (int q = 0; q < 9; ++q) { v[q] = s_tot[lane * 9 + q]; sum += v[q]; }
-        uint32_t total;
-        uint32_t run = warp_excl_sum(sum, total);
-#pragma unroll
-        for (int q = 0; q < 9; ++q) { s_tot[lane * 9 + q] = run; run += v[q]; }
-    }
-    __syncthreads();
-    pack_emit8(s_stream, s_off + tid * PACK_IPT, s_tot[tid], cl);
-    if (tid < PACK_LOOK / PACK_IPT) pack_emit8(s_stream, s_off_look, s_tot[PACK_THREADS + tid], cl2);
-    __syncthreads();
-#pragma unroll
-    for (int e = 0; e < PACK_IPT; ++e) {
-        const uint32_t j = warp * (32u * PACK_IPT) + e * 32u + lane;
-        const uint64_t g = base + j;
-        const uint32_t o = s_off[j];
-        const uint32_t wi = o >> 5, sh = o & 31u;
-        const uint32_t w0 = s_stream[wi], w1 = s_stream[wi + 1], w2 = s_stream[wi + 2];
-        const uint32_t hi = __funnelshift_l(w1, w0, sh), lo = __funnelshift_l(w2, w1, sh);
-        const uint64_t key = (((uint64_t)hi << 32) | lo) >> (64 - bits);
-        const bool valid = g < n;
-        if (valid) {
-            if (CARRY) keys[g] = key | ((uint64_t)__ldg(text + (g ? g - 1 : (uint64_t)n - 1)) << 56);   // an L1 hit: the tile was just read
-            else keys[g] = key;
-        }
-        hist_add_key_unsorted<PASSES>(s_hist, key, valid);
-    }
-    __syncthreads();      // the next tile clears the stream
-    }
-    hist_flush(s_hist, ghist, passes);
-}
-
-// ---------------------------------------------------------------- round 0 keys from the k-gram code
-// digits of the 8 symbols a thread owns, as one 8-byte word (positions past the end: digit 0)
-__device__ __forceinline__ uint2 gram_digits8(const uint8_t *__restrict__ text, uint64_t n, uint64_t p0, bool aligned8,
-                                              const uint8_t *s_digit)
-{
-    uint32_t d[8];
-    if (aligned8 && p0 + 8 <= n) {
-        const uint2 a = __ldg(reinterpret_cast<const uint2 *>(text + p0));
-#pragma unroll
-        for (int e = 0; e < 8; ++e) d[e] = s_digit[((e < 4 ? a.x : a.y) >> (8 * (e & 3))) & 0xFFu];
-    } else {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) d[e] = (p0 + e < n) ? (uint32_t)s_digit[text[p0 + e]] : 0u;
-    }
-    return make_uint2(d[0] | (d[1] << 8) | (d[2] << 16) | (d[3] << 24), d[4] | (d[5] << 8) | (d[6] << 16) | (d[7] << 24));
-}
-
-// the grams starting at the 8 positions from j0 (digits in shared memory), by a rolling base-B number
-__device__ __forceinline__ void gram_roll8(const uint8_t *s_dig, uint32_t j0, uint32_t k, uint32_t B, uint32_t pw, uint32_t g[8])
-{
-    uint32_t cur = 0;
-    for (uint32_t q = 0; q < k; ++q) cur = cur * B + s_dig[j0 + q];
-    g[0] = cur;
-#pragma unroll
-    for (int e = 1; e < 8; ++e) {
-        cur = (cur - (uint32_t)s_dig[j0 + e - 1] * pw) * B + s_dig[j0 + e - 1 + k];
-        g[e] = cur;
-    }
-}
-
 // sampled k-gram histogram: CTA b counts the grams of tile b * stride (2048 positions) with global atomics
 __global__ void __launch_bounds__(PACK_THREADS)
 gram_hist_kernel(const uint8_t *__restrict__ text, uint32_t n, GramCode gc, uint32_t stride, uint32_t *__restrict__ gh)
@@ -268,11 +123,11 @@ gram_hist_kernel(const uint8_t *__restrict__ text, uint32_t n, GramCode gc, uint
     const uint64_t base = (uint64_t)blockIdx.x * stride * PACK_TILE;
     const bool aligned8 = (reinterpret_cast<uintptr_t>(text) & 7) == 0;
     const uint64_t p0 = base + (uint64_t)tid * PACK_IPT;
-    reinterpret_cast<uint2 *>(s_dig)[tid] = gram_digits8(text, n, p0, aligned8, s_digit);
-    if (tid < 2) reinterpret_cast<uint2 *>(s_dig)[PACK_THREADS + tid] = gram_digits8(text, n, base + PACK_TILE + tid * 8u, aligned8, s_digit);
+    reinterpret_cast<uint2 *>(s_dig)[tid] = GramKeys::digits8(s_digit, text, n, p0, aligned8);
+    if (tid < 2) reinterpret_cast<uint2 *>(s_dig)[PACK_THREADS + tid] = GramKeys::digits8(s_digit, text, n, base + PACK_TILE + tid * 8u, aligned8);
     __syncthreads();
     uint32_t g[8];
-    gram_roll8(s_dig, tid * PACK_IPT, gc.k, gc.B, gc.pw, g);
+    GramKeys::roll8(s_dig, tid * PACK_IPT, gc.k, gc.B, gc.pw, g);
 #pragma unroll
     for (int e = 0; e < 8; ++e)
         if (p0 + e < n) atomicAdd(&gh[g[e]], 1u);
@@ -394,89 +249,171 @@ gram_assign_kernel(const uint64_t *__restrict__ cum, const uint64_t *__restrict_
     }
 }
 
-// key[i] = the first `bits` bits of code(gram at i) code(gram at i + k) ...  Per tile: (1) the digits of the tile's
-// symbols (+ the look-ahead a key can reach) into shared memory; (2) the gram at every position by a rolling base-B
-// number, its table entry -- a 4-byte load whose hot part (the grams that occur: 16 KB for DNA) stays in L1 -- into
-// shared memory; (3) a key = the entries at i, i + k, i + 2k, ... OR-ed in at the bits consumed so far (the code word
-// sits left-aligned in the entry: one 64-bit shift per gram).  Persistent, digit histograms fused, BWT symbol in the
-// top byte as in sa_pack0_kernel.
-constexpr int GRAM_LOOK = GRAM_PER_KEY * GRAM_MAX_K;            // positions a key can reach beyond its own
-template <int PASSES, bool CARRY>
+int plan_round0(const uint64_t *h_hist, Round0Plan &p, const uint8_t *d_text, uint64_t n, const GramScratch *gs,
+                cudaStream_t st)
+{
+    const char *e_bits0 = getenv("HKCSA_BITS0");       // tuning knob: the key width
+    const char *e_gram = getenv("HKCSA_GRAM");
+    const int want_bits0 = e_bits0 ? 8 * (atoi(e_bits0) / 8) : 0;
+    uint32_t sigma = 0;
+    for (int ch = 0; ch < 256; ++ch)
+        if (h_hist[ch]) ++sigma;
+    const int b = std::max(1, (int)bits_for(sigma));   // fixed-width code size, for reference
+    // round-0 keys: the first bits0 bits of the alphabetic code stream; as many symbols on average as a
+    // fixed-width packing of 64 / b symbols would hold, in fewer bits when the symbol distribution allows
+    AlphaCode &ac = p.ac;
+    double avg_len = b;
+    int max_len = b;
+    if (!build_alpha_code(h_hist, ac, avg_len, max_len)) {
+        uint32_t code = 0;                               // degenerate distribution: fixed-width codes
+        ac.code[256] = 0; ac.len[256] = (uint8_t)b;
+        for (int ch = 0; ch < 256; ++ch)
+            if (h_hist[ch]) { ac.code[ch] = ++code; ac.len[ch] = (uint8_t)b; }
+        avg_len = max_len = b;
+    }
+    const int k_target = 64 / b;
+    int bits0 = 8 * (int)ceil(k_target * avg_len / 8.0 - 1e-9);
+    bits0 = std::max(16, std::min(64, bits0));
+    if (e_bits0) bits0 = std::max(16, std::min(64, want_bits0));
+    p.sigma = sigma;
+    p.b = b;
+    p.max_len = max_len;
+    p.bits0 = bits0;
+    p.k0 = std::max(1, bits0 / max_len);         // symbols every key is guaranteed to cover
+    p.passes0 = bits0 / 8;
+
+    // ---- the k-gram code (suffix_array.cuh): sampled gram histogram -> code built on the device -> its statistics
+    //      decide the key width.  Small texts and failures keep the per-symbol code above.
+    GramCode &gc = p.gram;
+    gc.tab = nullptr;
+    const uint32_t B = sigma + 1;
+    uint32_t k = 1, G = B;
+    while (k < (uint32_t)GRAM_MAX_K && (uint64_t)G * B <= (uint64_t)GRAM_MAX_G) { G *= B; ++k; }
+    if (!d_text || n < 1024 || k < (uint32_t)GRAM_MIN_K || (e_gram && atoi(e_gram) == 0)) return HKCSA_OK;
+    memset(gc.digit, 0, sizeof(gc.digit));
+    uint32_t dgt = 0;
+    for (int ch = 0; ch < 256; ++ch)
+        if (h_hist[ch]) gc.digit[ch] = (uint8_t)++dgt;      // k >= 4 means B <= 19
+    gc.k = k; gc.B = B; gc.G = G;
+    gc.pw = 1;
+    for (uint32_t q = 1; q < k; ++q) gc.pw *= B;
+    const uint32_t N = (uint32_t)n;
+    const uint32_t tiles = (N + PACK_TILE - 1) / PACK_TILE;
+    const uint32_t stride = std::max<uint32_t>(1, tiles / 256);           // about half a million samples at most
+    uint8_t *pin = static_cast<uint8_t *>(pinned_page());
+    HK_REQUIRE(pin != nullptr, HKCSA_ECUDA, "pinned page allocation failed");
+    double *h_gs = reinterpret_cast<double *>(pin + 2560);
+    HK_CUDA(cudaMemsetAsync(gs->hist, 0, (size_t)G * sizeof(uint32_t), st));
+    HK_CUDA(cudaMemsetAsync(gs->stats, 0, 8 * sizeof(uint64_t), st));
+    // the sampled positions: every stride-th tile of 2048
+    uint64_t nsamp = 0;
+    for (uint32_t t = 0; t < tiles; t += stride) nsamp += std::min<uint64_t>(PACK_TILE, n - (uint64_t)t * PACK_TILE);
+    const uint64_t smooth = std::max<uint64_t>(1, nsamp / G);
+    uint64_t *d_ctot = gs->cum + GRAM_MAX_G + 8;
+    {
+        prof::Scope ps(st, prof::OTHER, (uint64_t)N / stride + (uint64_t)G * 24);
+        gram_hist_kernel<<<(tiles + stride - 1) / stride, PACK_THREADS, 0, st>>>(d_text, N, gc, stride, gs->hist);
+        HK_LAUNCH_CHECK();
+        gram_scan_kernel<<<(G + GRAM_CHUNK - 1) / GRAM_CHUNK, 1024, 0, st>>>(gs->hist, G, smooth, gs->cum, d_ctot);
+        HK_LAUNCH_CHECK();
+        gram_assign_kernel<<<(G + 63) / 64, 64, 0, st>>>(gs->cum, d_ctot, gs->hist, G, B, (double)nsamp, gs->tab,
+                                                         reinterpret_cast<double *>(gs->stats));
+        HK_LAUNCH_CHECK();
+    }
+    HK_CUDA(cudaMemcpyAsync(h_gs, gs->stats, 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    HK_CUDA(cudaStreamSynchronize(st));
+    if (!(nsamp > 0 && h_gs[3] == 0 && h_gs[2] >= 1 && h_gs[2] <= (double)GRAM_MAX_LEN)) return HKCSA_OK;
+    gc.tab = gs->tab;
+    const double samples = (double)nsamp;
+    const double gram_len = h_gs[1] / samples;                          // mean code bits per gram
+    const double mu = h_gs[4] / samples;                                // information per gram: mean ...
+    const double var = std::max(1e-9, h_gs[5] / samples - mu * mu);     // ... and variance
+    const int gram_max_len = (int)h_gs[2];
+    const int min_bits = std::max(16, 8 * ((gram_max_len + 7) / 8));    // a key holds at least one whole gram
+    const double h_rate = h_gs[6] / samples;                            // information of a symbol given the k - 1 before it
+    const double h_var = std::max(1e-9, h_gs[7] / samples - h_rate * h_rate);
+    // Key width: the narrowest whose predicted survivors stay under 0.5 % of the suffixes.  A key of `cand` code bits
+    // covers s = cand * k / gram_len symbols; their information is about normal with the first gram's marginal mean /
+    // variance plus, per further symbol, the conditional ones (the text's entropy rate at order k - 1: the marginal
+    // statistics of DNA 6-grams are nearly flat, the skew sits in the conditionals).  A suffix survives round 0 when
+    // its key is likelier than 1 / n.  A survivor costs about as much as 40 elements of a radix pass, so a pass is
+    // worth dropping while it adds less than 2.5 % survivors; the prediction ran 4x low on the DNA workload, hence 0.5 %.
+    int bits = 64;
+    for (int cand = min_bits; cand <= 64; cand += 8) {
+        const double more = std::max(0.0, cand * (double)k / gram_len - k);
+        const double z = (log2((double)n) - (mu + more * h_rate)) / sqrt(var + more * h_var);
+        if (0.5 * erfc(-z / sqrt(2.0)) <= 0.005) { bits = cand; break; }
+    }
+    if (getenv("HKCSA_DEBUG_PLAN"))
+        fprintf(stderr, "[hkcsa] gram code: k=%u B=%u G=%u samples=%.0f len/gram=%.3f max_len=%d info/gram=%.3f var=%.3f "
+                "rate=%.3f var=%.3f -> bits0=%d\n", k, B, G, samples, gram_len, gram_max_len, mu, var, h_rate, h_var, bits);
+    if (e_bits0) bits = std::max(min_bits, std::min(64, want_bits0));
+    p.bits0 = bits;
+    p.max_len = gram_max_len;
+    p.k0 = (int)k * std::max(1, std::min(GRAM_PER_KEY, bits / gram_max_len));
+    p.passes0 = bits / 8;
+    return HKCSA_OK;
+}
+
+// ---------------------------------------------------------------- round 0: pack
+// key[i] = the first 8 * PASSES bits of the code stream of suffix i, from the key source Keys (suffix_array.cuh).
+// Keys are produced warp-striped so the stores are fully coalesced.  The suffix ids are not written at all: the first
+// radix pass takes "value = index" (radix_sort_pairs_u64, identity_vals).
+// PASSES = radix passes of round 0 = key bits / 8, a template parameter: the key shift and the digit histogram of
+// every pass (the bulk of the kernel's instructions: one shared atomic per key and pass) are straight-line code.
+// CARRY: the symbol before the suffix (its BWT symbol, csa/bwt.py:6-11) rides in the top byte of the key, above
+// the sorted bits (keys of at most 56 bits): the sort delivers the BWT in suffix-array order and nobody has to gather
+// text[SA[i] - 1] at random afterwards.
+// Persistent: a CTA takes every gridDim.x-th tile, so the digit histograms leave shared memory once per CTA, not once
+// per tile (1536 global atomics per 2048 keys otherwise: 0.55 -> 0.48 ms at C2), and the code tables are set up once.
+template <typename Keys, int PASSES, bool CARRY>
 __global__ void __launch_bounds__(PACK_THREADS, 6)
-sa_pack0_gram_kernel(const uint8_t *__restrict__ text, uint32_t n, GramCode gc, uint64_t *__restrict__ keys,
-                     uint32_t *__restrict__ ghist)
+sa_pack0_kernel(const uint8_t *__restrict__ text, uint32_t n, Keys src, uint64_t *__restrict__ keys,
+                uint32_t *__restrict__ ghist)
 {
     static_assert(!CARRY || PASSES <= 7, "the carried symbol needs the top byte of the key");
     constexpr int bits = 8 * PASSES;
-    constexpr int LOOK_THREADS = GRAM_LOOK / PACK_IPT;            // 16 threads also take a look-ahead group
-    __shared__ uint32_t s_cl[PACK_TILE + GRAM_LOOK];
+    __shared__ typename Keys::Smem s;
     __shared__ uint32_t s_hist[8 * RADIX];
-    __shared__ __align__(8) uint8_t s_dig[PACK_TILE + GRAM_LOOK + 16];
-    __shared__ uint8_t s_digit[256];
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    s_digit[tid] = gc.digit[tid];
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     hist_zero(s_hist, PASSES);
-    const bool aligned8 = (reinterpret_cast<uintptr_t>(text) & 7) == 0;
-    const uint32_t k = gc.k, B = gc.B, pw = gc.pw;
-    const uint32_t tiles = (n + PACK_TILE - 1) / PACK_TILE;
+    src.setup(s);
     __syncthreads();
+    const bool aligned8 = (reinterpret_cast<uintptr_t>(text) & 7) == 0;
+    const uint32_t tiles = (n + PACK_TILE - 1) / PACK_TILE;
     for (uint32_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
         const uint64_t base = (uint64_t)tile * PACK_TILE;
-        reinterpret_cast<uint2 *>(s_dig)[tid] = gram_digits8(text, n, base + (uint64_t)tid * PACK_IPT, aligned8, s_digit);
-        if (tid < LOOK_THREADS + 2)
-            reinterpret_cast<uint2 *>(s_dig)[PACK_THREADS + tid] =
-                gram_digits8(text, n, base + PACK_TILE + (uint64_t)tid * PACK_IPT, aligned8, s_digit);
-        __syncthreads();
-        {
-            uint32_t g[8], c[8];
-            gram_roll8(s_dig, tid * PACK_IPT, k, B, pw, g);
-#pragma unroll
-            for (int e = 0; e < 8; ++e) c[e] = __ldg(gc.tab + g[e]);
-            uint4 *dst = reinterpret_cast<uint4 *>(s_cl + tid * PACK_IPT);
-            dst[0] = make_uint4(c[0], c[1], c[2], c[3]);
-            dst[1] = make_uint4(c[4], c[5], c[6], c[7]);
-            if (tid < LOOK_THREADS) {
-                gram_roll8(s_dig, PACK_TILE + tid * PACK_IPT, k, B, pw, g);
-#pragma unroll
-                for (int e = 0; e < 8; ++e) c[e] = __ldg(gc.tab + g[e]);
-                uint4 *dl = reinterpret_cast<uint4 *>(s_cl + PACK_TILE + tid * PACK_IPT);
-                dl[0] = make_uint4(c[0], c[1], c[2], c[3]);
-                dl[1] = make_uint4(c[4], c[5], c[6], c[7]);
-            }
-        }
-        __syncthreads();
+        src.fill(s, text, n, base, aligned8);
 #pragma unroll
         for (int e = 0; e < PACK_IPT; ++e) {
             const uint32_t j = warp * (32u * PACK_IPT) + e * 32u + lane;
-            const uint64_t gpos = base + j;
-            uint64_t acc = 0;
-            uint32_t used = 0;
-            const uint32_t *p = s_cl + j;
-            // three grams without a test (3 x 27 bits cannot run past bit 63 of the shift count's range), then until
-            // the key is full: most keys of the DNA workload take four
-#pragma unroll
-            for (int t = 0; t < 3; ++t, p += k) {
-                const uint32_t c = *p;
-                acc |= ((uint64_t)(c & ~GRAM_LEN_MASK) << 32) >> used;
-                used += c & GRAM_LEN_MASK;
-            }
-#pragma unroll 1
-            for (int t = 3; t < GRAM_PER_KEY && used < (uint32_t)bits; ++t, p += k) {
-                const uint32_t c = *p;
-                acc |= ((uint64_t)(c & ~GRAM_LEN_MASK) << 32) >> used;
-                used += c & GRAM_LEN_MASK;
-            }
-            const uint64_t key = acc >> (64 - bits);
-            const bool valid = gpos < n;
+            const uint64_t g = base + j;
+            const uint64_t key = src.window(s, j, bits) >> (64 - bits);
+            const bool valid = g < n;
             if (valid) {
-                if (CARRY) keys[gpos] = key | ((uint64_t)__ldg(text + (gpos ? gpos - 1 : (uint64_t)n - 1)) << 56);
-                else keys[gpos] = key;
+                if (CARRY) keys[g] = key | ((uint64_t)__ldg(text + (g ? g - 1 : (uint64_t)n - 1)) << 56);   // an L1 hit: the tile was just read
+                else keys[g] = key;
             }
             hist_add_key_unsorted<PASSES>(s_hist, key, valid);
         }
-        __syncthreads();      // the next tile overwrites the digits and the entries
+        __syncthreads();      // the next tile overwrites the tile storage
     }
     hist_flush(s_hist, ghist, PASSES);
+}
+
+// sa_pack0_kernel<Keys, passes, carry> over the whole text (carry needs passes <= 7)
+template <typename Keys, int P = 2>
+static void launch_pack0(const Keys &src, int passes, bool carry, const uint8_t *text, uint32_t n, uint64_t *keys,
+                         uint32_t *ghist, cudaStream_t st)
+{
+    if constexpr (P < 8) {
+        if (passes != P) return launch_pack0<Keys, P + 1>(src, passes, carry, text, n, keys, ghist, st);
+    }
+    const uint32_t blocks = std::min<uint32_t>((n + PACK_TILE - 1) / PACK_TILE, (uint32_t)num_sms() * 6u);
+    if constexpr (P < 8) {
+        if (carry) { sa_pack0_kernel<Keys, P, true><<<blocks, PACK_THREADS, 0, st>>>(text, n, src, keys, ghist); return; }
+    }
+    sa_pack0_kernel<Keys, P, false><<<blocks, PACK_THREADS, 0, st>>>(text, n, src, keys, ghist);
 }
 
 // ---------------------------------------------------------------- later rounds: key build
@@ -497,7 +434,7 @@ struct LazyRank {
     int bits;                  // width of a round-0 key
     int shift;                 // key >> shift = bucket id
     uint64_t mask;             // the sorted bits of a round-0 key (the top byte may carry the BWT symbol)
-    GramCode gram;             // gram.tab != nullptr: round-0 keys come from the k-gram code
+    GramKeys gram;             // gram.code.tab != nullptr: round-0 keys come from the k-gram code
 };
 
 constexpr int LAZY_BUCKET_BITS = 20;
@@ -532,14 +469,10 @@ __global__ void sa_bucket_index_kernel(const uint64_t *__restrict__ keys0, uint3
 
 // COHERENT: the rank array is written by the calling kernel itself (sa_finish_small_kernel): read it with volatile loads
 template <bool COHERENT = false>
-__device__ __forceinline__ uint32_t lazy_rank_lookup(const LazyRank &lz, const uint32_t *s_code, const uint8_t *s_len,
-                                                     uint32_t n, uint32_t t, const uint32_t *rank)
+__device__ __forceinline__ uint32_t lazy_rank_lookup(const LazyRank &lz, const AlphaKeys::Tab &s_tab, uint32_t n,
+                                                     uint32_t t, const uint32_t *rank)
 {
-    const uint64_t key = lz.gram.tab ? gram_key(lz.gram, lz.text, n, t, lz.bits)
-                                     : alpha_pack(s_code, s_len, lz.bits, [&](int q) {
-                                           const uint64_t g = (uint64_t)t + q;
-                                           return g < n ? (uint32_t)lz.text[g] : 256u;
-                                       });
+    const uint64_t key = lz.gram.code.tab ? lz.gram.at(lz.text, n, t, lz.bits) : AlphaKeys::at(s_tab, lz.text, n, t, lz.bits);
     const uint32_t v = (uint32_t)(key >> lz.shift);
     uint32_t lo = __ldg(lz.bucket + v), hi = __ldg(lz.bucket + v + 1);
     if (hi - lo > (2u << LAZY_SAMPLE_SHIFT)) {
@@ -571,9 +504,8 @@ sa_keybuild_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__restrict
                    uint64_t *__restrict__ keys, uint32_t *__restrict__ ghist, LazyRank lz, AlphaCode ac)
 {
     __shared__ uint32_t s_hist[8 * RADIX];
-    __shared__ uint32_t s_code[257];
-    __shared__ uint8_t s_len[257];
-    for (uint32_t i = threadIdx.x; i < 257; i += blockDim.x) { s_code[i] = ac.code[i]; s_len[i] = ac.len[i]; }
+    __shared__ AlphaKeys::Tab s_tab;
+    s_tab.load(ac);
     hist_zero(s_hist, passes);
     __syncthreads();
     for (uint64_t base = (uint64_t)blockIdx.x * blockDim.x; base < m; base += (uint64_t)gridDim.x * blockDim.x) {
@@ -584,7 +516,7 @@ sa_keybuild_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__restrict
             const uint32_t i = cidx[j];
             const uint64_t t = (uint64_t)i + h;
             uint32_t k2 = 0;
-            if (t < n) k2 = (lz.text ? lazy_rank_lookup(lz, s_code, s_len, n, (uint32_t)t, rank) : rank[t]) + 1u;
+            if (t < n) k2 = (lz.text ? lazy_rank_lookup(lz, s_tab, n, (uint32_t)t, rank) : rank[t]) + 1u;
             key = ((uint64_t)cgrp[j] << b2) | k2;
             keys[j] = key;
         }
@@ -847,10 +779,10 @@ seg_apply_kernel(const uint16_t *__restrict__ flags, const uint32_t *__restrict_
 
 // ---------------------------------------------------------------- group-local refinement (no radix sort)
 // After round 0 nearly all surviving groups hold two or three suffixes.  Sorting them with seven or eight radix
-// passes over the whole working set is out of proportion: here the thread of a group's first element loads the
-// group's suffix ids, orders them by comparing the text directly from the known depth on (up to GS_DEPTH more
-// symbols; the end of the text is smallest), writes them back in order and gives every element the key
-// (group start << 32 | number of its sub-group): equal keys = still tied within GS_DEPTH symbols.  The usual
+// passes over the whole working set is out of proportion: here every small group is ordered by comparing the text
+// directly from the known depth on (up to GS_DEPTH more symbols; the end of the text is smallest), written back in
+// order, and every element gets the key (group start << 32 | number of its sub-group): equal keys = still tied within
+// GS_DEPTH symbols.  The usual
 // seg_reduce / seg_scan / seg_apply then refine on these keys.  Groups above GS_MAX elements are left alone (one key
 // for the whole group): they go to the next regular round, whose depth therefore stays where it was.
 // -1 / 0 / +1: order of suffixes a and b beyond the `depth` symbols they share, 0 = tied within GS_DEPTH symbols
@@ -1092,49 +1024,10 @@ group_sort_marked_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict
     group_sort_serial<WIDE>(cidx, j, s, g, text, n, depth, ids64, keys);
 }
 
-// Small working sets (one wave of CTAs: the kernel lasts as long as its longest chain of dependent loads, and a group
-// whose members share more than the guaranteed depth -- k-gram keys: 6 symbols guaranteed, ~21 shared -- ties inside
-// its first window): every key starts as (g << 32), the thread of a group's first element orders the group serially.
-__global__ void group_key_init_kernel(const uint32_t *__restrict__ cgrp, uint32_t m, uint64_t *__restrict__ keys)
-{
-    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j < m) keys[j] = (uint64_t)cgrp[j] << 32;
-}
-template <bool WIDE>
-__global__ void __launch_bounds__(256)
-group_sort_heads_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp, uint32_t m,
-                        const uint8_t *__restrict__ text, uint64_t n, uint64_t depth,
-                        const uint64_t *__restrict__ ids64, uint64_t *__restrict__ keys)
-{
-    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= m) return;
-    const uint32_t g = cgrp[j];
-    if (j > 0 && cgrp[j - 1] == g) return;                      // not the first element of its group
-    uint32_t s = 1;
-    while (s <= GS_MAX && j + s < m && cgrp[j + s] == g) ++s;
-    if (s > GS_MAX || s < 2) return;                            // large group: keys stay (g << 32) for every member
-    group_sort_serial<WIDE>(cidx, j, s, g, text, n, depth, ids64, keys);
-}
-
-// serial / element-parallel: 0.79 M survivors (C2) 0.088 / 0.077 ms, 5.1 M (C3) 0.197 / 0.160 ms, 164 M 10.2 / 5.5 ms
-// (64-bit ids 13.0 / 5.5 ms): the element-parallel form everywhere; HKCSA_GC_MIN_M=<m> keeps the serial one below m
-constexpr uint32_t GC_MIN_M = 0;
-
 cudaError_t group_local_keys(uint32_t *cidx, const uint32_t *cgrp, uint32_t m, const uint8_t *text, uint64_t n,
                              uint64_t depth, const uint64_t *ids64, uint64_t *keys, cudaStream_t st)
 {
     if (m == 0) return cudaSuccess;
-    uint32_t min_m = GC_MIN_M;
-    if (const char *e = getenv("HKCSA_GC_MIN_M")) min_m = (uint32_t)strtoul(e, nullptr, 10);   // tests: a huge value = always the serial form
-    if (m < min_m) {
-        const uint32_t blocks = (m + 255) / 256;
-        group_key_init_kernel<<<blocks, 256, 0, st>>>(cgrp, m, keys);
-        count_launch();
-        if (ids64) group_sort_heads_kernel<true><<<blocks, 256, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
-        else group_sort_heads_kernel<false><<<blocks, 256, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
-        count_launch();
-        return cudaGetLastError();
-    }
     const uint32_t blocks = (m + GC_STRIDE - 1) / GC_STRIDE;
     const uint32_t blocks2 = (m + 255) / 256;
     if (ids64) {
@@ -1163,11 +1056,10 @@ sa_finish_small_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__rest
 {
     __shared__ uint64_t s_key[FIN_MAX];
     __shared__ uint32_t s_idx[FIN_MAX], s_grp[FIN_MAX], s_pos[FIN_MAX], s_aux[FIN_MAX];
-    __shared__ uint32_t s_code[257];
-    __shared__ uint8_t s_len[257];
+    __shared__ AlphaKeys::Tab s_tab;
     __shared__ uint32_t s_w[32], s_w2[32];
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    for (uint32_t i = tid; i < 257; i += FIN_MAX) { s_code[i] = ac.code[i]; s_len[i] = ac.len[i]; }
+    s_tab.load(ac);
     if (tid < m) { s_idx[tid] = cidx[tid]; s_grp[tid] = cgrp[tid]; s_pos[tid] = cpos[tid]; }
     __syncthreads();
     for (int iter = 0; iter < 64 && m > 0; ++iter) {
@@ -1179,7 +1071,7 @@ sa_finish_small_kernel(const uint32_t *__restrict__ cidx, const uint32_t *__rest
             const uint64_t t = (uint64_t)idx + h;
             uint32_t k2 = 0;
             if (t < n)
-                k2 = (lz.text ? lazy_rank_lookup<true>(lz, s_code, s_len, n, (uint32_t)t, rank)
+                k2 = (lz.text ? lazy_rank_lookup<true>(lz, s_tab, n, (uint32_t)t, rank)
                               : *reinterpret_cast<const volatile uint32_t *>(rank + t)) + 1u;
             key = ((uint64_t)s_grp[tid] << 32) | k2;
         }
@@ -1265,8 +1157,7 @@ struct SaBuffers {
     uint64_t *hist64;
     uint32_t *bucket;
     uint64_t *samples;
-    uint32_t *gram_tab, *gram_hist;
-    uint64_t *gram_cum, *gram_stats;
+    GramScratch gram;
     SortScratch sort;
 };
 
@@ -1289,10 +1180,10 @@ SaBuffers carve_sa(Carver &c, uint64_t n)
     b.hist64 = c.take<uint64_t>(256);
     b.bucket = c.take<uint32_t>((1u << LAZY_BUCKET_BITS) + 2);
     b.samples = c.take<uint64_t>((n >> LAZY_SAMPLE_SHIFT) + 2);
-    b.gram_tab = c.take<uint32_t>(GRAM_MAX_G);
-    b.gram_hist = c.take<uint32_t>(GRAM_MAX_G);
-    b.gram_cum = c.take<uint64_t>(GRAM_MAX_G + 8 + GRAM_MAX_CHUNKS + 8);      // per-chunk prefix sums, then the chunk totals
-    b.gram_stats = c.take<uint64_t>(8);
+    b.gram.tab = c.take<uint32_t>(GRAM_MAX_G);
+    b.gram.hist = c.take<uint32_t>(GRAM_MAX_G);
+    b.gram.cum = c.take<uint64_t>(GRAM_MAX_G + 8 + GRAM_MAX_CHUNKS + 8);      // per-chunk prefix sums, then the chunk totals
+    b.gram.stats = c.take<uint64_t>(8);
     b.sort = carve_sort_scratch(c, n);
     return b;
 }
@@ -1341,86 +1232,11 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
     HK_CUDA(cudaMemcpyAsync(h_hist, B.hist64, 256 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     HK_CUDA(cudaStreamSynchronize(st));
     static thread_local Round0Plan r0;
-    make_round0_plan(h_hist, r0, /*want_carry=*/d_bwt != nullptr);
+    if (int rc = plan_round0(h_hist, r0, d_text, n, &B.gram, st)) return rc;
     const AlphaCode &ac = r0.ac;
+    const GramCode &gc = r0.gram;
     const uint32_t sigma = r0.sigma;
     const uint32_t N = (uint32_t)n;
-    // ---- the k-gram code (suffix_array.cuh): sampled gram histogram -> code built on the device -> its statistics
-    //      decide the key width.  Small texts and failures keep the per-symbol code of the plan above.
-    GramCode &gc = r0.gram;
-    gc.tab = nullptr;
-    {
-        SaBuffers &B_ = B;
-        const char *e = getenv("HKCSA_GRAM");
-        const uint32_t B = sigma + 1;
-        uint32_t k = 1, G = B;
-        while (k < (uint32_t)GRAM_MAX_K && (uint64_t)G * B <= (uint64_t)GRAM_MAX_G) { G *= B; ++k; }
-        if (n >= 1024 && k >= (uint32_t)GRAM_MIN_K && !(e && atoi(e) == 0)) {
-            memset(gc.digit, 0, sizeof(gc.digit));
-            uint32_t dgt = 0;
-            for (int ch = 0; ch < 256; ++ch)
-                if (h_hist[ch]) gc.digit[ch] = (uint8_t)++dgt;      // k >= 4 means B <= 19
-            gc.k = k; gc.B = B; gc.G = G;
-            gc.pw = 1;
-            for (uint32_t q = 1; q < k; ++q) gc.pw *= B;
-            const uint32_t tiles = (N + PACK_TILE - 1) / PACK_TILE;
-            const uint32_t stride = std::max<uint32_t>(1, tiles / 256);           // about half a million samples at most
-            double *h_gs = reinterpret_cast<double *>(pin + 2560);
-            HK_CUDA(cudaMemsetAsync(B_.gram_hist, 0, (size_t)G * sizeof(uint32_t), st));
-            HK_CUDA(cudaMemsetAsync(B_.gram_stats, 0, 8 * sizeof(uint64_t), st));
-            // the sampled positions: every stride-th tile of 2048
-            uint64_t nsamp = 0;
-            for (uint32_t t = 0; t < tiles; t += stride) nsamp += std::min<uint64_t>(PACK_TILE, n - (uint64_t)t * PACK_TILE);
-            const uint64_t smooth = std::max<uint64_t>(1, nsamp / G);
-            uint64_t *d_ctot = B_.gram_cum + GRAM_MAX_G + 8;
-            {
-                prof::Scope ps(st, prof::OTHER, (uint64_t)N / stride + (uint64_t)G * 24);
-                gram_hist_kernel<<<(tiles + stride - 1) / stride, PACK_THREADS, 0, st>>>(d_text, N, gc, stride, B_.gram_hist);
-                HK_LAUNCH_CHECK();
-                gram_scan_kernel<<<(G + GRAM_CHUNK - 1) / GRAM_CHUNK, 1024, 0, st>>>(B_.gram_hist, G, smooth, B_.gram_cum, d_ctot);
-                HK_LAUNCH_CHECK();
-                gram_assign_kernel<<<(G + 63) / 64, 64, 0, st>>>(B_.gram_cum, d_ctot, B_.gram_hist, G, B, (double)nsamp,
-                                                                 B_.gram_tab, reinterpret_cast<double *>(B_.gram_stats));
-                HK_LAUNCH_CHECK();
-            }
-            HK_CUDA(cudaMemcpyAsync(h_gs, B_.gram_stats, 8 * sizeof(double), cudaMemcpyDeviceToHost, st));
-            HK_CUDA(cudaStreamSynchronize(st));
-            if (nsamp > 0 && h_gs[3] == 0 && h_gs[2] >= 1 && h_gs[2] <= (double)GRAM_MAX_LEN) {
-                gc.tab = B_.gram_tab;
-                const double samples = (double)nsamp;
-                const double gram_len = h_gs[1] / samples;                          // mean code bits per gram
-                const double mu = h_gs[4] / samples;                                // information per gram: mean ...
-                const double var = std::max(1e-9, h_gs[5] / samples - mu * mu);     // ... and variance
-                const int gram_max_len = (int)h_gs[2];
-                const int min_bits = std::max(16, 8 * ((gram_max_len + 7) / 8));    // a key holds at least one whole gram
-                const double h_rate = h_gs[6] / samples;                            // information of a symbol given the k - 1 before it
-                const double h_var = std::max(1e-9, h_gs[7] / samples - h_rate * h_rate);
-                // Key width: the narrowest whose predicted survivors stay under 0.5 % of the suffixes.  A key of `cand`
-                // code bits covers s = cand * k / gram_len symbols; their information is about normal with the first
-                // gram's marginal mean / variance plus, per further symbol, the conditional ones (the text's entropy
-                // rate at order k - 1: the marginal statistics of DNA 6-grams are nearly flat, the skew sits in the
-                // conditionals).  A suffix survives round 0 when its key is likelier than 1 / n.  A survivor costs
-                // about as much as 40 elements of a radix pass, so a pass is worth dropping while it adds less than
-                // 2.5 % survivors; the prediction ran 4x low on the DNA workload, hence 0.5 %.
-                int bits = 64;
-                for (int cand = min_bits; cand <= 64; cand += 8) {
-                    const double more = std::max(0.0, cand * (double)k / gram_len - k);
-                    const double z = (log2((double)n) - (mu + more * h_rate)) / sqrt(var + more * h_var);
-                    if (0.5 * erfc(-z / sqrt(2.0)) <= 0.005) { bits = cand; break; }
-                }
-                if (getenv("HKCSA_DEBUG_PLAN"))
-                    fprintf(stderr, "[hkcsa] gram code: k=%u B=%u G=%u samples=%.0f len/gram=%.3f max_len=%d info/gram=%.3f var=%.3f "
-                            "rate=%.3f var=%.3f -> bits0=%d\n", k, B, G, samples, gram_len, gram_max_len, mu, var, h_rate, h_var, bits);
-                const char *c56 = getenv("HKCSA_CARRY56");
-                if (d_bwt && bits > 56 && c56 && atoi(c56)) bits = 56;
-                if (const char *eb = getenv("HKCSA_BITS0")) bits = std::max(min_bits, std::min(64, 8 * (atoi(eb) / 8)));
-                r0.bits0 = bits;
-                r0.max_len = gram_max_len;
-                r0.k0 = (int)k * std::max(1, std::min(GRAM_PER_KEY, bits / gram_max_len));
-                r0.passes0 = bits / 8;
-            }
-        }
-    }
     stats.gram_k = gc.tab ? gc.k : 0;
     const int max_len = r0.max_len, bits0 = r0.bits0, k0 = r0.k0, passes0 = r0.passes0;
     stats.sigma = sigma;
@@ -1439,31 +1255,9 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
     uint32_t *va = (passes0 % 2 == 0) ? d_sa : B.val[0];
     uint32_t *vb = (passes0 % 2 == 0) ? B.val[0] : d_sa;
     {
-        const uint32_t blocks = std::min<uint32_t>((N + PACK_TILE - 1) / PACK_TILE, (uint32_t)num_sms() * 6u);
         prof::Scope ps(st, prof::SA_PACK0, (uint64_t)N * 9);
-        if (gc.tab) {
-#define HK_PACKG(P)                                                                                                 \
-    case P:                                                                                                          \
-        if (carry) sa_pack0_gram_kernel<P, true><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, gc, ka, B.sort.hist);  \
-        else sa_pack0_gram_kernel<P, false><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, gc, ka, B.sort.hist);       \
-        break;
-            switch (passes0) {
-                HK_PACKG(2) HK_PACKG(3) HK_PACKG(4) HK_PACKG(5) HK_PACKG(6) HK_PACKG(7)
-                default: sa_pack0_gram_kernel<8, false><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, gc, ka, B.sort.hist); break;
-            }
-#undef HK_PACKG
-        } else {
-#define HK_PACK0(P)                                                                                              \
-    case P:                                                                                                       \
-        if (carry) sa_pack0_kernel<P, true><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, ac, (uint32_t)max_len, ka, B.sort.hist);     \
-        else sa_pack0_kernel<P, false><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, ac, (uint32_t)max_len, ka, B.sort.hist);          \
-        break;
-        switch (passes0) {
-            HK_PACK0(2) HK_PACK0(3) HK_PACK0(4) HK_PACK0(5) HK_PACK0(6) HK_PACK0(7)
-            default: sa_pack0_kernel<8, false><<<blocks, PACK_THREADS, 0, st>>>(d_text, N, ac, (uint32_t)max_len, ka, B.sort.hist); break;
-        }
-#undef HK_PACK0
-        }
+        if (gc.tab) launch_pack0(GramKeys{gc}, passes0, carry, d_text, N, ka, B.sort.hist, st);
+        else launch_pack0(AlphaKeys{ac, (uint32_t)max_len}, passes0, carry, d_text, N, ka, B.sort.hist, st);
         HK_LAUNCH_CHECK();
     }
     HK_CUDA(radix_sort_pairs_u64(ka, va, kb, vb, N, passes0, B.sort, st, /*identity_vals=*/true));
@@ -1487,7 +1281,7 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
     const int bucket_bits = std::min(LAZY_BUCKET_BITS, bits0);
     lz.shift = bits0 - bucket_bits;
     lz.mask = mask0;
-    lz.gram = gc;
+    lz.gram = GramKeys{gc};
     uint64_t *kx = nullptr, *ky = nullptr;             // key ping-pong of the later rounds
     uint32_t *vfree = B.val[1];                        // free value buffer (receives the compacted ids)
     uint32_t *vother = B.val[0];                       // the round-0 sort's other value buffer: free from here on

@@ -130,12 +130,13 @@ def test_sa_bwt_oracle(E, name):
     assert host(E.bwt(d_text, sa)).tobytes() == O.bwt_transform(text, want).tobytes()
 
 
-@pytest.mark.parametrize("env", [{}, {"HKCSA_CARRY56": "1"}, {"HKCSA_BITS0": "24"}, {"HKCSA_BITS0": "56", "HKCSA_NO_GROUP_ROUND": "1"},
-                                 {"HKCSA_GRAM": "0", "HKCSA_CARRY56": "1"}])
+@pytest.mark.parametrize("env", [{}, pytest.param({"HKCSA_BITS0": "56"}, id="bits0_56"), {"HKCSA_BITS0": "24"},
+                                 {"HKCSA_BITS0": "56", "HKCSA_NO_GROUP_ROUND": "1"},
+                                 pytest.param({"HKCSA_GRAM": "0", "HKCSA_BITS0": "56"}, id="gram0_bits0_56")])
 @pytest.mark.parametrize("name", list(TEXTS))
 def test_sa_bwt_one_call(E, name, env, monkeypatch):
     """hkcsa_sa_bwt_build: the BWT symbol rides in the top byte of the round-0 key (keys of at most 56 bits) or the
-    gather runs after the build (64-bit keys, unless HKCSA_CARRY56=1 trims them to 56); narrow keys leave many suffixes to the later
+    gather runs after the build (64-bit keys, unless HKCSA_BITS0 trims them to 56); narrow keys leave many suffixes to the later
     rounds, whose slots get their BWT rows rewritten."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
@@ -484,17 +485,11 @@ def test_distributed_build_reference_benchmark_workload(E):
     _check_slices(_emulated_build(E, text, 4, False), text, False)
 
 
-def name_hash(name):
-    return sum(name.encode()) % 2          # half of the texts through each form
-
-
 @pytest.mark.parametrize("env", [{}, {"HKCSA_BITS0": "24"}, {"HKCSA_GRAM": "0", "HKCSA_BITS0": "16"}, {"HKCSA_BITS0": "40"}])
 @pytest.mark.parametrize("name", list(TEXTS))
 def test_sa_bwt_with_element_parallel_group_round(E, name, env, monkeypatch):
-    """Round 1 of the single-GPU builder through the element-parallel group kernel (the default) and through the serial
-    form (HKCSA_GC_MIN_M beyond any working set); narrow round-0 keys (HKCSA_BITS0) leave many groups, big ones
-    included."""
-    monkeypatch.setenv("HKCSA_GC_MIN_M", "0" if name_hash(name) else "4294967295")
+    """Round 1 of the single-GPU builder through the element-parallel group kernel and its second launch for the groups
+    it marks; narrow round-0 keys (HKCSA_BITS0) leave many groups, big ones included."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     text = TEXTS[name]
@@ -507,11 +502,11 @@ def test_sa_bwt_with_element_parallel_group_round(E, name, env, monkeypatch):
 @pytest.mark.parametrize("name", ["eng_300k", "dna_300k", "runs", "rand256_50k", "dna_1m_dollar", "rand2_100k", "fib"])
 @pytest.mark.parametrize("parts", [1, 3, 8])
 def test_distributed_build_with_element_parallel_group_round(E, name, parts, monkeypatch):
-    """The group round's two forms give the same slices, 32- and 64-bit ids: the element-parallel kernel (default;
-    groups across CTA boundaries, groups of more than 16, windows that tie or reach the end of the text -- marked for
-    the serial second launch; 64-bit ids with and without the key extension bits) and the serial form."""
+    """The element-parallel group round gives the right slices, 32- and 64-bit ids: groups across CTA boundaries, groups
+    of more than 16, windows that tie or reach the end of the text -- marked for the serial second launch; 64-bit ids
+    with and without the key extension bits."""
     text = TEXTS[name]
-    for env in ({}, {"HKCSA_DSA_NO_XBITS": "1"}, {"HKCSA_GC_MIN_M": "4294967295"}):
+    for env in ({}, {"HKCSA_DSA_NO_XBITS": "1"}):
         with monkeypatch.context() as mp:
             for k, v in env.items():
                 mp.setenv(k, v)
