@@ -4,14 +4,18 @@
 //
 //  * inverse-SA samples: isa[k] = row of the suffix that starts at text position k * rate (k < S = ceil(n / rate)),
 //    isa[S] = isa[0].  Derived from the sampled SA alone -- every marked row j has slot r = rank1(marks, j) and
-//    samples[r] = SA[j] / rate -- so a loaded index (no text, no full SA) has them too.
+//    samples[r] = SA[j] / rate -- so a loaded index (no text, no full SA) has them too.  The sliced index of the
+//    distributed build runs the same kernel once per slice, with the slice's first global row as the row offset.
 //  * batched extract: a request [begin, end) is cut at sample boundaries into segments
 //    [k * rate, (k + 1) * rate) & [begin, end); each segment is one independent walk that starts at row isa[k + 1]
 //    (the suffix just past the segment: its BWT symbol is the segment's last symbol) and emits text[p - 1],
 //    text[p - 2], ... by LF steps.  Whole-text extraction is n / rate walks of <= rate steps: a parallel BWT
 //    inversion.  Adjacent threads own adjacent segments, so the byte stores of a long range land close together.
-//    The LF step is the wavelet tree's access + rank descent, or the sampled Occ table's (layouts 0 and 1).
+//    The LF step comes from a source: the wavelet tree's access + rank descent or the sampled Occ table's (layouts 0
+//    and 1), with 32-bit rows and the plain step; or the sliced index (MsDev), with 64-bit global rows and the exact
+//    step, so that it gives the text back on every text.
 #include "common.cuh"
+#include "multi_slice.cuh"
 #include "occ.cuh"
 #include "prof.cuh"
 #include "wavelet.cuh"
@@ -22,9 +26,13 @@ constexpr int EXT_THREADS = 256;
 constexpr int SCAN_THREADS = 1024;
 
 // ---------------------------------------------------------------- inverse-SA samples
-// one thread per mark rank block: the marked rows of the block in order, their slots from the block's rank header
+// one thread per mark rank block: the marked rows of the block in order, their slots from the block's rank header.
+// Row: uint32_t for the index of one text, uint64_t for the sliced index (row_off = the slice's first global row,
+// S = the whole text's sample count).
+template <typename Row>
 __global__ void __launch_bounds__(256)
-isa_samples_kernel(BitVec marks, const uint32_t *__restrict__ samples, uint64_t n, uint64_t S, uint32_t *__restrict__ isa)
+isa_samples_kernel(BitVec marks, const uint32_t *__restrict__ samples, uint64_t n, uint64_t S, uint64_t row_off,
+                   Row *__restrict__ isa)
 {
     const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g * HKCSA_BLOCK_BITS >= n) return;
@@ -41,8 +49,8 @@ isa_samples_kernel(BitVec marks, const uint32_t *__restrict__ samples, uint64_t 
             m &= m - 1;
             if (j >= n) break;
             const uint32_t s = samples[r++];
-            isa[s] = (uint32_t)j;
-            if (s == 0) isa[S] = (uint32_t)j;     // the walk of the text's last stretch starts at the row of suffix 0
+            isa[s] = (Row)(row_off + j);
+            if (s == 0) isa[S] = (Row)(row_off + j);   // the walk of the text's last stretch starts at the row of suffix 0
         }
     }
 }
@@ -147,8 +155,9 @@ __device__ __forceinline__ uint64_t request_of(const uint64_t *__restrict__ seg_
     return lo;
 }
 
+template <typename Row>
 struct ExtractArgs {
-    const uint32_t *isa;
+    const Row *isa;
     uint32_t rate;
     uint64_t n;
     const int64_t *begin, *end, *out_off;
@@ -157,11 +166,59 @@ struct ExtractArgs {
     uint8_t *out;
 };
 
-// the walks of every segment, grid-strided; each LF step of the rank source (WtDev or OccDev<SHIFT>, occ.cuh) gives
-// LF(j) and the symbol bwt[j]
+// The sliced index of the distributed build (multi_slice.cuh) as an extract source: 64-bit global rows and the
+// exact step of ms_locate_kernel.  A step finds the slice of j among the starts, runs the access + rank descent on
+// that slice's tree (node tables from global memory on the read-only path, as ms_rank) and maps the code to its
+// byte; the next row is C[c] + lf_fix(cum[s][c] + occ, ...).  The starts, C[] and cum[][] (16 KB at 8 slices) are
+// in shared memory, c0 and fix are read once per CTA from row0.
+struct MsSmem {
+    uint64_t start[HKCSA_MAX_SLICES + 1];
+    uint64_t cum[HKCSA_MAX_SLICES][256];
+    uint64_t C[256];
+    uint64_t row0;
+    uint32_t S, c0, fix;
+};
+struct MsStep {
+    uint32_t slice, sym, occ;             // occ: occurrences of sym in the slice before j
+};
+struct MsDev {
+    const MultiDesc *d;
+
+    using Smem = MsSmem;
+    using Row = uint64_t;
+    __device__ __forceinline__ void load(MsSmem &s) const
+    {
+        const uint32_t S = d->S;
+        for (uint32_t i = threadIdx.x; i < S * 256u; i += blockDim.x) (&s.cum[0][0])[i] = (&d->cum[0][0])[i];
+        for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s.C[i] = d->C[i];
+        for (uint32_t i = threadIdx.x; i <= S; i += blockDim.x) s.start[i] = d->start[i];
+        if (threadIdx.x == 0) {
+            s.S = S;
+            s.row0 = d->row0;
+            ms_suffix0(d, s.c0, s.fix);
+        }
+    }
+    __device__ __forceinline__ MsStep step(const MsSmem &s, uint64_t j) const
+    {
+        MsStep t;
+        t.slice = ms_slice_of(s.start, s.S, j);
+        const WtDev &w = d->slice[t.slice];
+        const uint32_t code = wt_access_rank(*w.tab, w, (uint32_t)(j - s.start[t.slice]), t.occ);
+        t.sym = __ldg(&w.tab->sym_of_code[code]);
+        return t;
+    }
+    __device__ __forceinline__ uint64_t next(const MsSmem &s, const MsStep &t, uint64_t j) const
+    {
+        return s.C[t.sym] + lf_fix(s.cum[t.slice][t.sym] + t.occ, t.sym, j, s.c0, s.row0, s.fix);
+    }
+};
+
+// the walks of every segment, grid-strided.  Each step of the source (WtDev, OccDev<SHIFT> or MsDev) gives the symbol
+// bwt[j], and its `next` gives LF(j) from that step
 template <typename Src>
-__global__ void __launch_bounds__(EXT_THREADS) extract_kernel(Src src, ExtractArgs a)
+__global__ void __launch_bounds__(EXT_THREADS) extract_kernel(Src src, ExtractArgs<typename Src::Row> a)
 {
+    using Row = typename Src::Row;
     __shared__ typename Src::Smem s;
     src.load(s);
     __syncthreads();
@@ -174,11 +231,11 @@ __global__ void __launch_bounds__(EXT_THREADS) extract_kernel(Src src, ExtractAr
         const uint64_t lo = max(r.b, k * a.rate);
         const uint64_t hi = min(r.e, (k + 1) * a.rate);
         uint64_t p = min((k + 1) * a.rate, a.n);   // the walk starts at the row of the suffix that begins at p
-        uint32_t j = __ldg(a.isa + k + 1);
+        Row j = __ldg(a.isa + k + 1);
         uint8_t *dst = a.out + a.out_off[q];
         while (p > lo) {
-            const LfStep st = src.step(s, j);
-            j = s.C[st.code] + st.occ;
+            const auto st = src.step(s, j);
+            j = src.next(s, st, j);
             --p;                                   // st.sym = text[p]
             if (p < hi) dst[p - r.b] = (uint8_t)st.sym;
         }
@@ -208,6 +265,24 @@ static int ssa_plan_check(const hkcsa_ssa_plan *p)
     return HKCSA_OK;
 }
 
+// the samples of one (slice of a) sampled SA into isa[]: S = the whole text's sample count, row_off = the first row
+template <typename Row>
+static int isa_samples_launch(const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa, uint64_t S, uint64_t row_off,
+                              Row *d_isa, cudaStream_t st)
+{
+    const uint64_t n = h_ssa->n;
+    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
+    BitVec marks;
+    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
+    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
+    marks.len = n;
+    const uint64_t nblocks = (n + HKCSA_BLOCK_BITS - 1) / HKCSA_BLOCK_BITS;
+    isa_samples_kernel<Row><<<(uint32_t)((nblocks + 255) / 256), 256, 0, st>>>(
+        marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), n, S, row_off, d_isa);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
+}
+
 extern "C" int hkcsa_isa_samples(const void *d_ssa_blob, const hkcsa_ssa_plan *h_ssa, uint32_t *d_isa, void *stream)
 {
     HK_REQUIRE(d_ssa_blob && h_ssa && d_isa, HKCSA_EINVAL, "null pointer");
@@ -216,17 +291,46 @@ extern "C" int hkcsa_isa_samples(const void *d_ssa_blob, const hkcsa_ssa_plan *h
     const uint64_t n = h_ssa->n, S = h_ssa->n_samples;
     if (n == 0) return HKCSA_OK;
     cudaStream_t st = as_stream(stream);
-    const uint8_t *sb = static_cast<const uint8_t *>(d_ssa_blob);
-    BitVec marks;
-    marks.blocks = reinterpret_cast<const RankBlock *>(sb + h_ssa->off_blocks);
-    marks.super = reinterpret_cast<const uint64_t *>(sb + h_ssa->off_super);
-    marks.len = n;
     const uint64_t nblocks = (n + HKCSA_BLOCK_BITS - 1) / HKCSA_BLOCK_BITS;
     // mark blocks and samples read once, S + 1 entries scattered
     prof::Scope ps(st, prof::SSA_BUILD, nblocks * sizeof(RankBlock) + S * 4 + (S + 1) * 4);
-    isa_samples_kernel<<<(uint32_t)((nblocks + 255) / 256), 256, 0, st>>>(
-        marks, reinterpret_cast<const uint32_t *>(sb + h_ssa->off_samples), n, S, d_isa);
-    HK_LAUNCH_CHECK();
+    return isa_samples_launch<uint32_t>(d_ssa_blob, h_ssa, S, 0, d_isa, st);
+}
+
+extern "C" int hkcsa_multi_isa_samples(uint32_t S, const void *const *d_ssa_blobs,
+                                       const hkcsa_ssa_plan *const *h_ssa_plans, const uint64_t *h_starts,
+                                       uint64_t *d_isa, void *stream)
+{
+    HK_REQUIRE(S >= 1 && S <= HKCSA_MAX_SLICES, HKCSA_EINVAL, "1..HKCSA_MAX_SLICES slices");
+    HK_REQUIRE(d_ssa_blobs && h_ssa_plans && h_starts && d_isa, HKCSA_EINVAL, "null pointer");
+    const uint64_t n = h_starts[S];
+    HK_REQUIRE(n <= (1ull << 40), HKCSA_ERANGE, "n exceeds 2^40");
+    HK_REQUIRE(h_ssa_plans[0], HKCSA_EINVAL, "null slice");
+    const uint32_t rate = h_ssa_plans[0]->rate;
+    HK_REQUIRE(rate >= 1, HKCSA_EINVAL, "sampling rate must be >= 1");
+    uint64_t samples = 0, blocks = 0;
+    for (uint32_t s = 0; s < S; ++s) {
+        const hkcsa_ssa_plan *p = h_ssa_plans[s];
+        HK_REQUIRE(d_ssa_blobs[s] && p, HKCSA_EINVAL, "null slice");
+        HK_REQUIRE(p->rate == rate, HKCSA_EINVAL, "slices sampled at different rates");
+        HK_REQUIRE(h_starts[s] <= h_starts[s + 1] && p->n == h_starts[s + 1] - h_starts[s], HKCSA_EINVAL,
+                   "slice length != plan length");
+        samples += p->n_samples;
+        blocks += (p->n + HKCSA_BLOCK_BITS - 1) / HKCSA_BLOCK_BITS;
+    }
+    const uint64_t total = (n + rate - 1) / rate;
+    HK_REQUIRE(total <= (1ull << 32), HKCSA_ERANGE, "ceil(n / rate) exceeds 2^32 (the samples are 32-bit)");
+    HK_REQUIRE(samples == total, HKCSA_EINVAL,
+               "the slices' samples do not add up to ceil(n / rate) (slices of different builds?)");
+    if (n == 0) return HKCSA_OK;
+    cudaStream_t st = as_stream(stream);
+    // mark blocks and samples read once, S + 1 entries scattered
+    prof::Scope ps(st, prof::SSA_BUILD, blocks * sizeof(RankBlock) + total * 4 + (total + 1) * 8);
+    for (uint32_t s = 0; s < S; ++s) {
+        if (h_ssa_plans[s]->n == 0) continue;
+        const int rc = isa_samples_launch<uint64_t>(d_ssa_blobs[s], h_ssa_plans[s], total, h_starts[s], d_isa, st);
+        if (rc != HKCSA_OK) return rc;
+    }
     return HKCSA_OK;
 }
 
@@ -242,6 +346,32 @@ extern "C" size_t hkcsa_extract_scratch_bytes(uint64_t R)
 {
     uint64_t *a, *b;
     return extract_scratch(R, &a, &b, nullptr);
+}
+
+// Both extract entry points once their own checks passed: the request pointers and the scratch, the segment offsets
+// (three scan launches), then the walks over the source's rows.  R >= 1.
+template <typename Src>
+static int extract_run(Src src, const typename Src::Row *d_isa, uint32_t rate, uint64_t n, const int64_t *d_begin,
+                       const int64_t *d_end, const int64_t *d_out_off, uint64_t R, uint8_t *d_out, void *d_scratch,
+                       size_t scratch_bytes, cudaStream_t st)
+{
+    HK_REQUIRE(d_begin && d_end && d_out_off && d_out && d_scratch, HKCSA_EINVAL, "null pointer");
+    uint64_t *seg_off, *bsum;
+    HK_REQUIRE(extract_scratch(R, &seg_off, &bsum, d_scratch) <= scratch_bytes, HKCSA_ESCRATCH, "extract scratch too small");
+
+    const uint32_t nb = (uint32_t)((R + SCAN_THREADS - 1) / SCAN_THREADS);
+    seg_block_sum_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum);
+    HK_LAUNCH_CHECK();
+    seg_scan_sums_kernel<<<1, SCAN_THREADS, 0, st>>>(bsum, nb);
+    HK_LAUNCH_CHECK();
+    seg_offsets_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum, seg_off);
+    HK_LAUNCH_CHECK();
+
+    ExtractArgs<typename Src::Row> a{d_isa, rate, n, d_begin, d_end, d_out_off, R, seg_off, d_out};
+    prof::Scope ps(st, prof::LOCATE, 0);
+    extract_kernel<<<resident_grid(extract_kernel<Src>), EXT_THREADS, 0, st>>>(src, a);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
 }
 
 extern "C" int hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan, const void *d_occ_blob,
@@ -261,26 +391,23 @@ extern "C" int hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_pl
                    HKCSA_EINVAL, "unknown occ table layout");
     }
     if (R == 0) return HKCSA_OK;
-    HK_REQUIRE(d_begin && d_end && d_out_off && d_out && d_scratch, HKCSA_EINVAL, "null pointer");
-    uint64_t *seg_off, *bsum;
-    HK_REQUIRE(extract_scratch(R, &seg_off, &bsum, d_scratch) <= scratch_bytes, HKCSA_ESCRATCH, "extract scratch too small");
-    cudaStream_t st = as_stream(stream);
-
-    const uint32_t nb = (uint32_t)((R + SCAN_THREADS - 1) / SCAN_THREADS);
-    seg_block_sum_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum);
-    HK_LAUNCH_CHECK();
-    seg_scan_sums_kernel<<<1, SCAN_THREADS, 0, st>>>(bsum, nb);
-    HK_LAUNCH_CHECK();
-    seg_offsets_kernel<<<nb, SCAN_THREADS, 0, st>>>(d_begin, d_end, d_out_off, R, n, rate, bsum, seg_off);
-    HK_LAUNCH_CHECK();
-
-    ExtractArgs a{d_isa, rate, n, d_begin, d_end, d_out_off, R, seg_off, d_out};
-    prof::Scope ps(st, prof::LOCATE, 0);
     const auto launch = [&](auto src) {
-        extract_kernel<<<resident_grid(extract_kernel<decltype(src)>), EXT_THREADS, 0, st>>>(src, a);
-        HK_LAUNCH_CHECK();
-        return HKCSA_OK;
+        return extract_run(src, d_isa, rate, n, d_begin, d_end, d_out_off, R, d_out, d_scratch, scratch_bytes,
+                           as_stream(stream));
     };
     if (!h_occ_plan) return launch(make_wt_dev(d_wt_blob, h_wt_plan));
     return with_occ_source(d_wt_blob, h_wt_plan, d_occ_blob, h_occ_plan, launch);
+}
+
+extern "C" int hkcsa_multi_extract(const void *d_desc, uint64_t n, uint32_t rate, const uint64_t *d_isa,
+                                   const int64_t *d_begin, const int64_t *d_end, const int64_t *d_out_off, uint64_t R,
+                                   uint8_t *d_out, void *d_scratch, size_t scratch_bytes, void *stream)
+{
+    HK_REQUIRE(d_desc && d_isa, HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(rate >= 1, HKCSA_EINVAL, "sampling rate must be >= 1");
+    HK_REQUIRE(n >= 1, HKCSA_EINVAL, "empty index");
+    HK_REQUIRE(n <= (1ull << 40), HKCSA_ERANGE, "n exceeds 2^40");
+    if (R == 0) return HKCSA_OK;
+    return extract_run(MsDev{static_cast<const MultiDesc *>(d_desc)}, d_isa, rate, n, d_begin, d_end, d_out_off, R,
+                       d_out, d_scratch, scratch_bytes, as_stream(stream));
 }

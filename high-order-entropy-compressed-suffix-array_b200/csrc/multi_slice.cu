@@ -4,31 +4,13 @@
 // (occurrences of c in the slices before the one holding i) + a rank walk inside that slice, so the recurrences
 // of EnhancedFMIndex.find_range (reference csa/enhanced_fm_index.py:21-32) run unchanged on global row numbers.
 // Every GPU holds all slices (they are all-gathered after the build); patterns are sharded as in config 4.
+// The descriptor (MultiDesc) is in multi_slice.cuh; extract.cu walks the same index across slices.
 #include "common.cuh"
+#include "multi_slice.cuh"
 #include "prof.cuh"
 #include "wavelet.cuh"
 
 namespace hkcsa {
-
-struct MultiDesc {
-    WtDev slice[HKCSA_MAX_SLICES];
-    BitVec marks[HKCSA_MAX_SLICES];
-    const uint32_t *samples[HKCSA_MAX_SLICES];
-    uint64_t start[HKCSA_MAX_SLICES + 1];
-    uint64_t cum[HKCSA_MAX_SLICES + 1][256];   // occurrences of byte c in slices < s  ([S] = total)
-    uint64_t C[256];                           // symbols of the whole text smaller than byte c
-    uint32_t S;
-    uint32_t rate;                             // 0 = no sampled SA
-    uint64_t n;
-    uint64_t row0;                             // global row of suffix 0 (UINT64_MAX: no sampled SA)
-};
-
-__device__ __forceinline__ uint32_t ms_slice_of(const MultiDesc *d, uint64_t i)
-{
-    uint32_t s = 0;
-    for (uint32_t k = 1; k < d->S; ++k) s += (i >= d->start[k]) ? 1u : 0u;
-    return s;
-}
 
 // occurrences of `byte` in global rows [0, i)
 __device__ __forceinline__ uint64_t ms_rank(const MultiDesc *d, uint32_t byte, uint64_t i)
@@ -74,18 +56,7 @@ ms_locate_kernel(const MultiDesc *__restrict__ d, const uint64_t *__restrict__ r
 {
     __shared__ uint32_t s_c0, s_fix;
     const uint64_t row0 = d->row0;
-    if (threadIdx.x == 0) {             // c0 = bwt[row0] = text[n-1]; LF needs fixing iff c0 occurs before row0
-        s_c0 = 0;
-        s_fix = 0;
-        if (row0 < d->n) {
-            const uint32_t s = ms_slice_of(d, row0);
-            const WtDev &w = d->slice[s];
-            uint32_t occ0;
-            const uint32_t code = wt_access_rank(*w.tab, w, (uint32_t)(row0 - d->start[s]), occ0);
-            s_c0 = w.tab->sym_of_code[code];
-            s_fix = (d->cum[s][s_c0] + occ0) != 0;
-        }
-    }
+    if (threadIdx.x == 0) ms_suffix0(d, s_c0, s_fix);
     __syncthreads();
     const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= m) return;

@@ -47,6 +47,7 @@ struct OccDev {
     uint32_t n;
 
     using Smem = OccSmem;
+    using Row = uint32_t;
     __device__ __forceinline__ void load(OccSmem &s) const
     {
         for (uint32_t i = threadIdx.x; i < 260u; i += blockDim.x) s.C[i] = __ldg(&tab->C[i]);
@@ -105,6 +106,11 @@ struct OccDev {
             t.occ = base + __popcll(occ_match_bits<SHIFT>(x, t.sym * 0x01010101u) & ((1ull << o) - 1ull));
         }
         return t;
+    }
+    // the plain LF step of extract, as WtDev::next
+    __device__ __forceinline__ uint32_t next(const OccSmem &s, const LfStep &t, uint32_t) const
+    {
+        return s.C[t.code] + t.occ;
     }
 };
 

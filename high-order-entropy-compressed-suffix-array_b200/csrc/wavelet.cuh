@@ -56,9 +56,12 @@ struct WtDev {
     uint64_t n;
 
     using Smem = WtSmem;
+    using Row = uint32_t;
     __device__ void load(WtSmem &s) const;
     __device__ void rank2(const WtSmem &s, uint32_t code, uint32_t ch, uint32_t &a, uint32_t &b) const;
     __device__ LfStep step(const WtSmem &s, uint32_t j) const;
+    // the plain LF step of extract: LF(j) = C[code] + occ (the walk is exact when the sentinel is unique)
+    __device__ uint32_t next(const WtSmem &s, const LfStep &t, uint32_t) const { return s.C[t.code] + t.occ; }
 };
 
 static inline uint64_t rank_blocks_for(uint64_t bits) { return bits / HKCSA_BLOCK_BITS + 1; }

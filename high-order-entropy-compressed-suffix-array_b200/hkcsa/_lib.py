@@ -218,6 +218,9 @@ SIGNATURES = {
                                       C.POINTER(_vp), C.POINTER(C.POINTER(SsaPlan)), _u64, _vp, _vp]),
     "hkcsa_multi_count_batch": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),
     "hkcsa_multi_locate_rows": (_i32, [_vp, _vp, _u64, _vp, _vp]),
+    "hkcsa_multi_isa_samples": (_i32, [_u32, C.POINTER(_vp), C.POINTER(C.POINTER(SsaPlan)), C.POINTER(_u64), _vp,
+                                       _vp]),
+    "hkcsa_multi_extract": (_i32, [_vp, _u64, _u32, _vp, _vp, _vp, _vp, _u64, _vp, _vp, _sz, _vp]),
     "hkcsa_expand_ranges": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp]),
     "hkcsa_gather_u32": (_i32, [_vp, _vp, _u64, _vp, _vp]),
     "hkcsa_locate_rows": (_i32, [_vp, C.POINTER(WtPlan), _vp, C.POINTER(SsaPlan), _u32, _vp, _u64, _vp, _vp]),

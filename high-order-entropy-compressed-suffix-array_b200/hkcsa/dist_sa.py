@@ -546,6 +546,57 @@ class MultiSliceIndex:
         check(_lib.load().hkcsa_multi_locate_rows(_ptr(self.desc), _ptr(rows), rows.numel(), _ptr(out), _stream()))
         return out
 
+    # extract (csrc/extract.cu): text[begin:end) from the slices alone, with the exact LF step on every text
+    def isa_samples(self) -> torch.Tensor:
+        """int64[S + 1]: the global row of the suffix at text position k * rate for k < S = ceil(n / rate), and
+        [S] = [0].  Derived from the slices' sampled suffix arrays; built on first use."""
+        if not self.ssas:
+            raise ValueError("index was built without a sampled suffix array")
+        if getattr(self, "_isa", None) is None:
+            S = len(self.ssas)
+            out = _empty(-(-self.n // self.rate) + 1, torch.int64, self.device)
+            blobs = (C.c_void_p * S)(*[s.blob.data_ptr() for s in self.ssas])
+            plans = (C.POINTER(_lib.SsaPlan) * S)(*[C.pointer(s.plan) for s in self.ssas])
+            starts = (C.c_uint64 * (S + 1))(*self.starts)
+            check(_lib.load().hkcsa_multi_isa_samples(S, blobs, plans, starts, _ptr(out), _stream()))
+            self._isa = out
+        return self._isa
+
+    def extract_batch(self, begin: torch.Tensor, end: torch.Tensor):
+        """text[begin[q]:end[q]) for every q (int64 tensors; 0 <= begin <= end <= n, sentinel included) ->
+        (out_off int64[R+1], bytes uint8[total]) on the device, request q at bytes[out_off[q]:out_off[q+1]]."""
+        if not self.ssas:
+            raise ValueError("index was built without a sampled suffix array")
+        L = _lib.load()
+        begin = begin.to(device=self.device, dtype=torch.int64).contiguous()
+        end = end.to(device=self.device, dtype=torch.int64).contiguous()
+        if begin.shape != end.shape or begin.dim() != 1:
+            raise ValueError("begin and end must be 1-d tensors of the same length")
+        R = begin.numel()
+        out_off = torch.zeros(R + 1, dtype=torch.int64, device=self.device)
+        if R == 0:
+            return out_off, _empty(0, torch.uint8, self.device)
+        out_off[1:] = torch.cumsum(end - begin, 0)                          # plumbing: CSR offsets
+        bad = ((begin < 0) | (end < begin) | (end > self.n)).any()
+        total, bad = torch.stack([out_off[-1], bad.to(torch.int64)]).tolist()   # one read-back for both
+        if bad:
+            raise ValueError(f"extract ranges must satisfy 0 <= begin <= end <= n = {self.n}")
+        out = _empty(total, torch.uint8, self.device)
+        if total == 0:
+            return out_off, out
+        isa = self.isa_samples()
+        nbytes = L.hkcsa_extract_scratch_bytes(R)
+        scratch = _scratch(nbytes, self.device)
+        check(L.hkcsa_multi_extract(_ptr(self.desc), self.n, self.rate, _ptr(isa), _ptr(begin), _ptr(end),
+                                    _ptr(out_off), R, _ptr(out), _ptr(scratch), nbytes, _stream()))
+        return out_off, out
+
+    def extract(self, begin: int, end: int) -> torch.Tensor:
+        """text[begin:end) of the indexed text (sentinel included) as a uint8 device tensor."""
+        b = torch.tensor([begin], dtype=torch.int64, device=self.device)
+        e = torch.tensor([end], dtype=torch.int64, device=self.device)
+        return self.extract_batch(b, e)[1]
+
 
 def _sampled_sa_slice(sa_slice: torch.Tensor, rate: int):
     """Marks + samples for the rows of one slice (suffix ids are global, uint32 bit patterns)."""

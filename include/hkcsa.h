@@ -579,6 +579,27 @@ int    hkcsa_extract(const void *d_wt_blob, const hkcsa_wt_plan *h_wt_plan, cons
                      size_t scratch_bytes, void *stream);
 
 /* ------------------------------------------------------------------------ */
+/* K4c over the sliced index of the distributed build (hkcsa_multi_*).       */
+/* hkcsa_multi_isa_samples: the same isa[] as hkcsa_isa_samples, as global   */
+/* 64-bit rows, from the S slices' sampled SAs (h_starts as for              */
+/* hkcsa_multi_desc_build).  Checked on the host before any CUDA call: equal */
+/* rates, each plan's n == its slice length, the slices' n_samples add up to */
+/* ceil(n / rate) (slices of one build), ceil(n / rate) <= 2^32 (samples are */
+/* 32-bit), n <= 2^40.  d_isa: uint64[ceil(n / rate) + 1].                   */
+/* hkcsa_multi_extract: hkcsa_extract's contract (CSR output, ranges clamped */
+/* on the device, scratch from hkcsa_extract_scratch_bytes(R)) over the      */
+/* descriptor of hkcsa_multi_desc_build, which must carry the sampled SAs    */
+/* and row0; n and rate are the index's.  The LF step is the exact one of    */
+/* hkcsa_multi_locate_rows, so the bytes are the text on every text, also    */
+/* one that holds its last symbol elsewhere.                                 */
+/* ------------------------------------------------------------------------ */
+int hkcsa_multi_isa_samples(uint32_t S, const void *const *d_ssa_blobs, const hkcsa_ssa_plan *const *h_ssa_plans,
+                            const uint64_t *h_starts, uint64_t *d_isa, void *stream);
+int hkcsa_multi_extract(const void *d_desc, uint64_t n, uint32_t rate, const uint64_t *d_isa, const int64_t *d_begin,
+                        const int64_t *d_end, const int64_t *d_out_off, uint64_t R, uint8_t *d_out, void *d_scratch,
+                        size_t scratch_bytes, void *stream);
+
+/* ------------------------------------------------------------------------ */
 /* Host text in, index out: the reference's constructor takes a Python str   */
 /* (EnhancedFMIndex.__init__, csa/enhanced_fm_index.py:8-9; the corpus loader */
 /* returns one, utils/data_loader.py:4) whose bytes sit in PAGEABLE memory.   */
