@@ -206,7 +206,7 @@ __device__ __forceinline__ uint32_t lf_fix(uint32_t occ, uint32_t code, uint32_t
     if (!fix || code != c0 || j > row0) return occ;
     return j == row0 ? 0u : occ + 1u;
 }
-// the same step over 64-bit rows (the sliced index of the distributed build, csrc/multi_slice.cu)
+// the same step over 64-bit rows (MsDev, the sliced index of the distributed build: multi_slice.cuh)
 __device__ __forceinline__ uint64_t lf_fix(uint64_t occ, uint32_t code, uint64_t j, uint32_t c0, uint64_t row0,
                                            uint32_t fix)
 {

@@ -12,8 +12,8 @@
 //    text[p - 2], ... by LF steps.  Whole-text extraction is n / rate walks of <= rate steps: a parallel BWT
 //    inversion.  Adjacent threads own adjacent segments, so the byte stores of a long range land close together.
 //    The LF step comes from a source: the wavelet tree's access + rank descent or the sampled Occ table's (layouts 0
-//    and 1), with 32-bit rows and the plain step; or the sliced index (MsDev), with 64-bit global rows and the exact
-//    step, so that it gives the text back on every text.
+//    and 1), with 32-bit rows and the plain step; or the sliced index (MsDev, multi_slice.cuh), with 64-bit global
+//    rows and the exact step, so that it gives the text back on every text.
 #include "common.cuh"
 #include "multi_slice.cuh"
 #include "occ.cuh"
@@ -164,53 +164,6 @@ struct ExtractArgs {
     uint64_t R;
     const uint64_t *seg_off;
     uint8_t *out;
-};
-
-// The sliced index of the distributed build (multi_slice.cuh) as an extract source: 64-bit global rows and the
-// exact step of ms_locate_kernel.  A step finds the slice of j among the starts, runs the access + rank descent on
-// that slice's tree (node tables from global memory on the read-only path, as ms_rank) and maps the code to its
-// byte; the next row is C[c] + lf_fix(cum[s][c] + occ, ...).  The starts, C[] and cum[][] (16 KB at 8 slices) are
-// in shared memory, c0 and fix are read once per CTA from row0.
-struct MsSmem {
-    uint64_t start[HKCSA_MAX_SLICES + 1];
-    uint64_t cum[HKCSA_MAX_SLICES][256];
-    uint64_t C[256];
-    uint64_t row0;
-    uint32_t S, c0, fix;
-};
-struct MsStep {
-    uint32_t slice, sym, occ;             // occ: occurrences of sym in the slice before j
-};
-struct MsDev {
-    const MultiDesc *d;
-
-    using Smem = MsSmem;
-    using Row = uint64_t;
-    __device__ __forceinline__ void load(MsSmem &s) const
-    {
-        const uint32_t S = d->S;
-        for (uint32_t i = threadIdx.x; i < S * 256u; i += blockDim.x) (&s.cum[0][0])[i] = (&d->cum[0][0])[i];
-        for (uint32_t i = threadIdx.x; i < 256u; i += blockDim.x) s.C[i] = d->C[i];
-        for (uint32_t i = threadIdx.x; i <= S; i += blockDim.x) s.start[i] = d->start[i];
-        if (threadIdx.x == 0) {
-            s.S = S;
-            s.row0 = d->row0;
-            ms_suffix0(d, s.c0, s.fix);
-        }
-    }
-    __device__ __forceinline__ MsStep step(const MsSmem &s, uint64_t j) const
-    {
-        MsStep t;
-        t.slice = ms_slice_of(s.start, s.S, j);
-        const WtDev &w = d->slice[t.slice];
-        const uint32_t code = wt_access_rank(*w.tab, w, (uint32_t)(j - s.start[t.slice]), t.occ);
-        t.sym = __ldg(&w.tab->sym_of_code[code]);
-        return t;
-    }
-    __device__ __forceinline__ uint64_t next(const MsSmem &s, const MsStep &t, uint64_t j) const
-    {
-        return s.C[t.sym] + lf_fix(s.cum[t.slice][t.sym] + t.occ, t.sym, j, s.c0, s.row0, s.fix);
-    }
 };
 
 // the walks of every segment, grid-strided.  Each step of the source (WtDev, OccDev<SHIFT> or MsDev) gives the symbol

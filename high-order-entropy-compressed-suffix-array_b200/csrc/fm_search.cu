@@ -3,9 +3,11 @@
 // Replaces EnhancedFMIndex.find_range / .rank / .find (reference
 // csa/enhanced_fm_index.py:15-40).  occ[c][i] of build_occ (utils/utils.py:
 // 26-32) is answered by a rank source: the wavelet tree (WtDev, a rank walk that
-// reads one 32-byte block per level) or the sampled Occ table (OccDev, occ.cuh);
-// C[] and the source's tables live in shared memory.
+// reads one 32-byte block per level), the sampled Occ table (OccDev, occ.cuh) or
+// the sliced index of the distributed build (MsDev, multi_slice.cuh); C[] and the
+// source's tables live in shared memory.
 #include "common.cuh"
+#include "multi_slice.cuh"
 #include "occ.cuh"
 #include "prof.cuh"
 #include "radix_sort.cuh"
@@ -23,10 +25,18 @@ int build_markvector64(const uint64_t *d_sa, uint64_t n, uint32_t rate, RankBloc
 
 constexpr int COUNT_THREADS = 256;
 
+// the rows a search starts from: a field of the sources over one text, the last start of the sliced index
+template <typename Src>
+__device__ __forceinline__ typename Src::Row rows_of(const Src &src, const typename Src::Smem &)
+{
+    return (typename Src::Row)src.n;
+}
+__device__ __forceinline__ uint64_t rows_of(const MsDev &, const MsSmem &s) { return s.start[s.S]; }
+
 // One lane per pattern.  A warp owns a contiguous chunk of the batch and refills a lane as soon as
 // its pattern ends (last symbol consumed or range empty), so ragged lengths (8-64) and early misses do
 // not idle the warp: every iteration each busy lane consumes ONE symbol -- both boundaries of the SA
-// range take the rank step of the source together (Src: WtDev or OccDev<SHIFT>, occ.cuh).  find_range
+// range take the rank step of the source together (Src: WtDev, OccDev<SHIFT> or MsDev).  find_range
 // (csa/enhanced_fm_index.py:21-32) in half-open form:
 //   l = 0, r = n;  per symbol from the end: l = C[c] + occ(c, l), r = C[c] + occ(c, r);
 //   l >= r -> (-1, -1).  Result (l, r-1).
@@ -36,10 +46,11 @@ fm_count_kernel(Src src, const uint8_t *__restrict__ pat, const int64_t *__restr
                 int64_t *__restrict__ out_lo, int64_t *__restrict__ out_hi, const uint2 *__restrict__ kmer, uint32_t kk,
                 PeerOut po)
 {
+    using Row = typename Src::Row;
     __shared__ typename Src::Smem s;
     src.load(s);
     __syncthreads();
-    const uint32_t n = (uint32_t)src.n;
+    const Row n = rows_of(src, s);
     const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
     const uint64_t chunk = (P + nwarps - 1) / nwarps;
@@ -48,7 +59,7 @@ fm_count_kernel(Src src, const uint8_t *__restrict__ pat, const int64_t *__restr
 
     int64_t p = -1;            // pattern owned by this lane, -1 = idle
     int64_t k = 0, b = 0;      // next symbol to consume, first symbol of the pattern
-    uint32_t l = 0, r = 0;
+    Row l = 0, r = 0;
     uint32_t ch_next = 0;      // pat[k], loaded one step ahead so the step's rank loads do not wait for it
     while (true) {
         // ---- refill idle lanes with the next patterns of the chunk, in lane order
@@ -62,8 +73,9 @@ fm_count_kernel(Src src, const uint8_t *__restrict__ pat, const int64_t *__restr
                 l = 0;
                 r = n;
                 // jump table: the SA range of the pattern's last kk symbols was precomputed (by this same
-                // search) for every kk-mer over the alphabet; skip those steps
-                if (kmer != nullptr && k - b + 1 >= (int64_t)kk) {
+                // search) for every kk-mer over the alphabet; skip those steps.  Its uint2 ranges hold 32-bit rows:
+                // the sliced index has none
+                if constexpr (sizeof(Row) == 4) if (kmer != nullptr && k - b + 1 >= (int64_t)kk) {
                     uint32_t id = 0;
                     bool known = true;
                     for (uint32_t t = 0; t < kk; ++t) {
@@ -94,7 +106,7 @@ fm_count_kernel(Src src, const uint8_t *__restrict__ pat, const int64_t *__restr
             if (code == 0xFFFFu) { miss = true; }          // symbol absent: rank 0, C 0 -> empty range
             else {
                 src.rank2(s, code, ch, l, r);
-                const uint32_t c0 = s.C[code];
+                const Row c0 = s.C[code];
                 l += c0;
                 r += c0;
                 miss = l >= r;
@@ -222,6 +234,33 @@ locate_rows_kernel(Src src, BitVec marks, const uint32_t *__restrict__ samples, 
         if (steps >= rate) { out[q] = HKCSA_NO_POSITION; return; }
         const LfStep t = src.step(s, j);
         j = s.C[t.code] + lf_fix(t.occ, t.code, j, s_c0, row0, s_fix);
+        ++steps;
+    }
+}
+
+// The same walk over the sliced index (MsDev, 64-bit global rows): the marks and samples are per slice, so the slice
+// of j is looked up once per step and serves both the mark test and the LF step.
+__global__ void __launch_bounds__(256)
+ms_locate_kernel(MsDev src, const uint64_t *__restrict__ rows, uint64_t m, uint64_t *__restrict__ out)
+{
+    __shared__ MsSmem s;
+    src.load(s);
+    __syncthreads();
+    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= m) return;
+    const MultiDesc *d = src.d;
+    uint64_t j = rows[q];
+    uint32_t steps = 0;
+    while (true) {
+        const uint32_t sl = ms_slice_of(s.start, s.S, j);
+        uint64_t slot;
+        if (marked_slot(d->marks[sl], (uint32_t)(j - s.start[sl]), slot)) {
+            out[q] = (uint64_t)d->samples[sl][slot] * d->rate + steps;
+            return;
+        }
+        // as in locate_rows_kernel: the bound only keeps a walk over a corrupt index from spinning
+        if (steps >= d->rate) { out[q] = HKCSA_NO_POSITION64; return; }
+        j = src.next(s, src.step(s.start, sl, j), j);
         ++steps;
     }
 }
@@ -414,6 +453,17 @@ extern "C" int hkcsa_count_batch_peers(const void *d_wt_blob, const hkcsa_wt_pla
                                   P, nullptr, nullptr, po, st);
 }
 
+extern "C" int hkcsa_multi_count_batch(const void *d_desc, const uint8_t *d_pat, const int64_t *d_off, uint64_t P,
+                                       int64_t *d_lo, int64_t *d_hi, void *stream)
+{
+    if (P == 0) return HKCSA_OK;
+    HK_REQUIRE(d_desc && d_off && d_lo && d_hi, HKCSA_EINVAL, "null pointer");
+    PeerOut po;
+    memset(&po, 0, sizeof(po));
+    return count_launch<MsDev, 0>(MsDev{static_cast<const MultiDesc *>(d_desc)}, nullptr, 0, d_pat, d_off, P, d_lo, d_hi,
+                                  po, as_stream(stream));
+}
+
 extern "C" int hkcsa_ssa_plan_make(uint64_t n, uint32_t rate, hkcsa_ssa_plan *p)
 {
     HK_REQUIRE(p && rate >= 1, HKCSA_EINVAL, "bad argument");
@@ -567,6 +617,19 @@ extern "C" int hkcsa_locate_rows_occ(const void *d_wt_blob, const hkcsa_wt_plan 
     return with_occ_source(d_wt_blob, h_wt, d_occ_blob, p, [&](auto occ) {
         return locate_launch(occ, d_ssa_blob, h_ssa, row0, d_rows, m, d_out_pos, as_stream(stream));
     });
+}
+
+extern "C" int hkcsa_multi_locate_rows(const void *d_desc, const uint64_t *d_rows, uint64_t m, uint64_t *d_out_pos,
+                                       void *stream)
+{
+    if (m == 0) return HKCSA_OK;
+    HK_REQUIRE(d_desc && d_rows && d_out_pos, HKCSA_EINVAL, "null pointer");
+    cudaStream_t st = as_stream(stream);
+    prof::Scope ps(st, prof::LOCATE, 0);
+    ms_locate_kernel<<<(uint32_t)((m + 255) / 256), 256, 0, st>>>(MsDev{static_cast<const MultiDesc *>(d_desc)}, d_rows, m,
+                                                                 d_out_pos);
+    HK_LAUNCH_CHECK();
+    return HKCSA_OK;
 }
 
 extern "C" int hkcsa_symbol_positions(const uint8_t *d_bwt, uint64_t n, uint32_t *d_pos, uint64_t *d_start,

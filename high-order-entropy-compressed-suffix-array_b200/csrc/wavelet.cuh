@@ -132,7 +132,7 @@ __device__ __forceinline__ void wt_smem_load(WtSmem &s, const WtDev &wt)
 }
 
 // Reads of the descent tables: WtSmem is in shared memory; WtTables is the copy in global memory (the sliced index
-// of multi_slice.cu), read through the read-only path.
+// of MsDev, multi_slice.cuh), read through the read-only path.
 template <typename Tab, typename T>
 __device__ __forceinline__ T wt_ld(const T &x)
 {

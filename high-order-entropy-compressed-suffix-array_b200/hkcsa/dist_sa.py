@@ -28,7 +28,7 @@ import torch
 
 from . import _lib
 from ._lib import DsaPlan, check
-from .engine import _empty, _ptr, _scratch, _stream, byte_hist
+from .engine import _empty, _expand_ranges, _extract_requests, _ptr, _scratch, _stream, byte_hist
 
 EXT_ROUNDS_MAX = 6          # extension rounds before rank doubling takes over
 
@@ -525,15 +525,7 @@ class MultiSliceIndex:
         """CSR (offsets int64[P+1], positions int64 in SA order) through LF walks across slices."""
         if not self.ssas:
             raise ValueError("index was built without a sampled suffix array")
-        L = _lib.load()
-        lo, hi = self.count_batch(pat, off)
-        P = lo.numel()
-        cnt = torch.where(lo >= 0, hi - lo + 1, torch.zeros_like(lo))
-        out_off = torch.zeros(P + 1, dtype=torch.int64, device=self.device)
-        out_off[1:] = torch.cumsum(cnt, 0)
-        total = int(out_off[-1].item()) if P else 0
-        rows = _empty(total, torch.int64, self.device)
-        check(L.hkcsa_expand_ranges64(_ptr(lo), _ptr(hi), _ptr(out_off), P, _ptr(rows), _stream()))
+        out_off, rows = _expand_ranges(*self.count_batch(pat, off), wide=True)
         return out_off, self.locate_rows(rows)
 
     def locate_rows(self, rows: torch.Tensor) -> torch.Tensor:
@@ -568,22 +560,10 @@ class MultiSliceIndex:
         if not self.ssas:
             raise ValueError("index was built without a sampled suffix array")
         L = _lib.load()
-        begin = begin.to(device=self.device, dtype=torch.int64).contiguous()
-        end = end.to(device=self.device, dtype=torch.int64).contiguous()
-        if begin.shape != end.shape or begin.dim() != 1:
-            raise ValueError("begin and end must be 1-d tensors of the same length")
-        R = begin.numel()
-        out_off = torch.zeros(R + 1, dtype=torch.int64, device=self.device)
-        if R == 0:
-            return out_off, _empty(0, torch.uint8, self.device)
-        out_off[1:] = torch.cumsum(end - begin, 0)                          # plumbing: CSR offsets
-        bad = ((begin < 0) | (end < begin) | (end > self.n)).any()
-        total, bad = torch.stack([out_off[-1], bad.to(torch.int64)]).tolist()   # one read-back for both
-        if bad:
-            raise ValueError(f"extract ranges must satisfy 0 <= begin <= end <= n = {self.n}")
-        out = _empty(total, torch.uint8, self.device)
-        if total == 0:
+        begin, end, out_off, out = _extract_requests(begin, end, self.n, self.device)
+        if out.numel() == 0:
             return out_off, out
+        R = begin.numel()
         isa = self.isa_samples()
         nbytes = L.hkcsa_extract_scratch_bytes(R)
         scratch = _scratch(nbytes, self.device)

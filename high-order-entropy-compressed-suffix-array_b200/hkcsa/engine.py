@@ -590,6 +590,40 @@ def pack_patterns(patterns, device=None):
     return to_device_u8(flat, device), to_device_u8(off.view(np.uint8), device).view(torch.int64)
 
 
+# ------------------------------------------------------------------ query plumbing of DeviceIndex and MultiSliceIndex
+def _expand_ranges(lo: torch.Tensor, hi: torch.Tensor, wide: bool):
+    """SA ranges (lo, hi; -1: no match) -> (CSR offsets int64[P+1], their rows in SA order: int32, int64 if wide)."""
+    L = _lib.load()
+    P = lo.numel()
+    cnt = torch.where(lo >= 0, hi - lo + 1, torch.zeros_like(lo))       # plumbing: CSR offsets
+    out_off = torch.zeros(P + 1, dtype=torch.int64, device=lo.device)
+    out_off[1:] = torch.cumsum(cnt, 0)
+    total = int(out_off[-1].item()) if P else 0
+    rows = _empty(total, torch.int64 if wide else torch.int32, lo.device)
+    expand = L.hkcsa_expand_ranges64 if wide else L.hkcsa_expand_ranges
+    check(expand(_ptr(lo), _ptr(hi), _ptr(out_off), P, _ptr(rows), _stream()))
+    return out_off, rows
+
+
+def _extract_requests(begin, end, n: int, device):
+    """The requests of an extract batch -> (begin, end as int64 device tensors, out_off int64[R+1], out uint8[total]),
+    once 0 <= begin <= end <= n is checked (one read-back).  An empty `out` is already the answer."""
+    begin = begin.to(device=device, dtype=torch.int64).contiguous()
+    end = end.to(device=device, dtype=torch.int64).contiguous()
+    if begin.shape != end.shape or begin.dim() != 1:
+        raise ValueError("begin and end must be 1-d tensors of the same length")
+    R = begin.numel()
+    out_off = torch.zeros(R + 1, dtype=torch.int64, device=device)
+    if R == 0:
+        return begin, end, out_off, _empty(0, torch.uint8, device)
+    out_off[1:] = torch.cumsum(end - begin, 0)                          # plumbing: CSR offsets
+    bad = ((begin < 0) | (end < begin) | (end > n)).any()
+    total, bad = torch.stack([out_off[-1], bad.to(torch.int64)]).tolist()   # one read-back for both
+    if bad:
+        raise ValueError(f"extract ranges must satisfy 0 <= begin <= end <= n = {n}")
+    return begin, end, out_off, _empty(total, torch.uint8, device)
+
+
 @dataclass
 class BuildStats:
     sa: SaStats = field(default_factory=SaStats)
@@ -880,15 +914,7 @@ class DeviceIndex:
 
     # find, batched (csa/enhanced_fm_index.py:15-19): CSR (offsets, positions in SA order)
     def locate_batch(self, pat: torch.Tensor, off: torch.Tensor, *, use_samples: bool | None = None):
-        L = _lib.load()
-        lo, hi = self.count_batch(pat, off)
-        P = lo.numel()
-        cnt = torch.where(lo >= 0, hi - lo + 1, torch.zeros_like(lo))       # plumbing: CSR offsets
-        out_off = torch.zeros(P + 1, dtype=torch.int64, device=self.device)
-        out_off[1:] = torch.cumsum(cnt, 0)
-        total = int(out_off[-1].item()) if P else 0
-        rows = _empty(total, torch.int32, self.device)
-        check(L.hkcsa_expand_ranges(_ptr(lo), _ptr(hi), _ptr(out_off), P, _ptr(rows), _stream()))
+        out_off, rows = _expand_ranges(*self.count_batch(pat, off), wide=False)
         return out_off, self.locate_rows(rows, use_samples=use_samples)
 
     def locate_rows(self, rows: torch.Tensor, *, use_samples: bool | None = None) -> torch.Tensor:
@@ -952,25 +978,13 @@ class DeviceIndex:
         (out_off int64[R+1], bytes uint8[total]) on the device, request q at bytes[out_off[q]:out_off[q+1]].
         use_occ_table: None = LF steps on the sampled Occ table when one was built (as locate_rows), else the tree."""
         L = _lib.load()
-        begin = begin.to(device=self.device, dtype=torch.int64).contiguous()
-        end = end.to(device=self.device, dtype=torch.int64).contiguous()
-        if begin.shape != end.shape or begin.dim() != 1:
-            raise ValueError("begin and end must be 1-d tensors of the same length")
         if not self.invertible:
             raise ValueError("LF does not invert the suffix order on this index (its text holds the sentinel "
                              "elsewhere too): extract cannot give the text back")
-        R = begin.numel()
-        out_off = torch.zeros(R + 1, dtype=torch.int64, device=self.device)
-        if R == 0:
-            return out_off, _empty(0, torch.uint8, self.device)
-        out_off[1:] = torch.cumsum(end - begin, 0)                          # plumbing: CSR offsets
-        bad = ((begin < 0) | (end < begin) | (end > self.n)).any()
-        total, bad = torch.stack([out_off[-1], bad.to(torch.int64)]).tolist()   # one read-back for both
-        if bad:
-            raise ValueError(f"extract ranges must satisfy 0 <= begin <= end <= n = {self.n}")
-        out = _empty(total, torch.uint8, self.device)
-        if total == 0:
+        begin, end, out_off, out = _extract_requests(begin, end, self.n, self.device)
+        if out.numel() == 0:
             return out_off, out
+        R = begin.numel()
         occ = getattr(self, "_occ", None)
         if use_occ_table is None:
             use_occ_table = occ is not None

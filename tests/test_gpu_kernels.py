@@ -667,6 +667,13 @@ def test_multi_slice_index_matches_single_index(E, name, parts):
     o1, p1 = idx.locate_batch(d_p, d_o, use_samples=False)
     o2, p2 = ms.locate_batch(d_p, d_o)
     assert torch.equal(o1, o2) and torch.equal(p1.to(torch.int64), p2)
+    # more patterns than the count grid has lanes (148 SMs x 8 CTAs x 256 threads): lanes refill with the next
+    # pattern of their warp's chunk
+    pats, off = O.gen_patterns(10, 400_000, base, 1, 40)
+    d_p, d_o = torch.from_numpy(pats).cuda(), torch.from_numpy(off).cuda()
+    lo, hi = idx.count_batch(d_p, d_o)
+    mlo, mhi = ms.count_batch(d_p, d_o)
+    assert torch.equal(lo, mlo) and torch.equal(hi, mhi)
 
 
 def test_property_random_small_texts(E):
