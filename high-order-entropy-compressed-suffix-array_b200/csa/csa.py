@@ -69,7 +69,7 @@ class CompressedSuffixArray:
     array sampled every s = ceil((log2 n)^epsilon) text positions, so ``locate`` walks at most
     s-1 LF steps per occurrence.  The full suffix array is dropped after sampling."""
 
-    def __init__(self, text, epsilon=0.5, sa_sample_rate=None, entropy_orders=()):
+    def __init__(self, text, epsilon=0.5, sa_sample_rate=None, entropy_orders=(), *, lcp=False):
         from hkcsa import engine
         self._E = engine
         self.text = text
@@ -94,6 +94,10 @@ class CompressedSuffixArray:
         self.n = n
         # H_k of the indexed text (text + '$') for the requested orders, while the suffix array still exists
         self.entropy = {int(k): self._idx.entropy(int(k)) for k in entropy_orders}
+        # lcp=True: Sadakane's 2n-bit encoding of the LCP array, built now because it needs the text and the full SA
+        self.has_lcp = bool(lcp)
+        if self.has_lcp:
+            self._idx.build_lcp_bits()
         self._idx.text = None
         if not has_sentinel:
             self._idx.sa = None                                # the full suffix array is dropped after sampling
@@ -153,6 +157,20 @@ class CompressedSuffixArray:
         off, pos = off.cpu().numpy(), pos.cpu().numpy()
         return [sorted(pos[off[k]:off[k + 1]].tolist()) for k in range(len(off) - 1)]
 
+    def lcp(self, rows):
+        """LCP[rows] of the indexed text (text + '$') as an int64 numpy array: rows is an int or a sequence of suffix-
+        array rows in [0, n); LCP[0] = 0, LCP[r] = longest common prefix of the suffixes in rows r-1 and r.  Answered
+        from the 2n-bit encoding (needs lcp=True at construction) and a locate per row."""
+        if not self.has_lcp:
+            raise ValueError("this index holds no LCP encoding: build it with CompressedSuffixArray(..., lcp=True); "
+                             "save() does not write the encoding, so an index opened with load() has none")
+        import torch
+        r = np.atleast_1d(np.asarray(rows, dtype=np.int64))
+        if r.ndim != 1 or ((r < 0) | (r >= self.n)).any():
+            raise ValueError(f"rows must lie in [0, n) with n = {self.n}")
+        out = self._idx.lcp_rows(torch.from_numpy(r).to(self._idx.device), use_samples=self.sentinel_unique)
+        return out.cpu().numpy().astype(np.int64)
+
     def space_report(self):
         """Index size next to the entropy bound: bits per symbol of the query blob and of the entropy-coded levels
         (what save(compressed=True) writes), the sampled SA, and n*H_k for the orders given at construction
@@ -162,6 +180,8 @@ class CompressedSuffixArray:
         rep["H_k_bits_per_symbol"] = dict(self.entropy)
         rep["n_H_k_bits"] = {k: v * self.n for k, v in self.entropy.items()}
         rep["coded_index_bits_per_symbol"] = rep["coded_level_bits_per_symbol"] + rep["sampled_sa_bits_per_symbol"]
+        if self.has_lcp:
+            rep["lcp_bits_per_symbol"] = self._idx._lcp_bits_held() / max(self.n, 1)
         return rep
 
     def extract(self, start, end):
@@ -220,12 +240,14 @@ class CompressedSuffixArray:
         self._idx = engine.DeviceIndex.load(path)
         self.n = n
         self.entropy = entropy
+        self.has_lcp = False
         return self
 
     def index_bytes(self):
         """Device bytes held by the index (wavelet tree blob + sampled SA blob [+ the suffix array, kept only when
-        the text already holds the sentinel])."""
+        the text already holds the sentinel] [+ the LCP encoding, built with lcp=True])."""
         extra = self._idx.sa.numel() * 4 if self._idx.sa is not None else 0
+        extra += self._idx._lcp_bits_held() // 8
         return int(self._idx.wt.blob.numel() + self._idx.ssa.blob.numel() + extra)
 
 

@@ -27,6 +27,7 @@ class EnhancedFMIndex:
             self._text0, self._text = None, (d_text if isinstance(text, torch.Tensor) else bytes(text) + b"$")
         self._idx = engine.DeviceIndex(d_text)                       # :10-12 (SA, BWT, wavelet tree = occ)
         self._sa = None
+        self._lcp = None
         self._bwt = None
         self._occ = None
         self._str = isinstance(text, str)
@@ -48,6 +49,15 @@ class EnhancedFMIndex:
         if self._sa is None:
             self._sa = _views.int_sequence(self._idx.sa)
         return self._sa
+
+    @property
+    def lcp_array(self):
+        """LCP array of self.text in suffix-array order (no reference counterpart): lcp_array[0] = 0, lcp_array[r] =
+        longest common prefix of the suffixes at suffix_array[r-1] and suffix_array[r].  Built on the device on
+        first use."""
+        if self._lcp is None:
+            self._lcp = _views.int_sequence(self._idx.lcp())
+        return self._lcp
 
     @property
     def bwt(self):

@@ -237,6 +237,9 @@ SIGNATURES = {
     "hkcsa_wt_restore_finish": (_i32, [C.POINTER(WtPlan), _vp, _vp, _sz, _vp]),
     "hkcsa_entropy_scratch_bytes": (_sz, [_u64]),
     "hkcsa_entropy_from_sa": (_i32, [_vp, _u64, _vp, _u32, C.POINTER(C.c_double), _vp, _sz, _vp]),
+    "hkcsa_lcp_scratch_bytes": (_sz, [_u64]),
+    "hkcsa_lcp_build": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _sz, C.POINTER(_u64), _vp]),
+    "hkcsa_plcp_bits": (_i32, [_vp, _u64, _vp, _vp]),
     "hkcsa_launch_count": (C.c_ulonglong, []),
     "hkcsa_h2d_staged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "hkcsa_d2h_staged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

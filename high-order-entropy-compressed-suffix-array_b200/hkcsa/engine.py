@@ -289,6 +289,27 @@ def entropy_from_sa(text: torch.Tensor, sa: torch.Tensor, k: int) -> dict:
     return {"hk": (out[0] - out[1]) / n, "windows": int(out[2]), "contexts": int(out[3]), "grams": int(out[4])}
 
 
+def lcp_arrays(text: torch.Tensor, sa: torch.Tensor, *, lcp: bool = True, plcp: bool = False,
+               stats: list | None = None):
+    """(LCP int32[n] in suffix-array order or None, PLCP int32[n] in text order or None) of `text` from its suffix
+    array (csrc/lcp.cu).  stats: a list that receives [irreducible positions, sum of their values] (the call then
+    waits for the device)."""
+    if not (lcp or plcp):
+        raise ValueError("ask for the LCP array, the PLCP array or both")
+    L = _lib.load()
+    n = text.numel()
+    out_lcp = _empty(n, torch.int32, text.device) if lcp else None
+    out_plcp = _empty(n, torch.int32, text.device) if plcp else None
+    nbytes = L.hkcsa_lcp_scratch_bytes(n)
+    scratch = _scratch(nbytes, text.device)
+    h = (C.c_uint64 * 2)() if stats is not None else None
+    check(L.hkcsa_lcp_build(_ptr(text), n, _ptr(sa), _ptr(out_lcp), _ptr(out_plcp), _ptr(scratch), nbytes, h,
+                            _stream()))
+    if stats is not None:
+        stats[:] = [int(h[0]), int(h[1])]
+    return out_lcp, out_plcp
+
+
 def sort_pairs_u64(keys: torch.Tensor, vals: torch.Tensor, key_bits: int = 64):
     """In-place LSD onesweep radix sort of (int64-as-uint64 key, int32 value) pairs."""
     L = _lib.load()
@@ -830,6 +851,56 @@ class DeviceIndex:
         if self.sa is None or self.text is None:
             raise ValueError("H_k is computed from the text and the suffix array, which this index no longer holds")
         return entropy_from_sa(self.text, self.sa, k)["hk"]
+
+    # LCP (csrc/lcp.cu): from the text and the suffix array, or from Sadakane's 2n-bit encoding once those are gone
+    def _lcp_source(self):
+        if self.sa is None or self.text is None:
+            raise ValueError("the LCP array is computed from the text and the suffix array, which this index no "
+                             "longer holds")
+        return self.text, self.sa
+
+    def lcp(self) -> torch.Tensor:
+        """int32[n]: LCP[0] = 0, LCP[r] = longest common prefix of the suffixes in rows r-1 and r.  Not cached."""
+        return lcp_arrays(*self._lcp_source(), lcp=True)[0]
+
+    def plcp(self) -> torch.Tensor:
+        """int32[n]: PLCP[i] = LCP[ISA[i]], the LCP array in text order.  Not cached."""
+        return lcp_arrays(*self._lcp_source(), lcp=False, plcp=True)[1]
+
+    def build_lcp_bits(self) -> None:
+        """Sadakane's encoding of PLCP for lcp_rows, built while the text and the suffix array are at hand: a bit
+        vector H with a one at PLCP[i] + 2i for every i (n ones in < 2n bits).  H is kept as at most two
+        DeviceBitVectors split at HKCSA_MAX_N bits (the limit of one bit vector)."""
+        plcp = self.plcp()
+        bits = _empty(2 * self.n, torch.uint8, self.device)
+        check(_lib.load().hkcsa_plcp_bits(_ptr(plcp), self.n, _ptr(bits), _stream()))
+        del plcp
+        cut = _lib.MAX_N
+        self._lcp_bits = [DeviceBitVector(bits[a:a + cut]) for a in range(0, max(bits.numel(), 1), cut)]
+
+    def _lcp_bits_held(self) -> int:
+        """Bits held by the LCP encoding (rank blocks and directories of H); 0 before build_lcp_bits()."""
+        return sum(8 * int(v.blob.numel()) for v in getattr(self, "_lcp_bits", None) or [])
+
+    def _plcp_decode(self, pos: torch.Tensor) -> torch.Tensor:
+        """int64 PLCP[pos] from H: select(H, i + 1) - 1 - 2i, the select on the piece that holds the (i+1)-th one."""
+        pieces = self._lcp_bits
+        k = pos + 1
+        sel = pieces[0].bv_select(0, k)
+        if len(pieces) == 2:
+            first = pieces[0].ones
+            sel2 = pieces[1].bv_select(0, (k - first).clamp(min=1)) + _lib.MAX_N
+            sel = torch.where(k > first, sel2, sel)
+        return sel - 1 - 2 * pos
+
+    def lcp_rows(self, rows: torch.Tensor, *, use_samples: bool | None = None) -> torch.Tensor:
+        """int32: LCP[rows] from the encoding of build_lcp_bits(): LCP[r] = PLCP[locate(r)], the locate of
+        locate_rows (sampled or full suffix array, as it chooses)."""
+        if getattr(self, "_lcp_bits", None) is None:
+            raise ValueError("no LCP encoding: call build_lcp_bits() while the index holds its text and suffix array")
+        rows = rows.to(device=self.device, dtype=torch.int32).contiguous()
+        pos = self.locate_rows(rows, use_samples=use_samples).to(torch.int64)
+        return self._plcp_decode(pos).to(torch.int32)
 
     def psi(self) -> torch.Tensor:
         """The Psi function of the compressed suffix array (Grossi-Vitter; README.md:4 of the reference): psi[i] =

@@ -479,6 +479,27 @@ int hkcsa_entropy_from_sa(const uint8_t *d_text, uint64_t n, const uint32_t *d_s
                           void *d_scratch, size_t scratch_bytes, void *stream);
 
 /* ------------------------------------------------------------------------ */
+/* K6  LCP -- longest common prefixes of adjacent suffixes (no reference       */
+/*     counterpart).  LCP[0] = 0, LCP[r] = lcp(text[SA[r-1]:], text[SA[r]:])   */
+/*     (SA order); PLCP[i] = LCP[ISA[i]] (text order).  Any text, sentinel or  */
+/*     not; values < n, stored as uint32.  Irreducible-PLCP method            */
+/*     (Karkkainen-Manzini-Puglisi 2009): only positions i with i == 0,        */
+/*     Phi[i] == 0, text[i-1] != text[Phi[i]-1] or i == SA[0] are compared     */
+/*     (their values sum to <= 2 n log2 n), the rest by a max-scan.            */
+/*     Scratch: 4n bytes (Phi with its flag, then PLCP) + 16 bytes per position */
+/*     of a chunk of min(n, max(2^22, n/16)) positions (the lists of long      */
+/*     pairs) -- about 5n bytes beside text, SA and outputs at HKCSA_MAX_N.    */
+/* ------------------------------------------------------------------------ */
+size_t hkcsa_lcp_scratch_bytes(uint64_t n);
+/* LCP (SA order) and / or PLCP (text order) of any text from its suffix array; either output may be NULL (not both).
+   h_stats: NULL, or uint64[2] = {irreducible positions, sum of their values} (then the call syncs; otherwise it does not). */
+int hkcsa_lcp_build(const uint8_t *d_text, uint64_t n, const uint32_t *d_sa, uint32_t *d_lcp, uint32_t *d_plcp,
+                    void *d_scratch, size_t scratch_bytes, uint64_t *h_stats, void *stream);
+/* Sadakane's encoding: d_bits[PLCP[i] + 2 i] = 1 for every i, all other bytes 0; d_bits holds 2n bytes (one per bit,
+   the input format of hkcsa_bitvec_build).  Then PLCP[i] = select(i + 1) - 1 - 2 i. */
+int hkcsa_plcp_bits(const uint32_t *d_plcp, uint64_t n, uint8_t *d_bits, void *stream);
+
+/* ------------------------------------------------------------------------ */
 /* Measurement hook (no reference counterpart; the reference times with       */
 /* time.time(), tests/benchmark.py:30-35).  When enabled, the library brackets */
 /* its own kernel launches with CUDA events on the launching stream;           */
