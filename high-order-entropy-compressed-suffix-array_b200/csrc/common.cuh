@@ -169,6 +169,73 @@ __device__ __forceinline__ uint32_t warp_incl_max(uint32_t v)
     return x;
 }
 
+// ---------------------------------------------------------------- CTA-wide scans
+// Exclusive scans over one CTA (blockDim.x a multiple of 32) under an associative operator `op` with identity `id`.
+// The operator is applied in order, prefix ⊕ value, so it need not commute.  Every thread of the CTA calls them.
+template <typename T>
+__device__ __forceinline__ T shfl_up(T v, uint32_t o)
+{
+    static_assert(sizeof(T) % 4 == 0, "shuffled in 32-bit words");
+    uint32_t w[sizeof(T) / 4];
+    memcpy(w, &v, sizeof(T));
+#pragma unroll
+    for (uint32_t i = 0; i < sizeof(T) / 4; ++i) w[i] = __shfl_up_sync(0xffffffffu, w[i], o);
+    memcpy(&v, w, sizeof(T));
+    return v;
+}
+
+// the prefix of this thread's v over the CTA; total = the whole CTA's.  Ends on a barrier, so it may be called again.
+template <typename T, typename Op>
+__device__ __forceinline__ T block_excl_scan(T v, T id, Op op, T &total)
+{
+    __shared__ T s_warp[32];
+    const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
+    T x = v;
+#pragma unroll
+    for (uint32_t o = 1; o < 32; o <<= 1) {
+        const T y = shfl_up(x, o);
+        if (lane >= o) x = op(y, x);
+    }
+    const T before = shfl_up(x, 1);                  // inclusive prefix of the lane before
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    if (warp == 0) {                                 // inclusive prefixes over the warps
+        T w = lane < (blockDim.x >> 5) ? s_warp[lane] : id;
+#pragma unroll
+        for (uint32_t o = 1; o < 32; o <<= 1) {
+            const T y = shfl_up(w, o);
+            if (lane >= o) w = op(y, w);
+        }
+        s_warp[lane] = w;
+    }
+    __syncthreads();
+    total = s_warp[(blockDim.x >> 5) - 1];
+    const T pre = warp ? s_warp[warp - 1] : id;
+    __syncthreads();
+    return lane ? op(pre, before) : pre;
+}
+
+// The same scan over `count` values in rounds of blockDim.x, carried from round to round: load(i) gives value i,
+// store(i, p) takes its exclusive prefix.  Returns the total of all `count` values.
+template <typename T, typename N, typename Op, typename Load, typename Store>
+__device__ __forceinline__ T block_excl_scan_carried(N count, T id, Op op, Load load, Store store)
+{
+    T carry = id;
+    for (N base = 0; base < count; base += blockDim.x) {
+        const N i = base + threadIdx.x;
+        T total;
+        const T ex = block_excl_scan(i < count ? load(i) : id, id, op, total);
+        if (i < count) store(i, op(carry, ex));
+        carry = op(carry, total);
+    }
+    return carry;
+}
+
+struct Plus {
+    template <typename T>
+    __device__ __forceinline__ T operator()(T a, T b) const { return a + b; }
+};
+
 // ---------------------------------------------------------------- rank blocks
 // One 32-byte block: low 32 bits of word 0 = ones before the block (relative to
 // its superblock); the other 224 bits are payload.  See include/hkcsa.h.

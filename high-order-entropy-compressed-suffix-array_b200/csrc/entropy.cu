@@ -95,29 +95,11 @@ hk_count_kernel(const uint8_t *__restrict__ text, uint64_t n, const uint32_t *__
 __global__ void __launch_bounds__(1024)
 hk_scan_kernel(uint32_t *__restrict__ tile_cnt, uint32_t tiles, uint32_t *__restrict__ totals /* [3] */)
 {
-    __shared__ uint32_t s_w[32];
-    __shared__ uint32_t s_carry;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
     for (int row = 0; row < 3; ++row) {
         uint32_t *c = tile_cnt + (size_t)row * tiles;
-        if (tid == 0) s_carry = 0;
-        __syncthreads();
-        for (uint32_t base = 0; base < tiles; base += 1024) {
-            const uint32_t t = base + tid;
-            const uint32_t v = t < tiles ? c[t] : 0u;
-            uint32_t wt;
-            const uint32_t ex = warp_excl_sum(v, wt);
-            if (lane == 31) s_w[warp] = wt;
-            __syncthreads();
-            uint32_t pre = s_carry;
-            for (uint32_t w = 0; w < warp; ++w) pre += s_w[w];
-            if (t < tiles) c[t] = pre + ex;
-            __syncthreads();
-            if (tid == 1023) s_carry = pre + ex + v;
-            __syncthreads();
-        }
-        if (tid == 0) totals[row] = s_carry;
-        __syncthreads();
+        const uint32_t t = block_excl_scan_carried(tiles, 0u, Plus(), [&](uint32_t i) { return c[i]; },
+                                                   [&](uint32_t i, uint32_t p) { c[i] = p; });
+        if (threadIdx.x == 0) totals[row] = t;
     }
 }
 

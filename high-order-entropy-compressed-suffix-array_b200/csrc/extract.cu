@@ -75,34 +75,6 @@ __device__ __forceinline__ uint64_t segments_of(const ExtRange &r, uint32_t rate
 }
 
 // seg_off[q] = segments of the requests before q; three passes (block sums, scan of the block sums, block scans)
-__device__ __forceinline__ uint64_t block_excl_sum(uint64_t v, uint64_t &total)
-{
-    __shared__ uint64_t s_warp[SCAN_THREADS / 32];
-    const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
-    uint64_t x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= (uint32_t)o) x += y;
-    }
-    if (lane == 31) s_warp[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-        uint64_t w = (lane < blockDim.x / 32) ? s_warp[lane] : 0;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t y = __shfl_up_sync(0xffffffffu, w, o);
-            if (lane >= (uint32_t)o) w += y;
-        }
-        s_warp[lane] = w;                          // inclusive prefix over the warps
-    }
-    __syncthreads();
-    total = s_warp[blockDim.x / 32 - 1];
-    const uint64_t ex = x - v + (warp ? s_warp[warp - 1] : 0);
-    __syncthreads();                               // s_warp is reused by the next call
-    return ex;
-}
-
 __global__ void __launch_bounds__(SCAN_THREADS)
 seg_block_sum_kernel(const int64_t *__restrict__ begin, const int64_t *__restrict__ end,
                      const int64_t *__restrict__ out_off, uint64_t R, uint64_t n, uint32_t rate, uint64_t *__restrict__ bsum)
@@ -110,22 +82,15 @@ seg_block_sum_kernel(const int64_t *__restrict__ begin, const int64_t *__restric
     const uint64_t q = (uint64_t)blockIdx.x * SCAN_THREADS + threadIdx.x;
     const uint64_t v = q < R ? segments_of(clamp_request(begin, end, out_off, q, n), rate) : 0;
     uint64_t total;
-    block_excl_sum(v, total);
+    block_excl_scan(v, (uint64_t)0, Plus(), total);
     if (threadIdx.x == 0) bsum[blockIdx.x] = total;
 }
 
 // one CTA: exclusive prefix of the block sums in place
 __global__ void __launch_bounds__(SCAN_THREADS) seg_scan_sums_kernel(uint64_t *__restrict__ bsum, uint64_t nb)
 {
-    uint64_t carry = 0;
-    for (uint64_t i0 = 0; i0 < nb; i0 += SCAN_THREADS) {
-        const uint64_t i = i0 + threadIdx.x;
-        const uint64_t v = i < nb ? bsum[i] : 0;
-        uint64_t total;
-        const uint64_t ex = block_excl_sum(v, total);
-        if (i < nb) bsum[i] = carry + ex;
-        carry += total;
-    }
+    block_excl_scan_carried(nb, (uint64_t)0, Plus(), [&](uint64_t i) { return bsum[i]; },
+                            [&](uint64_t i, uint64_t p) { bsum[i] = p; });
 }
 
 __global__ void __launch_bounds__(SCAN_THREADS)
@@ -136,7 +101,7 @@ seg_offsets_kernel(const int64_t *__restrict__ begin, const int64_t *__restrict_
     const uint64_t q = (uint64_t)blockIdx.x * SCAN_THREADS + threadIdx.x;
     const uint64_t v = q < R ? segments_of(clamp_request(begin, end, out_off, q, n), rate) : 0;
     uint64_t total;
-    const uint64_t ex = block_excl_sum(v, total) + bsum[blockIdx.x];
+    const uint64_t ex = block_excl_scan(v, (uint64_t)0, Plus(), total) + bsum[blockIdx.x];
     if (q < R) seg_off[q] = ex;
     if (q == R - 1) seg_off[R] = ex + v;
 }

@@ -15,14 +15,6 @@
 
 namespace hkcsa {
 
-// wavelet.cu: mark bit-vector + directory + samples of the sampled suffix array in one pass over d_sa
-int build_markvector(const uint32_t *d_sa, uint64_t n, uint32_t rate, RankBlock *d_blocks, uint64_t *d_super,
-                     uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones, uint32_t *d_state,
-                     uint32_t *d_samples, cudaStream_t st);
-int build_markvector64(const uint64_t *d_sa, uint64_t n, uint32_t rate, RankBlock *d_blocks, uint64_t *d_super,
-                       uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones, uint32_t *d_state,
-                       uint32_t *d_samples, cudaStream_t st);
-
 constexpr int COUNT_THREADS = 256;
 
 // the rows a search starts from: a field of the sources over one text, the last start of the sliced index
@@ -462,86 +454,6 @@ extern "C" int hkcsa_multi_count_batch(const void *d_desc, const uint8_t *d_pat,
     memset(&po, 0, sizeof(po));
     return count_launch<MsDev, 0>(MsDev{static_cast<const MultiDesc *>(d_desc)}, nullptr, 0, d_pat, d_off, P, d_lo, d_hi,
                                   po, as_stream(stream));
-}
-
-extern "C" int hkcsa_ssa_plan_make(uint64_t n, uint32_t rate, hkcsa_ssa_plan *p)
-{
-    HK_REQUIRE(p && rate >= 1, HKCSA_EINVAL, "bad argument");
-    HK_REQUIRE(n <= HKCSA_MAX_N, HKCSA_ERANGE, "n exceeds HKCSA_MAX_N");
-    memset(p, 0, sizeof(*p));
-    p->n = n;
-    p->rate = rate;
-    p->n_samples = (n + rate - 1) / rate;
-    uint64_t off = 0;
-    p->off_blocks = off;
-    off = align_up(off + rank_blocks_for(n) * sizeof(RankBlock), 256);
-    p->off_super = off;
-    off = align_up(off + super_for(n) * sizeof(uint64_t), 256);
-    p->off_samples = off;
-    off = align_up(off + (p->n_samples + 1) * sizeof(uint32_t), 256);
-    p->blob_bytes = off;
-    Carver c(nullptr);
-    const uint64_t tiles = rank_blocks_for(n) / 64 + 2;
-    c.take<uint32_t>(tiles);
-    c.take<uint64_t>(tiles);
-    c.take<uint64_t>(8);
-    c.take<uint32_t>(select_samples_for(n));
-    c.take<uint32_t>(tiles + 1);
-    p->scratch_bytes = c.total();
-    return HKCSA_OK;
-}
-
-extern "C" int hkcsa_ssa_plan_make_slice(uint64_t m, uint32_t rate, uint64_t n_marks, hkcsa_ssa_plan *p)
-{
-    int rc = hkcsa_ssa_plan_make(m, rate, p);
-    if (rc != HKCSA_OK) return rc;
-    HK_REQUIRE(n_marks <= m, HKCSA_EINVAL, "more marks than rows");
-    p->n_samples = n_marks;
-    p->off_samples = p->off_super + align_up(super_for(m) * sizeof(uint64_t), 256);
-    p->blob_bytes = p->off_samples + align_up((n_marks + 1) * sizeof(uint32_t), 256);
-    return HKCSA_OK;
-}
-
-template <typename IdT>
-static int ssa_build_t(const IdT *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch, size_t scratch_bytes,
-                       void *stream)
-{
-    HK_REQUIRE(p && d_blob && d_scratch && (d_sa || p->n == 0), HKCSA_EINVAL, "null pointer");
-    HK_REQUIRE(p->scratch_bytes <= scratch_bytes, HKCSA_ESCRATCH, "sampled-SA scratch too small");
-    HK_REQUIRE((reinterpret_cast<uintptr_t>(d_blob) & 31) == 0, HKCSA_EINVAL, "blob must be 32-byte aligned");
-    cudaStream_t st = as_stream(stream);
-    const uint64_t n = p->n;
-    if (n == 0) return HKCSA_OK;
-    Carver c(d_scratch);
-    const uint64_t tiles = rank_blocks_for(n) / 64 + 2;
-    uint32_t *d_agg = c.take<uint32_t>(tiles);
-    uint64_t *d_carry = c.take<uint64_t>(tiles);
-    uint64_t *d_ones = c.take<uint64_t>(8);
-    uint32_t *d_sel = c.take<uint32_t>(select_samples_for(n));
-    uint32_t *d_state = c.take<uint32_t>(tiles + 1);
-    uint8_t *blob = static_cast<uint8_t *>(d_blob);
-    // one pass: ids read once (+ the marked ones again from cache), mark blocks and samples written
-    prof::Scope ps(st, prof::SSA_BUILD, n * sizeof(IdT) + n / 7 + (n / p->rate) * (4 + sizeof(IdT)));
-    RankBlock *blocks = reinterpret_cast<RankBlock *>(blob + p->off_blocks);
-    uint64_t *super = reinterpret_cast<uint64_t *>(blob + p->off_super);
-    uint32_t *samples = reinterpret_cast<uint32_t *>(blob + p->off_samples);
-    if constexpr (sizeof(IdT) == 8)
-        return build_markvector64(d_sa, n, p->rate, blocks, super, d_sel, d_agg, d_carry, d_ones, d_state, samples, st);
-    else
-        return build_markvector(d_sa, n, p->rate, blocks, super, d_sel, d_agg, d_carry, d_ones, d_state, samples, st);
-}
-
-extern "C" int hkcsa_ssa_build(const uint32_t *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch,
-                               size_t scratch_bytes, void *stream)
-{
-    return ssa_build_t<uint32_t>(d_sa, p, d_blob, d_scratch, scratch_bytes, stream);
-}
-
-// suffix ids as uint64 (slices of a text beyond 4 GB); samples stay uint32 (id / rate must fit)
-extern "C" int hkcsa_ssa_build64(const uint64_t *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch,
-                                 size_t scratch_bytes, void *stream)
-{
-    return ssa_build_t<uint64_t>(d_sa, p, d_blob, d_scratch, scratch_bytes, stream);
 }
 
 extern "C" int hkcsa_expand_ranges(const int64_t *d_lo, const int64_t *d_hi, const int64_t *d_out_off, uint64_t P,

@@ -11,9 +11,6 @@
 
 namespace hkcsa {
 
-__global__ void wt_dir_scan_kernel(const uint32_t *__restrict__ agg, uint64_t tiles, uint64_t *__restrict__ carry,
-                                   uint64_t *__restrict__ ones_out);
-
 constexpr uint32_t G_BLOCKS = 8;
 constexpr uint32_t G_BITS = G_BLOCKS * HKCSA_BLOCK_BITS;   // 1792
 constexpr uint32_t G_ALL = 1u << 31;
@@ -55,49 +52,24 @@ __global__ void golomb_tail_kernel(BitVec v, uint64_t nbits, uint64_t chunks, ui
     (void)len;
 }
 
-// carry[c] = ones immediately preceding chunk c: exclusive scan of (tail, all)
-// under (t1,a1)+(t2,a2) = (a2 ? t1+t2 : t2, a1&&a2).  Single CTA.
+// carry[c] = ones immediately preceding chunk c: exclusive scan of (tail, all) under
+// (t1,a1)+(t2,a2) = (a2 ? t1+t2 : t2, a1&&a2), identity (0, all).  On the tail[] words: the flag of a sum is the
+// left one's when the right one is all ones (a run is at most 2^30 bits, the count never reaches the flag).
+// Single CTA.
 __global__ void __launch_bounds__(1024)
 golomb_carry_kernel(const uint32_t *__restrict__ tail, uint64_t chunks, uint32_t *__restrict__ carry)
 {
-    __shared__ uint32_t s_t[32];
-    __shared__ uint32_t s_carry;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    if (tid == 0) s_carry = 0;          // (0, all=false) acts as identity on the left for lengths
-    __syncthreads();
-    for (uint64_t base = 0; base < chunks; base += 1024) {
-        const uint64_t c = base + tid;
-        const uint32_t e = (c < chunks) ? tail[c] : 0u;   // padding: (0, not all) -- only ever to the right
-        uint32_t t = e & ~G_ALL;
-        bool a = (e & G_ALL) != 0;
-        // inclusive warp scan
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t pt = __shfl_up_sync(0xffffffffu, t, o);
-            const int pa = __shfl_up_sync(0xffffffffu, (int)a, o);
-            if (lane >= (uint32_t)o) {
-                if (a) t += pt;
-                a = a && pa;
-            }
-        }
-        if (lane == 31) s_t[warp] = t | (a ? G_ALL : 0u);
-        __syncthreads();
-        // prefix over earlier warps and the running carry
-        uint32_t pt = s_carry;
-        for (uint32_t w = 0; w < warp; ++w) {
-            const uint32_t we = s_t[w];
-            pt = (we & G_ALL) ? pt + (we & ~G_ALL) : (we & ~G_ALL);
-        }
-        // inclusive value including the prefix
-        const uint32_t incl = a ? pt + t : t;
-        // exclusive = inclusive of the previous lane (or the prefix for lane 0)
-        uint32_t excl = __shfl_up_sync(0xffffffffu, incl, 1);
-        if (lane == 0) excl = pt;
-        if (c < chunks) carry[c] = excl;
-        __syncthreads();
-        if (tid == 1023) s_carry = incl;
-        __syncthreads();
-    }
+    block_excl_scan_carried(chunks, G_ALL, [](uint32_t a, uint32_t b) { return (b & G_ALL) ? a + (b & ~G_ALL) : b; },
+                            [&](uint64_t c) { return tail[c]; }, [&](uint64_t c, uint32_t p) { carry[c] = p & ~G_ALL; });
+}
+
+// off[c] = code bits of the chunks before c, *total = all of them.  Single CTA.
+__global__ void __launch_bounds__(1024)
+golomb_off_kernel(const uint32_t *__restrict__ len, uint64_t chunks, uint64_t *__restrict__ off, uint64_t *__restrict__ total)
+{
+    const uint64_t t = block_excl_scan_carried(chunks, (uint64_t)0, Plus(), [&](uint64_t c) { return (uint64_t)len[c]; },
+                                               [&](uint64_t c, uint64_t p) { off[c] = p; });
+    if (threadIdx.x == 0) *total = t;
 }
 
 template <bool EMIT>
@@ -185,7 +157,7 @@ extern "C" int hkcsa_golomb_encode(const void *d_blob, const hkcsa_wt_plan *h_pl
     HK_LAUNCH_CHECK();
     golomb_emit_kernel<false><<<grid, 128, 0, st>>>(v, nbits, chunks, m, g.carry, g.len, nullptr, nullptr);
     HK_LAUNCH_CHECK();
-    wt_dir_scan_kernel<<<1, 1024, 0, st>>>(g.len, chunks, g.off, g.total);
+    golomb_off_kernel<<<1, 1024, 0, st>>>(g.len, chunks, g.off, g.total);
     HK_LAUNCH_CHECK();
     uint64_t *h_total = reinterpret_cast<uint64_t *>(static_cast<uint8_t *>(pinned_page()) + 3584);
     HK_CUDA(cudaMemcpyAsync(h_total, g.total, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));

@@ -417,16 +417,9 @@ radix_hist_kernel(const uint64_t *__restrict__ keys, uint32_t n, uint32_t *__res
 // block p: exclusive scan of hist[p][0..255] -> base[p][0..255]
 __global__ void radix_scan_kernel(const uint32_t *__restrict__ hist, uint32_t *__restrict__ base)
 {
-    __shared__ uint32_t s_w[8];
     const uint32_t tid = threadIdx.x;
-    const uint32_t v = hist[blockIdx.x * RADIX + tid];
     uint32_t total;
-    const uint32_t ex = warp_excl_sum(v, total);
-    if ((tid & 31u) == 0) s_w[tid >> 5] = total;
-    __syncthreads();
-    uint32_t pre = 0;
-    for (uint32_t w = 0; w < (tid >> 5); ++w) pre += s_w[w];
-    base[blockIdx.x * RADIX + tid] = ex + pre;
+    base[blockIdx.x * RADIX + tid] = block_excl_scan(hist[blockIdx.x * RADIX + tid], 0u, Plus(), total);
 }
 
 size_t sort_scratch_words(uint64_t n)

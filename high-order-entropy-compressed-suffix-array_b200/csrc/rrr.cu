@@ -99,33 +99,18 @@ rrr_size_kernel(const RankBlock *__restrict__ blocks, uint64_t nbits, uint64_t n
 }
 
 // single CTA: exclusive scans of both rows into the superblock table; totals -> tot[0] (ones), tot[1] (stream bits)
+struct RrrSums {
+    uint64_t ones, bits;
+};
 __global__ void __launch_bounds__(1024)
 rrr_scan_kernel(const uint64_t *__restrict__ sb_ones, const uint64_t *__restrict__ sb_bits, uint64_t nsuper,
                 RrrSuper *__restrict__ super, uint64_t *__restrict__ tot)
 {
-    __shared__ uint64_t s_a[32], s_b[32];
-    __shared__ uint64_t s_ca, s_cb;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    if (tid == 0) { s_ca = 0; s_cb = 0; }
-    __syncthreads();
-    for (uint64_t base = 0; base < nsuper; base += 1024) {
-        const uint64_t i = base + tid;
-        const uint64_t a = i < nsuper ? sb_ones[i] : 0ull, b = i < nsuper ? sb_bits[i] : 0ull;
-        uint64_t xa = a, xb = b;
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t ya = __shfl_up_sync(0xffffffffu, xa, o), yb = __shfl_up_sync(0xffffffffu, xb, o);
-            if (lane >= (uint32_t)o) { xa += ya; xb += yb; }
-        }
-        if (lane == 31) { s_a[warp] = xa; s_b[warp] = xb; }
-        __syncthreads();
-        uint64_t pa = s_ca, pb = s_cb;
-        for (uint32_t w = 0; w < warp; ++w) { pa += s_a[w]; pb += s_b[w]; }
-        if (i < nsuper) { super[i].ones = (uint32_t)(pa + xa - a); super[i].bitpos = (uint32_t)(pb + xb - b); }
-        __syncthreads();
-        if (tid == 1023) { s_ca = pa + xa; s_cb = pb + xb; }
-        __syncthreads();
-    }
-    if (tid == 0) { tot[0] = s_ca; tot[1] = s_cb; }
+    const RrrSums t = block_excl_scan_carried(
+        nsuper, RrrSums{0, 0}, [](RrrSums a, RrrSums b) { return RrrSums{a.ones + b.ones, a.bits + b.bits}; },
+        [&](uint64_t i) { return RrrSums{sb_ones[i], sb_bits[i]}; },
+        [&](uint64_t i, RrrSums p) { super[i] = RrrSuper{(uint32_t)p.ones, (uint32_t)p.bits}; });
+    if (threadIdx.x == 0) { tot[0] = t.ones; tot[1] = t.bits; }
 }
 
 // pass 2: classes (a thread owns the 32 class bytes of its superblock) and offsets (shared words: atomicOr)

@@ -142,8 +142,7 @@ __global__ void __launch_bounds__(1024)
 gram_scan_kernel(const uint32_t *__restrict__ gh, uint32_t G, uint64_t smooth, uint64_t *__restrict__ cum,
                  uint64_t *__restrict__ ctot)
 {
-    __shared__ uint64_t s_w[32];
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t tid = threadIdx.x;
     const uint32_t g0 = blockIdx.x * GRAM_CHUNK + tid * 4u;
     uint64_t w[4] = {0, 0, 0, 0};
     if (g0 + 4 <= G && (G & 3u) == 0) {
@@ -152,22 +151,13 @@ gram_scan_kernel(const uint32_t *__restrict__ gh, uint32_t G, uint64_t smooth, u
     } else {
         for (int q = 0; q < 4; ++q) if (g0 + q < G) w[q] = 16ull * gh[g0 + q] + smooth;
     }
-    const uint64_t sum = w[0] + w[1] + w[2] + w[3];
-    uint64_t x = sum;
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= (uint32_t)o) x += y;
-    }
-    if (lane == 31) s_w[warp] = x;
-    __syncthreads();
-    uint64_t pre = 0;
-    for (uint32_t q = 0; q < warp; ++q) pre += s_w[q];
-    uint64_t run = pre + x - sum;
+    uint64_t total;
+    uint64_t run = block_excl_scan(w[0] + w[1] + w[2] + w[3], (uint64_t)0, Plus(), total);
     for (int q = 0; q < 4; ++q) {
         if (g0 + q < G) cum[g0 + q] = run;
         run += w[q];
     }
-    if (tid == 1023) ctot[blockIdx.x] = pre + x;
+    if (tid == 0) ctot[blockIdx.x] = total;
 }
 
 // every leaf walks down from the root: a node [lo, hi) splits where its two halves weigh most alike (binary search on

@@ -18,17 +18,44 @@ namespace hkcsa {
 constexpr int WTP_THREADS = 256;
 constexpr int WTP_BLOCKS_PER_CTA = 64;                                   // rank blocks per CTA
 constexpr int WTP_SYMS = WTP_BLOCKS_PER_CTA * (int)HKCSA_BLOCK_BITS;     // 14336 symbols per CTA
-static_assert(HKCSA_SUPER_BLOCKS % WTP_BLOCKS_PER_CTA == 0, "superblocks must start on a CTA tile");
 
-// Packs one level: bit j = lut_bit[sym[j]]; writes rank blocks whose header is
-// the count of ones before the block INSIDE this CTA's tile; tile totals go to agg.
+// Stores a tile of WTP_BLOCKS_PER_CTA rank blocks from its 448 payload words in shared memory, 7 per block: threads
+// 0..63 write one block each, whose header is the count of ones before the block INSIDE the tile; the tile's ones go
+// to agg[tile].
+__device__ __forceinline__ void dir_store_tile(const uint32_t *s_words, RankBlock *__restrict__ blocks, uint64_t nblocks,
+                                               uint32_t tile, uint32_t *__restrict__ agg)
+{
+    __shared__ uint32_t s_wsum[2];
+    const uint32_t tid = threadIdx.x;
+    const uint64_t gb = (uint64_t)tile * WTP_BLOCKS_PER_CTA + tid;
+    uint32_t w[7] = {0, 0, 0, 0, 0, 0, 0};
+    uint32_t cnt = 0;
+    if (tid < WTP_BLOCKS_PER_CTA) {
+#pragma unroll
+        for (int t = 0; t < 7; ++t) { w[t] = s_words[tid * 7 + t]; cnt += __popc(w[t]); }
+    }
+    uint32_t wtot;
+    const uint32_t ex = warp_excl_sum(cnt, wtot);
+    if ((tid & 31u) == 31u && tid < WTP_BLOCKS_PER_CTA) s_wsum[tid >> 5] = wtot;
+    __syncthreads();
+    if (tid < WTP_BLOCKS_PER_CTA) {
+        const uint32_t rel = ex + ((tid >= 32) ? s_wsum[0] : 0u);
+        if (gb < nblocks) {
+            uint4 *dst = reinterpret_cast<uint4 *>(blocks + gb);
+            dst[0] = make_uint4(rel, w[0], w[1], w[2]);
+            dst[1] = make_uint4(w[3], w[4], w[5], w[6]);
+        }
+        if (tid == WTP_BLOCKS_PER_CTA - 1) agg[tile] = rel + cnt;
+    }
+}
+
+// Packs one level: bit j = lut_bit[sym[j]]; a tile of rank blocks per CTA (dir_store_tile).
 __global__ void __launch_bounds__(WTP_THREADS)
 wt_pack_kernel(const uint8_t *__restrict__ sym, uint64_t len, const uint8_t *__restrict__ lut_bit,
                RankBlock *__restrict__ blocks, uint64_t nblocks, uint32_t *__restrict__ agg)
 {
     __shared__ uint8_t s_lut[256];
     __shared__ __align__(16) uint8_t s_bits[WTP_SYMS / 8];   // 1792 bytes, 28 per rank block
-    __shared__ uint32_t s_wsum[2];
     const uint32_t tid = threadIdx.x;
     s_lut[tid] = lut_bit[tid];
     __syncthreads();
@@ -45,62 +72,7 @@ wt_pack_kernel(const uint8_t *__restrict__ sym, uint64_t len, const uint8_t *__r
         s_bits[q] = (uint8_t)byte;
     }
     __syncthreads();
-    // threads 0..63 assemble one rank block each; the scan runs over the whole CTA
-    const uint64_t gb = (uint64_t)blockIdx.x * WTP_BLOCKS_PER_CTA + tid;
-    uint32_t w[7] = {0, 0, 0, 0, 0, 0, 0};
-    uint32_t cnt = 0;
-    if (tid < WTP_BLOCKS_PER_CTA) {
-        const uint32_t *w32 = reinterpret_cast<const uint32_t *>(s_bits + tid * 28);
-#pragma unroll
-        for (int t = 0; t < 7; ++t) { w[t] = w32[t]; cnt += __popc(w[t]); }
-    }
-    uint32_t wtot;
-    const uint32_t ex = warp_excl_sum(cnt, wtot);
-    if ((tid & 31u) == 31u && tid < WTP_BLOCKS_PER_CTA) s_wsum[tid >> 5] = wtot;
-    __syncthreads();
-    if (tid < WTP_BLOCKS_PER_CTA) {
-        const uint32_t rel = ex + ((tid >= 32) ? s_wsum[0] : 0u);
-        if (gb < nblocks) {
-            uint4 lo4, hi4;
-            lo4.x = rel; lo4.y = w[0]; lo4.z = w[1]; lo4.w = w[2];
-            hi4.x = w[3]; hi4.y = w[4]; hi4.z = w[5]; hi4.w = w[6];
-            uint4 *dst = reinterpret_cast<uint4 *>(blocks + gb);
-            dst[0] = lo4;
-            dst[1] = hi4;
-        }
-        if (tid == WTP_BLOCKS_PER_CTA - 1) agg[blockIdx.x] = rel + cnt;
-    }
-}
-
-// single CTA: exclusive scan of tile totals (uint32 in, uint64 carry out); total -> *ones_out
-__global__ void __launch_bounds__(1024)
-wt_dir_scan_kernel(const uint32_t *__restrict__ agg, uint64_t tiles, uint64_t *__restrict__ carry,
-                   uint64_t *__restrict__ ones_out)
-{
-    __shared__ uint64_t s_w[32];
-    __shared__ uint64_t s_carry;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    if (tid == 0) s_carry = 0;
-    __syncthreads();
-    for (uint64_t base = 0; base < tiles; base += 1024) {
-        const uint64_t t = base + tid;
-        const uint64_t v = (t < tiles) ? agg[t] : 0ull;
-        uint64_t x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= (uint32_t)o) x += y;
-        }
-        if (lane == 31) s_w[warp] = x;
-        __syncthreads();
-        uint64_t pre = s_carry;
-        for (uint32_t w = 0; w < warp; ++w) pre += s_w[w];
-        if (t < tiles) carry[t] = pre + x - v;
-        __syncthreads();
-        if (tid == 1023) s_carry = pre + x;
-        __syncthreads();
-    }
-    if (tid == 0) *ones_out = s_carry;
+    dir_store_tile(reinterpret_cast<const uint32_t *>(s_bits), blocks, nblocks, blockIdx.x, agg);
 }
 
 // position (0-based, within the 224 payload bits) of the r-th one (r >= 1) of a block
@@ -122,31 +94,37 @@ __device__ __forceinline__ uint32_t block_select(const RankBlock &b, uint32_t r)
     return HKCSA_BLOCK_BITS;   // not found
 }
 
-// Turns tile-relative headers into superblock-relative ones, writes the
-// superblock counts and the select samples.
-__global__ void __launch_bounds__(256)
-wt_dir_fix_kernel(RankBlock *__restrict__ blocks, uint64_t nblocks, const uint64_t *__restrict__ carry,
-                  uint64_t *__restrict__ super, uint32_t *__restrict__ select_samples, uint32_t blocks_per_tile)
+struct BlockOnes {
+    uint64_t before;   // ones before the block
+    uint32_t in;       // ones in the block
+};
+
+// Finishes rank block g (contents b) of a level whose header still counts the ones before the block inside its tile
+// of TILE blocks; carry[t] = ones before tile t of the level.  The header becomes relative to the block's superblock,
+// a superblock that starts at g gets its count, and the select sample whose one falls in the block gets its position.
+template <uint32_t TILE>
+__device__ __forceinline__ BlockOnes dir_finish_block(const RankBlock &b, uint64_t g, RankBlock *__restrict__ blocks,
+                                                      const uint64_t *__restrict__ carry, uint64_t *__restrict__ super,
+                                                      uint32_t *__restrict__ select_samples)
 {
-    const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= nblocks) return;
-    const RankBlock b = load_block(blocks + g);
+    static_assert(HKCSA_SUPER_BLOCKS % TILE == 0, "superblocks must start on a tile");
     const uint32_t rel = (uint32_t)(b.w[0] & 0xFFFFFFFFu);
-    const uint64_t abs_before = carry[g / blocks_per_tile] + rel;
+    const uint64_t before = carry[g / TILE] + rel;
     const uint64_t sb = g / HKCSA_SUPER_BLOCKS;
-    const uint64_t sb_abs = carry[sb * (HKCSA_SUPER_BLOCKS / blocks_per_tile)];
-    reinterpret_cast<uint32_t *>(blocks + g)[0] = (uint32_t)(abs_before - sb_abs);
+    const uint64_t sb_abs = carry[sb * (HKCSA_SUPER_BLOCKS / TILE)];
+    reinterpret_cast<uint32_t *>(blocks + g)[0] = (uint32_t)(before - sb_abs);
     if (g % HKCSA_SUPER_BLOCKS == 0) super[sb] = sb_abs;
     const uint32_t cnt = block_rank(b, HKCSA_BLOCK_BITS);
     if (cnt) {
-        // ones numbered abs_before+1 .. abs_before+cnt; sample t marks one number 1 + t*SAMPLE
-        const uint64_t t = (abs_before + HKCSA_SELECT_SAMPLE - 1) / HKCSA_SELECT_SAMPLE;
+        // ones numbered before+1 .. before+cnt; sample t marks one number 1 + t*SAMPLE
+        const uint64_t t = (before + HKCSA_SELECT_SAMPLE - 1) / HKCSA_SELECT_SAMPLE;
         const uint64_t k = 1 + t * HKCSA_SELECT_SAMPLE;
-        if (k <= abs_before + cnt) {
-            const uint32_t bit = block_select(b, (uint32_t)(k - abs_before));
+        if (k <= before + cnt) {
+            const uint32_t bit = block_select(b, (uint32_t)(k - before));
             select_samples[t] = (uint32_t)(g * HKCSA_BLOCK_BITS + bit);
         }
     }
+    return BlockOnes{before, cnt};
 }
 
 // ---------------------------------------------------------------- all levels in one sweep
@@ -186,26 +164,9 @@ wt_tile_hist_kernel(const uint8_t *__restrict__ sym, uint64_t n, const WtTables 
 __global__ void __launch_bounds__(1024)
 wt_tile_scan_kernel(uint32_t *__restrict__ gcnt, uint32_t tiles)
 {
-    __shared__ uint32_t s_w[32];
-    __shared__ uint32_t s_carry;
     uint32_t *row = gcnt + (size_t)blockIdx.x * (tiles + 1);
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    if (tid == 0) s_carry = 0;
-    __syncthreads();
-    for (uint32_t b = 0; b <= tiles; b += 1024) {
-        const uint32_t t = b + tid;
-        const uint32_t v = (t < tiles) ? row[t] : 0u;
-        uint32_t wtot;
-        const uint32_t ex = warp_excl_sum(v, wtot);
-        if (lane == 31) s_w[warp] = wtot;
-        __syncthreads();
-        uint32_t pre = s_carry;
-        for (uint32_t w = 0; w < warp; ++w) pre += s_w[w];
-        if (t <= tiles) row[t] = pre + ex;
-        __syncthreads();
-        if (tid == 1023) s_carry = pre + ex + v;
-        __syncthreads();
-    }
+    block_excl_scan_carried(tiles + 1, 0u, Plus(), [&](uint32_t t) { return t < tiles ? row[t] : 0u; },
+                            [&](uint32_t t, uint32_t p) { row[t] = p; });
 }
 
 struct LevelWords {
@@ -373,10 +334,10 @@ wt_levels_kernel(const uint8_t *__restrict__ sym, uint64_t n, const WtTables *__
 // Headers for a level whose payload bits are already in place: per rank block, ones before it
 // inside this CTA's 256-block tile; tile totals to agg.
 constexpr int WTC_BLOCKS_PER_CTA = 256;
-static_assert(HKCSA_SUPER_BLOCKS % WTC_BLOCKS_PER_CTA == 0, "superblocks must start on a CTA tile");
 
-// The directories of ALL levels in three launches (count, scan, fix) instead of three per level: the tiles of 256 rank
-// blocks of every level are numbered consecutively (tile0[l] = first tile of level l) in agg / carry.
+// The directories of ALL levels in three launches (count, scan, fix) instead of three per level: the tiles of rank
+// blocks of every level are numbered consecutively (tile0[l] = first tile of level l) in agg / carry.  A bit vector
+// packed by dir_store_tile is a one-level description with tiles of WTP_BLOCKS_PER_CTA blocks.
 struct DirLevels {
     RankBlock *blocks[HKCSA_MAX_LEVELS];
     uint64_t *super[HKCSA_MAX_LEVELS];
@@ -396,8 +357,7 @@ __device__ __forceinline__ uint32_t dir_level_of_tile(const DirLevels &D, uint32
 __global__ void __launch_bounds__(WTC_BLOCKS_PER_CTA)
 wt_count_all_kernel(DirLevels D, uint32_t *__restrict__ agg)
 {
-    __shared__ uint32_t s_w[8];
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t tid = threadIdx.x;
     const uint32_t l = dir_level_of_tile(D, blockIdx.x);
     RankBlock *blocks = D.blocks[l];
     const uint64_t nblocks = D.nblocks[l];
@@ -407,14 +367,10 @@ wt_count_all_kernel(DirLevels D, uint32_t *__restrict__ agg)
         const RankBlock b = load_block(blocks + g);
         cnt = block_rank(b, HKCSA_BLOCK_BITS);
     }
-    uint32_t wt;
-    const uint32_t ex = warp_excl_sum(cnt, wt);
-    if (lane == 31) s_w[warp] = wt;
-    __syncthreads();
-    uint32_t p = 0;
-    for (uint32_t q = 0; q < warp; ++q) p += s_w[q];
-    if (g < nblocks) reinterpret_cast<uint32_t *>(blocks + g)[0] = p + ex;
-    if (tid == WTC_BLOCKS_PER_CTA - 1) agg[blockIdx.x] = p + ex + cnt;
+    uint32_t total;
+    const uint32_t ex = block_excl_scan(cnt, 0u, Plus(), total);
+    if (g < nblocks) reinterpret_cast<uint32_t *>(blocks + g)[0] = ex;
+    if (tid == 0) agg[blockIdx.x] = total;
 }
 
 // CTA l: exclusive scan of level l's tile totals -> carry (same numbering); ones of the level -> ones_out[l]
@@ -422,59 +378,23 @@ __global__ void __launch_bounds__(1024)
 wt_dir_scan_all_kernel(DirLevels D, const uint32_t *__restrict__ agg, uint64_t *__restrict__ carry,
                        uint64_t *__restrict__ ones_out)
 {
-    __shared__ uint64_t s_w[32];
-    __shared__ uint64_t s_carry;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    const uint32_t l = blockIdx.x;
-    const uint32_t t0 = D.tile0[l], tiles = D.tile0[l + 1] - t0;
-    if (tid == 0) s_carry = 0;
-    __syncthreads();
-    for (uint32_t base = 0; base < tiles; base += 1024) {
-        const uint32_t t = base + tid;
-        const uint64_t v = (t < tiles) ? agg[t0 + t] : 0ull;
-        uint64_t x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= (uint32_t)o) x += y;
-        }
-        if (lane == 31) s_w[warp] = x;
-        __syncthreads();
-        uint64_t pre = s_carry;
-        for (uint32_t w = 0; w < warp; ++w) pre += s_w[w];
-        if (t < tiles) carry[t0 + t] = pre + x - v;
-        __syncthreads();
-        if (tid == 1023) s_carry = pre + x;
-        __syncthreads();
-    }
-    if (tid == 0) ones_out[l] = s_carry;
+    const uint32_t l = blockIdx.x, t0 = D.tile0[l];
+    const uint64_t ones = block_excl_scan_carried(D.tile0[l + 1] - t0, (uint64_t)0, Plus(),
+                                                  [&](uint32_t t) { return (uint64_t)agg[t0 + t]; },
+                                                  [&](uint32_t t, uint64_t p) { carry[t0 + t] = p; });
+    if (threadIdx.x == 0) ones_out[l] = ones;
 }
 
+// one thread per rank block, CTAs of 256 blocks.  With TILE = 256 CTA c is tile c, which places it in its level; a
+// description with smaller tiles has one level.
+template <uint32_t TILE>
 __global__ void __launch_bounds__(WTC_BLOCKS_PER_CTA)
 wt_dir_fix_all_kernel(DirLevels D, const uint64_t *__restrict__ carry)
 {
     const uint32_t l = dir_level_of_tile(D, blockIdx.x);
-    const uint32_t t = blockIdx.x - D.tile0[l];
-    const uint64_t g = (uint64_t)t * WTC_BLOCKS_PER_CTA + threadIdx.x;
+    const uint64_t g = (uint64_t)(blockIdx.x - D.tile0[l]) * WTC_BLOCKS_PER_CTA + threadIdx.x;
     if (g >= D.nblocks[l]) return;
-    RankBlock *blocks = D.blocks[l];
-    const uint64_t *lcarry = carry + D.tile0[l];
-    const RankBlock b = load_block(blocks + g);
-    const uint32_t rel = (uint32_t)(b.w[0] & 0xFFFFFFFFu);
-    const uint64_t abs_before = lcarry[t] + rel;
-    const uint64_t sb = g / HKCSA_SUPER_BLOCKS;
-    const uint64_t sb_abs = lcarry[sb * (HKCSA_SUPER_BLOCKS / WTC_BLOCKS_PER_CTA)];
-    reinterpret_cast<uint32_t *>(blocks + g)[0] = (uint32_t)(abs_before - sb_abs);
-    if (g % HKCSA_SUPER_BLOCKS == 0) D.super[l][sb] = sb_abs;
-    const uint32_t cnt = block_rank(b, HKCSA_BLOCK_BITS);
-    if (cnt) {
-        const uint64_t ts = (abs_before + HKCSA_SELECT_SAMPLE - 1) / HKCSA_SELECT_SAMPLE;
-        const uint64_t k = 1 + ts * HKCSA_SELECT_SAMPLE;
-        if (k <= abs_before + cnt) {
-            const uint32_t bit = block_select(b, (uint32_t)(k - abs_before));
-            D.select[l][ts] = (uint32_t)(g * HKCSA_BLOCK_BITS + bit);
-        }
-    }
+    dir_finish_block<TILE>(load_block(D.blocks[l] + g), g, D.blocks[l], carry + D.tile0[l], D.super[l], D.select[l]);
 }
 
 // node_ones[l][code] = rank1(level l, start of code's node)
@@ -577,17 +497,64 @@ wt_access_kernel(WtDev wt, const uint64_t *__restrict__ pos, uint64_t m, uint8_t
 // ------------------------------------------------------------------ host side
 using namespace hkcsa;
 
-// scratch of hkcsa_wt_build: per-symbol tile counts, directory tile aggregates and carries of all levels, ones per level
+// Directory scratch of `levels` levels of at most n bits, in tiles of `tile_blocks` rank blocks: tile totals and
+// carries (numbered as in DirLevels) and the ones of every level.
+struct DirScratch {
+    uint32_t *agg;
+    uint64_t *carry;
+    uint64_t *ones;
+};
+static DirScratch carve_dir_scratch(Carver &c, uint64_t n, uint32_t levels, uint32_t tile_blocks)
+{
+    const uint64_t tiles = levels * (rank_blocks_for(n) / tile_blocks + 2);
+    DirScratch d;
+    d.agg = c.take<uint32_t>(tiles);
+    d.carry = c.take<uint64_t>(tiles);
+    d.ones = c.take<uint64_t>(HKCSA_MAX_LEVELS);
+    return d;
+}
+
+// scratch of hkcsa_wt_build: per-symbol tile counts, then the directories of all levels
 static size_t wt_scratch_for(uint64_t n, uint32_t sigma)
 {
     Carver c(nullptr);
     const uint64_t wtiles = (n + WTL_TILE - 1) / WTL_TILE;
     c.take<uint32_t>((uint64_t)(sigma ? sigma : 1) * (wtiles + 1));
-    const uint64_t tiles = HKCSA_MAX_LEVELS * (rank_blocks_for(n) / WTC_BLOCKS_PER_CTA + 2);
-    c.take<uint32_t>(tiles);
-    c.take<uint64_t>(tiles);
-    c.take<uint64_t>(HKCSA_MAX_LEVELS);
+    carve_dir_scratch(c, n, HKCSA_MAX_LEVELS, WTC_BLOCKS_PER_CTA);
     return c.total();
+}
+
+// The blob of a plan: the node tables, then per level of level_len[l] bits (0 past the tree) its rank blocks,
+// superblocks and select samples, each 256-byte aligned.
+static void wt_layout_blob(hkcsa_wt_plan *p)
+{
+    uint64_t off = 0;
+    p->off_tables = off;
+    off = align_up(off + sizeof(WtTables), 256);
+    for (uint32_t l = 0; l < HKCSA_MAX_LEVELS; ++l) {
+        const uint64_t bits = p->level_len[l];
+        p->off_blocks[l] = off;
+        off = align_up(off + rank_blocks_for(bits) * sizeof(RankBlock), 256);
+        p->off_super[l] = off;
+        off = align_up(off + super_for(bits) * sizeof(uint64_t), 256);
+        p->off_select[l] = off;
+        off = align_up(off + select_samples_for(bits) * sizeof(uint32_t), 256);
+    }
+    p->blob_bytes = off;
+}
+
+// the one-level description of a bit vector of nbits bits packed by dir_store_tile
+static DirLevels packed_dir(RankBlock *blocks, uint64_t *super, uint32_t *select, uint64_t nbits)
+{
+    DirLevels D;
+    memset(&D, 0, sizeof(D));
+    D.levels = 1;
+    D.blocks[0] = blocks;
+    D.super[0] = super;
+    D.select[0] = select;
+    D.nblocks[0] = rank_blocks_for(nbits);
+    D.tile0[1] = (uint32_t)((D.nblocks[0] + WTP_BLOCKS_PER_CTA - 1) / WTP_BLOCKS_PER_CTA);
+    return D;
 }
 
 extern "C" int hkcsa_wt_plan_from_hist(const uint64_t h_hist[256], hkcsa_wt_plan *p)
@@ -643,20 +610,7 @@ extern "C" int hkcsa_wt_plan_from_hist(const uint64_t h_hist[256], hkcsa_wt_plan
         ++level;
     }
     p->levels = level;
-    // blob layout
-    uint64_t off = 0;
-    p->off_tables = off;
-    off = align_up(off + sizeof(WtTables), 256);
-    for (uint32_t l = 0; l < HKCSA_MAX_LEVELS; ++l) {
-        const uint64_t bits = (l < level) ? p->level_len[l] : 0;
-        p->off_blocks[l] = off;
-        off = align_up(off + rank_blocks_for(bits) * sizeof(RankBlock), 256);
-        p->off_super[l] = off;
-        off = align_up(off + super_for(bits) * sizeof(uint64_t), 256);
-        p->off_select[l] = off;
-        off = align_up(off + select_samples_for(bits) * sizeof(uint32_t), 256);
-    }
-    p->blob_bytes = off;
+    wt_layout_blob(p);
     p->scratch_bytes = wt_scratch_for(n, sigma);
     return HKCSA_OK;
 }
@@ -665,46 +619,17 @@ extern "C" int hkcsa_wt_plan_from_hist(const uint64_t h_hist[256], hkcsa_wt_plan
 // before the byte histogram is known (hkcsa_index_build)
 extern "C" size_t hkcsa_wt_blob_bound(uint64_t n)
 {
-    uint64_t off = align_up(sizeof(WtTables), 256);
-    for (uint32_t l = 0; l < HKCSA_MAX_LEVELS; ++l) {
-        off = align_up(off + rank_blocks_for(n) * sizeof(RankBlock), 256);
-        off = align_up(off + super_for(n) * sizeof(uint64_t), 256);
-        off = align_up(off + select_samples_for(n) * sizeof(uint32_t), 256);
-    }
-    return off;
+    hkcsa_wt_plan p;
+    for (uint32_t l = 0; l < HKCSA_MAX_LEVELS; ++l) p.level_len[l] = n;
+    wt_layout_blob(&p);
+    return p.blob_bytes;
 }
 extern "C" size_t hkcsa_wt_scratch_bound(uint64_t n) { return wt_scratch_for(n, 256); }
-
-// Builds one packed bit-vector with its directory from a byte sequence and a
-// byte -> bit table (shared by the wavelet levels and the sampled-SA marks).
-namespace hkcsa {
-int build_bitvector(const uint8_t *d_sym, uint64_t len, const uint8_t *d_lut_bit, RankBlock *d_blocks,
-                    uint64_t *d_super, uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones,
-                    cudaStream_t st)
-{
-    const uint64_t nblocks = rank_blocks_for(len);
-    const uint64_t tiles = (nblocks + WTP_BLOCKS_PER_CTA - 1) / WTP_BLOCKS_PER_CTA;
-    {
-        prof::Scope ps(st, prof::WT_PACK, len + len / 8);
-        wt_pack_kernel<<<(uint32_t)tiles, WTP_THREADS, 0, st>>>(d_sym, len, d_lut_bit, d_blocks, nblocks, d_agg);
-        HK_LAUNCH_CHECK();
-    }
-    {
-        prof::Scope ps(st, prof::WT_DIR, nblocks * 8);
-        wt_dir_scan_kernel<<<1, 1024, 0, st>>>(d_agg, tiles, d_carry, d_ones);
-        HK_LAUNCH_CHECK();
-        wt_dir_fix_kernel<<<(uint32_t)((nblocks + 255) / 256), 256, 0, st>>>(d_blocks, nblocks, d_carry, d_super,
-                                                                             d_select, WTP_BLOCKS_PER_CTA);
-        HK_LAUNCH_CHECK();
-    }
-    return HKCSA_OK;
-}
-}  // namespace hkcsa
 
 // Sampled suffix array with the suffix array streamed ONCE: `ssa_mark_pack_kernel` packs the mark bit-vector (bit j =
 // SA[j] % rate == 0) into rank blocks -- a thread takes four consecutive rows per step (one 16-byte load for 32-bit
 // ids), the flag nibbles of eight lanes are OR-ed into the 32-bit word of their rows with three shuffles --, the
-// single-CTA scan turns the tile totals into carries, and `ssa_fix_sample_kernel` finishes the directory and writes
+// directory scan turns the tile totals into carries, and `ssa_fix_sample_kernel` finishes the directory and writes
 // the samples SA[j] / rate of the marked rows in row order: the thread of a rank block knows the marks before it and
 // reads only the marked entries again (one in `rate`).  (A single kernel with a decoupled look-back over one counter
 // per 14336-row tile was measured first: its chain of inclusive prefixes advances 32 tiles per L2 round trip, 218 hops
@@ -785,7 +710,6 @@ ssa_mark_pack_kernel(const IdT *__restrict__ sa, uint64_t n, uint32_t rate, Rank
                      uint64_t nblocks, uint32_t *__restrict__ agg)
 {
     __shared__ uint32_t s_words[SSA_WORDS];
-    __shared__ uint32_t s_wsum[2];
     const uint32_t tid = threadIdx.x;
     const uint32_t tile = blockIdx.x;
     const uint64_t row_base = (uint64_t)tile * WTP_SYMS;
@@ -795,35 +719,12 @@ ssa_mark_pack_kernel(const IdT *__restrict__ sa, uint64_t n, uint32_t rate, Rank
     if (fast) ssa_flag_steps<IdT, POW2, true>(sa, n, row_base, rate, mask, aligned16, s_words);
     else ssa_flag_steps<IdT, POW2, false>(sa, n, row_base, rate, mask, aligned16, s_words);
     __syncthreads();
-    // threads 0..63: one rank block each (7 words), block headers relative to the tile
-    const uint64_t gb = (uint64_t)tile * WTP_BLOCKS_PER_CTA + tid;
-    uint32_t w[7] = {0, 0, 0, 0, 0, 0, 0};
-    uint32_t cnt = 0;
-    if (tid < WTP_BLOCKS_PER_CTA) {
-#pragma unroll
-        for (int t = 0; t < 7; ++t) { w[t] = s_words[tid * 7 + t]; cnt += __popc(w[t]); }
-    }
-    uint32_t wtot;
-    const uint32_t ex = warp_excl_sum(cnt, wtot);
-    if ((tid & 31u) == 31u && tid < WTP_BLOCKS_PER_CTA) s_wsum[tid >> 5] = wtot;
-    __syncthreads();
-    if (tid < WTP_BLOCKS_PER_CTA) {
-        const uint32_t rel = ex + ((tid >= 32) ? s_wsum[0] : 0u);
-        if (gb < nblocks) {
-            uint4 lo4, hi4;
-            lo4.x = rel; lo4.y = w[0]; lo4.z = w[1]; lo4.w = w[2];
-            hi4.x = w[3]; hi4.y = w[4]; hi4.z = w[5]; hi4.w = w[6];
-            uint4 *dst = reinterpret_cast<uint4 *>(blocks + gb);
-            dst[0] = lo4;
-            dst[1] = hi4;
-        }
-        if (tid == WTP_BLOCKS_PER_CTA - 1) agg[tile] = rel + cnt;
-    }
+    dir_store_tile(s_words, blocks, nblocks, tile, agg);
 }
 
-// wt_dir_fix_kernel for the mark vector, and the samples: the thread of a rank block knows the marks before it (tile
-// carry + header) and walks the block's set bits in row order: samples[marks before + k] = SA[row] / rate.  Only the
-// marked entries are read again -- one in `rate`, 7 per block at rate 32 -- so the suffix array is streamed once.
+// The directory of the mark vector (dir_finish_block), and the samples: the thread of a rank block knows the marks
+// before it and walks the block's set bits in row order: samples[marks before + k] = SA[row] / rate.  Only the marked
+// entries are read again -- one in `rate`, 7 per block at rate 32 -- so the suffix array is streamed once.
 template <typename IdT, bool POW2>
 __global__ void __launch_bounds__(256)
 ssa_fix_sample_kernel(RankBlock *__restrict__ blocks, uint64_t nblocks, const uint64_t *__restrict__ carry,
@@ -833,23 +734,11 @@ ssa_fix_sample_kernel(RankBlock *__restrict__ blocks, uint64_t nblocks, const ui
     const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= nblocks) return;
     const RankBlock b = load_block(blocks + g);
-    const uint32_t rel = (uint32_t)(b.w[0] & 0xFFFFFFFFu);
-    const uint64_t abs_before = carry[g / WTP_BLOCKS_PER_CTA] + rel;
-    const uint64_t sb = g / HKCSA_SUPER_BLOCKS;
-    const uint64_t sb_abs = carry[sb * (HKCSA_SUPER_BLOCKS / WTP_BLOCKS_PER_CTA)];
-    reinterpret_cast<uint32_t *>(blocks + g)[0] = (uint32_t)(abs_before - sb_abs);
-    if (g % HKCSA_SUPER_BLOCKS == 0) super[sb] = sb_abs;
-    const uint32_t cnt = block_rank(b, HKCSA_BLOCK_BITS);
-    if (cnt == 0) return;
-    const uint64_t ts = (abs_before + HKCSA_SELECT_SAMPLE - 1) / HKCSA_SELECT_SAMPLE;
-    const uint64_t ksel = 1 + ts * HKCSA_SELECT_SAMPLE;
-    if (ksel <= abs_before + cnt) {
-        const uint32_t bit = block_select(b, (uint32_t)(ksel - abs_before));
-        select_samples[ts] = (uint32_t)(g * HKCSA_BLOCK_BITS + bit);
-    }
+    const BlockOnes ones = dir_finish_block<WTP_BLOCKS_PER_CTA>(b, g, blocks, carry, super, select_samples);
+    if (ones.in == 0) return;
     const int sh = __ffs(rate) - 1;
     const IdT *row0 = sa + g * HKCSA_BLOCK_BITS;
-    uint32_t *out = samples + abs_before;
+    uint32_t *out = samples + ones.before;
     uint32_t k = 0;
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
@@ -863,42 +752,101 @@ ssa_fix_sample_kernel(RankBlock *__restrict__ blocks, uint64_t nblocks, const ui
         }
     }
 }
+}  // namespace hkcsa
 
-template <typename IdT>
-static int build_markvector_t(const IdT *d_sa, uint64_t n, uint32_t rate, RankBlock *d_blocks, uint64_t *d_super,
-                              uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones, uint32_t *d_state,
-                              uint32_t *d_samples, cudaStream_t st)
+// the sampled SA's scratch: the directory of the mark vector and its select samples (the blob keeps none)
+struct SsaScratch {
+    DirScratch dir;
+    uint32_t *select;
+};
+static SsaScratch carve_ssa_scratch(Carver &c, uint64_t n)
 {
-    (void)d_state;
-    const uint64_t nblocks = rank_blocks_for(n);
-    const uint64_t tiles = (nblocks + WTP_BLOCKS_PER_CTA - 1) / WTP_BLOCKS_PER_CTA;
+    SsaScratch s;
+    s.dir = carve_dir_scratch(c, n, 1, WTP_BLOCKS_PER_CTA);
+    s.select = c.take<uint32_t>(select_samples_for(n));
+    return s;
+}
+
+extern "C" int hkcsa_ssa_plan_make(uint64_t n, uint32_t rate, hkcsa_ssa_plan *p)
+{
+    HK_REQUIRE(p && rate >= 1, HKCSA_EINVAL, "bad argument");
+    HK_REQUIRE(n <= HKCSA_MAX_N, HKCSA_ERANGE, "n exceeds HKCSA_MAX_N");
+    memset(p, 0, sizeof(*p));
+    p->n = n;
+    p->rate = rate;
+    p->n_samples = (n + rate - 1) / rate;
+    uint64_t off = 0;
+    p->off_blocks = off;
+    off = align_up(off + rank_blocks_for(n) * sizeof(RankBlock), 256);
+    p->off_super = off;
+    off = align_up(off + super_for(n) * sizeof(uint64_t), 256);
+    p->off_samples = off;
+    off = align_up(off + (p->n_samples + 1) * sizeof(uint32_t), 256);
+    p->blob_bytes = off;
+    Carver c(nullptr);
+    carve_ssa_scratch(c, n);
+    p->scratch_bytes = c.total();
+    return HKCSA_OK;
+}
+
+extern "C" int hkcsa_ssa_plan_make_slice(uint64_t m, uint32_t rate, uint64_t n_marks, hkcsa_ssa_plan *p)
+{
+    int rc = hkcsa_ssa_plan_make(m, rate, p);
+    if (rc != HKCSA_OK) return rc;
+    HK_REQUIRE(n_marks <= m, HKCSA_EINVAL, "more marks than rows");
+    p->n_samples = n_marks;
+    p->off_samples = p->off_super + align_up(super_for(m) * sizeof(uint64_t), 256);
+    p->blob_bytes = p->off_samples + align_up((n_marks + 1) * sizeof(uint32_t), 256);
+    return HKCSA_OK;
+}
+
+// mark vector, directory and samples in one pass over d_sa: ids read once (+ the marked ones again from cache)
+template <typename IdT>
+static int ssa_build_t(const IdT *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch, size_t scratch_bytes,
+                       void *stream)
+{
+    HK_REQUIRE(p && d_blob && d_scratch && (d_sa || p->n == 0), HKCSA_EINVAL, "null pointer");
+    HK_REQUIRE(p->scratch_bytes <= scratch_bytes, HKCSA_ESCRATCH, "sampled-SA scratch too small");
+    HK_REQUIRE((reinterpret_cast<uintptr_t>(d_blob) & 31) == 0, HKCSA_EINVAL, "blob must be 32-byte aligned");
+    cudaStream_t st = as_stream(stream);
+    const uint64_t n = p->n;
+    const uint32_t rate = p->rate;
+    if (n == 0) return HKCSA_OK;
+    Carver c(d_scratch);
+    const SsaScratch s = carve_ssa_scratch(c, n);
+    const DirScratch &dir = s.dir;
+    uint8_t *blob = static_cast<uint8_t *>(d_blob);
+    const DirLevels D = packed_dir(reinterpret_cast<RankBlock *>(blob + p->off_blocks),
+                                   reinterpret_cast<uint64_t *>(blob + p->off_super), s.select, n);
+    RankBlock *blocks = D.blocks[0];
+    const uint64_t nblocks = D.nblocks[0];
+    uint32_t *samples = reinterpret_cast<uint32_t *>(blob + p->off_samples);
+    prof::Scope ps(st, prof::SSA_BUILD, n * sizeof(IdT) + n / 7 + (n / rate) * (4 + sizeof(IdT)));
     const bool pow2 = (rate & (rate - 1u)) == 0;
-    if (pow2) ssa_mark_pack_kernel<IdT, true><<<(uint32_t)tiles, WTP_THREADS, 0, st>>>(d_sa, n, rate, d_blocks, nblocks, d_agg);
-    else ssa_mark_pack_kernel<IdT, false><<<(uint32_t)tiles, WTP_THREADS, 0, st>>>(d_sa, n, rate, d_blocks, nblocks, d_agg);
+    if (pow2) ssa_mark_pack_kernel<IdT, true><<<D.tile0[1], WTP_THREADS, 0, st>>>(d_sa, n, rate, blocks, nblocks, dir.agg);
+    else ssa_mark_pack_kernel<IdT, false><<<D.tile0[1], WTP_THREADS, 0, st>>>(d_sa, n, rate, blocks, nblocks, dir.agg);
     HK_LAUNCH_CHECK();
-    wt_dir_scan_kernel<<<1, 1024, 0, st>>>(d_agg, tiles, d_carry, d_ones);
+    wt_dir_scan_all_kernel<<<1, 1024, 0, st>>>(D, dir.agg, dir.carry, dir.ones);
     HK_LAUNCH_CHECK();
     const uint32_t grid = (uint32_t)((nblocks + 255) / 256);
-    if (pow2) ssa_fix_sample_kernel<IdT, true><<<grid, 256, 0, st>>>(d_blocks, nblocks, d_carry, d_super, d_select, d_sa, rate, d_samples);
-    else ssa_fix_sample_kernel<IdT, false><<<grid, 256, 0, st>>>(d_blocks, nblocks, d_carry, d_super, d_select, d_sa, rate, d_samples);
+    if (pow2) ssa_fix_sample_kernel<IdT, true><<<grid, 256, 0, st>>>(blocks, nblocks, dir.carry, D.super[0], s.select, d_sa, rate, samples);
+    else ssa_fix_sample_kernel<IdT, false><<<grid, 256, 0, st>>>(blocks, nblocks, dir.carry, D.super[0], s.select, d_sa, rate, samples);
     HK_LAUNCH_CHECK();
     return HKCSA_OK;
 }
-int build_markvector(const uint32_t *d_sa, uint64_t n, uint32_t rate, RankBlock *d_blocks, uint64_t *d_super,
-                     uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones, uint32_t *d_state,
-                     uint32_t *d_samples, cudaStream_t st)
+
+extern "C" int hkcsa_ssa_build(const uint32_t *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch,
+                               size_t scratch_bytes, void *stream)
 {
-    return build_markvector_t<uint32_t>(d_sa, n, rate, d_blocks, d_super, d_select, d_agg, d_carry, d_ones, d_state,
-                                        d_samples, st);
+    return ssa_build_t<uint32_t>(d_sa, p, d_blob, d_scratch, scratch_bytes, stream);
 }
-int build_markvector64(const uint64_t *d_sa, uint64_t n, uint32_t rate, RankBlock *d_blocks, uint64_t *d_super,
-                       uint32_t *d_select, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones, uint32_t *d_state,
-                       uint32_t *d_samples, cudaStream_t st)
+
+// suffix ids as uint64 (slices of a text beyond 4 GB); samples stay uint32 (id / rate must fit)
+extern "C" int hkcsa_ssa_build64(const uint64_t *d_sa, const hkcsa_ssa_plan *p, void *d_blob, void *d_scratch,
+                                 size_t scratch_bytes, void *stream)
 {
-    return build_markvector_t<uint64_t>(d_sa, n, rate, d_blocks, d_super, d_select, d_agg, d_carry, d_ones, d_state,
-                                        d_samples, st);
+    return ssa_build_t<uint64_t>(d_sa, p, d_blob, d_scratch, scratch_bytes, stream);
 }
-}  // namespace hkcsa
 
 // host-side node tables of a plan -> the blob's table region
 static int wt_write_tables(const hkcsa_wt_plan *p, uint8_t *blob, cudaStream_t st)
@@ -953,8 +901,8 @@ static int wt_write_tables(const hkcsa_wt_plan *p, uint8_t *blob, cudaStream_t s
 
 // block headers, superblocks and select samples of every level from the payload bits in place; node_ones; syncs
 // once to read the ones per level (h_ones_out[levels])
-static int wt_build_dirs(const hkcsa_wt_plan *p, void *d_blob, uint32_t *d_agg, uint64_t *d_carry, uint64_t *d_ones,
-                         uint64_t *h_ones_out, cudaStream_t st)
+static int wt_build_dirs(const hkcsa_wt_plan *p, void *d_blob, const DirScratch &dir, uint64_t *h_ones_out,
+                         cudaStream_t st)
 {
     uint8_t *blob = static_cast<uint8_t *>(d_blob);
     WtTables *d_tab = reinterpret_cast<WtTables *>(blob + p->off_tables);
@@ -972,18 +920,18 @@ static int wt_build_dirs(const hkcsa_wt_plan *p, void *d_blob, uint32_t *d_agg, 
     }
     if (D.tile0[p->levels]) {
         prof::Scope ps(st, prof::WT_DIR, all_blocks * 72);
-        wt_count_all_kernel<<<D.tile0[p->levels], WTC_BLOCKS_PER_CTA, 0, st>>>(D, d_agg);
+        wt_count_all_kernel<<<D.tile0[p->levels], WTC_BLOCKS_PER_CTA, 0, st>>>(D, dir.agg);
         HK_LAUNCH_CHECK();
-        wt_dir_scan_all_kernel<<<p->levels, 1024, 0, st>>>(D, d_agg, d_carry, d_ones);
+        wt_dir_scan_all_kernel<<<p->levels, 1024, 0, st>>>(D, dir.agg, dir.carry, dir.ones);
         HK_LAUNCH_CHECK();
-        wt_dir_fix_all_kernel<<<D.tile0[p->levels], WTC_BLOCKS_PER_CTA, 0, st>>>(D, d_carry);
+        wt_dir_fix_all_kernel<WTC_BLOCKS_PER_CTA><<<D.tile0[p->levels], WTC_BLOCKS_PER_CTA, 0, st>>>(D, dir.carry);
         HK_LAUNCH_CHECK();
     }
     WtDev wt = make_wt_dev(d_blob, p);
     wt_node_ones_kernel<<<p->levels, 256, 0, st>>>(wt, d_tab);
     HK_LAUNCH_CHECK();
     uint64_t *h_ones = reinterpret_cast<uint64_t *>(static_cast<uint8_t *>(pinned_page()) + 3072);
-    HK_CUDA(cudaMemcpyAsync(h_ones, d_ones, p->levels * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HK_CUDA(cudaMemcpyAsync(h_ones, dir.ones, p->levels * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     HK_CUDA(cudaStreamSynchronize(st));
     for (uint32_t l = 0; l < p->levels; ++l) h_ones_out[l] = h_ones[l];
     return HKCSA_OK;
@@ -1007,10 +955,7 @@ extern "C" int hkcsa_wt_build(const uint8_t *d_sym, hkcsa_wt_plan *p, void *d_bl
     Carver c(d_scratch);
     const uint32_t wtiles = (uint32_t)((n + WTL_TILE - 1) / WTL_TILE);
     uint32_t *d_gcnt = c.take<uint32_t>((uint64_t)p->sigma * (wtiles + 1));
-    const uint64_t tiles_max = HKCSA_MAX_LEVELS * (rank_blocks_for(n) / WTC_BLOCKS_PER_CTA + 2);
-    uint32_t *d_agg = c.take<uint32_t>(tiles_max);
-    uint64_t *d_carry = c.take<uint64_t>(tiles_max);
-    uint64_t *d_ones = c.take<uint64_t>(HKCSA_MAX_LEVELS);
+    const DirScratch dir = carve_dir_scratch(c, n, HKCSA_MAX_LEVELS, WTC_BLOCKS_PER_CTA);
 
     // payload bits are OR-ed in: the level regions must start from zero
     HK_CUDA(cudaMemsetAsync(blob + p->off_blocks[0], 0, p->blob_bytes - p->off_blocks[0], st));
@@ -1025,7 +970,7 @@ extern "C" int hkcsa_wt_build(const uint8_t *d_sym, hkcsa_wt_plan *p, void *d_bl
         wt_levels_kernel<<<wtiles, WTL_THREADS, 0, st>>>(d_sym, n, d_tab, d_gcnt, wtiles, lw, p->levels, p->sigma);
         HK_LAUNCH_CHECK();
     }
-    return wt_build_dirs(p, d_blob, d_agg, d_carry, d_ones, p->level_ones, st);
+    return wt_build_dirs(p, d_blob, dir, p->level_ones, st);
 }
 
 // Restoring a blob from stored level payloads (hkcsa_rrr_restore_level): _begin writes the node tables and clears the
@@ -1051,12 +996,9 @@ extern "C" int hkcsa_wt_restore_finish(const hkcsa_wt_plan *p, void *d_blob, voi
     if (p->levels == 0 || p->n == 0) return HKCSA_OK;
     HK_REQUIRE(d_scratch && p->scratch_bytes <= scratch_bytes, HKCSA_ESCRATCH, "wavelet scratch too small");
     Carver c(d_scratch);
-    const uint64_t tiles_max = HKCSA_MAX_LEVELS * (rank_blocks_for(p->n) / WTC_BLOCKS_PER_CTA + 2);
-    uint32_t *d_agg = c.take<uint32_t>(tiles_max);
-    uint64_t *d_carry = c.take<uint64_t>(tiles_max);
-    uint64_t *d_ones = c.take<uint64_t>(HKCSA_MAX_LEVELS);
+    const DirScratch dir = carve_dir_scratch(c, p->n, HKCSA_MAX_LEVELS, WTC_BLOCKS_PER_CTA);
     uint64_t ones[HKCSA_MAX_LEVELS];
-    int rc = wt_build_dirs(p, d_blob, d_agg, d_carry, d_ones, ones, as_stream(stream));
+    int rc = wt_build_dirs(p, d_blob, dir, ones, as_stream(stream));
     if (rc != HKCSA_OK) return rc;
     for (uint32_t l = 0; l < p->levels; ++l)
         HK_REQUIRE(ones[l] == p->level_ones[l], HKCSA_EINVAL, "restored level holds a different number of ones than its plan");
@@ -1159,24 +1101,9 @@ extern "C" int hkcsa_bitvec_plan(uint64_t nbits, hkcsa_wt_plan *p)
     p->levels = 1;
     p->level_len[0] = nbits;
     p->level_nodes[0] = 1;
-    uint64_t off = 0;
-    p->off_tables = off;
-    off = align_up(off + sizeof(WtTables), 256);
-    for (uint32_t l = 0; l < HKCSA_MAX_LEVELS; ++l) {
-        const uint64_t bits = (l == 0) ? nbits : 0;
-        p->off_blocks[l] = off;
-        off = align_up(off + rank_blocks_for(bits) * sizeof(RankBlock), 256);
-        p->off_super[l] = off;
-        off = align_up(off + super_for(bits) * sizeof(uint64_t), 256);
-        p->off_select[l] = off;
-        off = align_up(off + select_samples_for(bits) * sizeof(uint32_t), 256);
-    }
-    p->blob_bytes = off;
+    wt_layout_blob(p);
     Carver c(nullptr);
-    const uint64_t tiles = rank_blocks_for(nbits) / WTP_BLOCKS_PER_CTA + 2;
-    c.take<uint32_t>(tiles);
-    c.take<uint64_t>(tiles);
-    c.take<uint64_t>(8);
+    carve_dir_scratch(c, nbits, 1, WTP_BLOCKS_PER_CTA);
     c.take<uint8_t>(256);
     p->scratch_bytes = c.total();
     return HKCSA_OK;
@@ -1190,21 +1117,31 @@ extern "C" int hkcsa_bitvec_build(const uint8_t *d_bits, hkcsa_wt_plan *p, void 
     HK_REQUIRE((reinterpret_cast<uintptr_t>(d_blob) & 31) == 0, HKCSA_EINVAL, "blob must be 32-byte aligned");
     HK_REQUIRE(d_bits || p->n == 0, HKCSA_EINVAL, "null pointer");
     cudaStream_t st = as_stream(stream);
+    const uint64_t n = p->n;
     uint8_t *blob = static_cast<uint8_t *>(d_blob);
     Carver c(d_scratch);
-    const uint64_t tiles = rank_blocks_for(p->n) / WTP_BLOCKS_PER_CTA + 2;
-    uint32_t *d_agg = c.take<uint32_t>(tiles);
-    uint64_t *d_carry = c.take<uint64_t>(tiles);
-    uint64_t *d_ones = c.take<uint64_t>(8);
+    const DirScratch dir = carve_dir_scratch(c, n, 1, WTP_BLOCKS_PER_CTA);
     uint8_t *d_lut = c.take<uint8_t>(256);
     nonzero_lut_kernel<<<1, 256, 0, st>>>(d_lut);
     HK_LAUNCH_CHECK();
-    int rc = build_bitvector(d_bits, p->n, d_lut, reinterpret_cast<RankBlock *>(blob + p->off_blocks[0]),
-                             reinterpret_cast<uint64_t *>(blob + p->off_super[0]),
-                             reinterpret_cast<uint32_t *>(blob + p->off_select[0]), d_agg, d_carry, d_ones, st);
-    if (rc != HKCSA_OK) return rc;
+    const DirLevels D = packed_dir(reinterpret_cast<RankBlock *>(blob + p->off_blocks[0]),
+                                   reinterpret_cast<uint64_t *>(blob + p->off_super[0]),
+                                   reinterpret_cast<uint32_t *>(blob + p->off_select[0]), n);
+    const uint64_t nblocks = D.nblocks[0];
+    {
+        prof::Scope ps(st, prof::WT_PACK, n + n / 8);
+        wt_pack_kernel<<<D.tile0[1], WTP_THREADS, 0, st>>>(d_bits, n, d_lut, D.blocks[0], nblocks, dir.agg);
+        HK_LAUNCH_CHECK();
+    }
+    {
+        prof::Scope ps(st, prof::WT_DIR, nblocks * 8);
+        wt_dir_scan_all_kernel<<<1, 1024, 0, st>>>(D, dir.agg, dir.carry, dir.ones);
+        HK_LAUNCH_CHECK();
+        wt_dir_fix_all_kernel<WTP_BLOCKS_PER_CTA><<<(uint32_t)((nblocks + 255) / 256), 256, 0, st>>>(D, dir.carry);
+        HK_LAUNCH_CHECK();
+    }
     uint64_t *h_ones = reinterpret_cast<uint64_t *>(static_cast<uint8_t *>(pinned_page()) + 3072);
-    HK_CUDA(cudaMemcpyAsync(h_ones, d_ones, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HK_CUDA(cudaMemcpyAsync(h_ones, dir.ones, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     HK_CUDA(cudaStreamSynchronize(st));
     p->level_ones[0] = h_ones[0];
     return HKCSA_OK;
