@@ -1319,6 +1319,7 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
             scatter_all = false;
             lz.samples = B.samples;
             lazy_index_due = true;          // bucket index + key samples are built when a look-up round actually comes
+            stats.lazy_ranks = 1;
         }
         uint32_t *cpos = B.pos[pcur ^ 1];
         uint32_t *cidx = vfree;

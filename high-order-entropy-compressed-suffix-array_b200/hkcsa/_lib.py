@@ -45,7 +45,7 @@ class SaStats(C.Structure):
         ("key_bits0", C.c_uint32),
         ("bwt_carried", C.c_uint32),
         ("gram_k", C.c_uint32),
-        ("reserved", C.c_uint32),
+        ("lazy_ranks", C.c_uint32),
     ]
 
 

@@ -85,7 +85,8 @@ typedef struct hkcsa_sa_stats {
     uint32_t key_bits0;         /* sorted bits of a round-0 key                 */
     uint32_t bwt_carried;       /* 1: the BWT came out of the round-0 sort      */
     uint32_t gram_k;            /* round-0 keys coded over k-grams (0: symbols) */
-    uint32_t reserved;
+    uint32_t lazy_ranks;        /* 1: round 0 scattered no ranks; later rounds  */
+                                /* look them up in the sorted round-0 keys      */
 } hkcsa_sa_stats;
 
 size_t hkcsa_sa_scratch_bytes(uint64_t n);
