@@ -420,8 +420,11 @@ static int dsa_refine(DsaState &S, cudaStream_t st)
     S.cidx = S.vfree;
     {
         prof::Scope ps(st, prof::SEG_APPLY, (uint64_t)m * 12);
-        seg_apply_kernel<<<tiles, SEG_THREADS, 0, st>>>(S.flags, S.sidx, S.pos, m, S.agg_head, S.agg_keep, S.sa, nullptr,
-                                                       S.cpos, S.cidx, S.grp, S.round != 0, false, nullptr, 0, nullptr);
+        if (S.round == 0)      // nothing placed yet: the survivors only
+            seg_compact0(S.flags, S.sidx, m, S.agg_head, S.agg_keep, S.cpos, S.cidx, S.grp, st);
+        else
+            seg_apply_kernel<<<tiles, SEG_THREADS, 0, st>>>(S.flags, S.sidx, S.pos, m, S.agg_head, S.agg_keep, S.sa,
+                                                           nullptr, S.cpos, S.cidx, S.grp, true, false, nullptr, 0, nullptr);
         HK_LAUNCH_CHECK();
     }
     HK_CUDA(cudaMemcpyAsync(h_m, S.counter, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
@@ -737,7 +740,7 @@ extern "C" int hkcsa_dsa_group_round(hkcsa_dsa_state *state, void *stream)
     S.pos = S.posbuf[S.pcur];
     {
         prof::Scope ps(st, prof::SA_KEYBUILD, (uint64_t)m * 48);
-        HK_CUDA(group_local_keys(S.cidx, S.grp, m, S.text, S.n, S.depth, S.ids64, S.kx, st));
+        HK_CUDA(group_local_keys(S.cidx, S.grp, m, S.text, S.n, S.depth, false, S.ids64, S.kx, st));
     }
     S.skey = S.kx;
     S.sidx = S.cidx;

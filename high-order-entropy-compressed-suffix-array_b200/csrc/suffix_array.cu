@@ -616,74 +616,107 @@ seg_reduce_kernel(const uint64_t *__restrict__ skey, uint32_t m, uint32_t *__res
 }
 
 // single CTA: exclusive (max, sum) scan over tile aggregates, in place; total keep -> *out_m.
-// Each thread scans SCAN_IPT consecutive tiles in registers, so a pass of the block covers 4096 tiles between
-// barriers.  The tiles travel between global memory and
-// the threads' blocked order through shared memory: coalesced rows of 1024 on the global side (a thread reading its
-// eight consecutive words directly touches one sector per word and lane: 65 us for the 48.8 k tiles of C2 on one SM).
-constexpr int SCAN_IPT = 4;
-constexpr int SCAN_PAD = SCAN_IPT + 1;      // blocked reads at stride 5 words: no bank conflicts (2 x 20 KB of shared memory)
+// Two levels: warp w owns a contiguous range of the tiles, reduces it, and the 32 warp totals give every warp its carry;
+// then each warp scans its range in steps of 32 lanes x SCAN_IPT tiles (16-byte loads), loading the next step before
+// it stores the current one.  (The one-level form went through the tiles 4096 at a time with four barriers and a
+// serial pass over the warp totals per step: 37 us for the 48.8 k tiles of C2.)
+constexpr int SCAN_IPT = 8;
+constexpr uint32_t SCAN_STEP = 32 * SCAN_IPT;      // tiles a warp scans per step
+
+struct ScanStep {
+    uint32_t h[SCAN_IPT], k[SCAN_IPT];
+};
+
+// tiles [i, i + SCAN_IPT) of the two arrays, zeros from `end` on (i is a multiple of 8: 32-byte aligned)
+__device__ __forceinline__ void scan_load(const uint32_t *agg_head, const uint32_t *agg_keep, uint32_t i, uint32_t end,
+                                          ScanStep &v)
+{
+    if (i + SCAN_IPT <= end) {
+#pragma unroll
+        for (int q = 0; q < SCAN_IPT; q += 4) {
+            const uint4 a = *reinterpret_cast<const uint4 *>(agg_head + i + q);
+            const uint4 b = *reinterpret_cast<const uint4 *>(agg_keep + i + q);
+            v.h[q] = a.x; v.h[q + 1] = a.y; v.h[q + 2] = a.z; v.h[q + 3] = a.w;
+            v.k[q] = b.x; v.k[q + 1] = b.y; v.k[q + 2] = b.z; v.k[q + 3] = b.w;
+        }
+    } else {
+#pragma unroll
+        for (int q = 0; q < SCAN_IPT; ++q) {
+            v.h[q] = i + q < end ? agg_head[i + q] : 0u;
+            v.k[q] = i + q < end ? agg_keep[i + q] : 0u;
+        }
+    }
+}
+
 __global__ void __launch_bounds__(1024)
 seg_scan_kernel(uint32_t *__restrict__ agg_head, uint32_t *__restrict__ agg_keep, uint32_t tiles,
                 uint32_t *__restrict__ out_m)
 {
-    __shared__ uint32_t s_bh[1024 * SCAN_PAD], s_bk[1024 * SCAN_PAD];
     __shared__ uint32_t s_h[32], s_k[32];
-    __shared__ uint32_t s_carry_h, s_carry_k;
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    if (tid == 0) { s_carry_h = 0; s_carry_k = 0; }
-    __syncthreads();
-    for (uint32_t base = 0; base < tiles; base += 1024 * SCAN_IPT) {
+    const uint32_t per = (tiles + 32 * SCAN_STEP - 1) / (32 * SCAN_STEP) * SCAN_STEP;
+    const uint32_t lo = min(warp * per, tiles), hi = min(lo + per, tiles);
+    // level 1: (max, sum) of the warp's range -- independent loads
+    uint32_t th = 0, tk = 0;
+#pragma unroll 2
+    for (uint32_t i = lo + lane * SCAN_IPT; i < hi; i += SCAN_STEP) {
+        ScanStep v;
+        scan_load(agg_head, agg_keep, i, hi, v);
 #pragma unroll
-        for (int e = 0; e < SCAN_IPT; ++e) {
-            const uint32_t j = e * 1024u + tid, t = base + j;          // tile base + j sits at thread j / IPT, slot j % IPT
-            s_bh[(j / SCAN_IPT) * SCAN_PAD + (j % SCAN_IPT)] = (t < tiles) ? agg_head[t] : 0u;
-            s_bk[(j / SCAN_IPT) * SCAN_PAD + (j % SCAN_IPT)] = (t < tiles) ? agg_keep[t] : 0u;
-        }
-        __syncthreads();
-        uint32_t h[SCAN_IPT], k[SCAN_IPT];
-        uint32_t th = 0, tk = 0;                       // this thread's (max, sum) over its tiles
-#pragma unroll
-        for (int e = 0; e < SCAN_IPT; ++e) {
-            h[e] = s_bh[tid * SCAN_PAD + e];
-            k[e] = s_bk[tid * SCAN_PAD + e];
-            th = max(th, h[e]);
-            tk += k[e];
-        }
-        const uint32_t ih = warp_incl_max(th);
-        uint32_t wk_total;
-        const uint32_t ek = warp_excl_sum(tk, wk_total);
-        const uint32_t eh = __shfl_up_sync(0xffffffffu, ih, 1);
-        const uint32_t excl_h_in_warp = lane ? eh : 0u;
-        if (lane == 31) { s_h[warp] = ih; s_k[warp] = wk_total; }
-        __syncthreads();
-        uint32_t ph = s_carry_h, pk = s_carry_k;
-        for (uint32_t w = 0; w < warp; ++w) { ph = max(ph, s_h[w]); pk += s_k[w]; }
-        uint32_t run_h = max(ph, excl_h_in_warp), run_k = pk + ek;
-#pragma unroll
-        for (int e = 0; e < SCAN_IPT; ++e) {
-            s_bh[tid * SCAN_PAD + e] = run_h;
-            s_bk[tid * SCAN_PAD + e] = run_k;
-            run_h = max(run_h, h[e]);
-            run_k += k[e];
-        }
-        __syncthreads();
-        if (tid == 1023) {
-            s_carry_h = run_h;
-            s_carry_k = run_k;
-        }
-#pragma unroll
-        for (int e = 0; e < SCAN_IPT; ++e) {
-            const uint32_t j = e * 1024u + tid, t = base + j;
-            if (t < tiles) {
-                agg_head[t] = s_bh[(j / SCAN_IPT) * SCAN_PAD + (j % SCAN_IPT)];
-                agg_keep[t] = s_bk[(j / SCAN_IPT) * SCAN_PAD + (j % SCAN_IPT)];
-            }
-        }
-        __syncthreads();
+        for (int q = 0; q < SCAN_IPT; ++q) { th = max(th, v.h[q]); tk += v.k[q]; }
     }
-    if (tid == 0) *out_m = s_carry_k;
+    th = __reduce_max_sync(0xffffffffu, th);
+    tk = __reduce_add_sync(0xffffffffu, tk);
+    if (lane == 0) { s_h[warp] = th; s_k[warp] = tk; }
+    __syncthreads();
+    uint32_t ch = __reduce_max_sync(0xffffffffu, lane < warp ? s_h[lane] : 0u);     // carry into this warp's range
+    uint32_t ck = __reduce_add_sync(0xffffffffu, lane < warp ? s_k[lane] : 0u);
+    const uint32_t total = __reduce_add_sync(0xffffffffu, s_k[lane]);
+    if (tid == 0) *out_m = total;
+    // level 2: the warp's range, one step of 32 x SCAN_IPT tiles after the other
+    ScanStep cur;
+    if (lo < hi) scan_load(agg_head, agg_keep, lo + lane * SCAN_IPT, hi, cur);
+    for (uint32_t i = lo; i < hi; i += SCAN_STEP) {
+        ScanStep nxt;
+        if (i + SCAN_STEP < hi) scan_load(agg_head, agg_keep, i + SCAN_STEP + lane * SCAN_IPT, hi, nxt);
+        uint32_t lh = 0, lk = 0;
+#pragma unroll
+        for (int q = 0; q < SCAN_IPT; ++q) { lh = max(lh, cur.h[q]); lk += cur.k[q]; }
+        const uint32_t ih = warp_incl_max(lh);
+        uint32_t step_k;
+        const uint32_t ek = warp_excl_sum(lk, step_k);
+        const uint32_t up = __shfl_up_sync(0xffffffffu, ih, 1);
+        uint32_t run_h = max(ch, lane ? up : 0u), run_k = ck + ek;
+        const uint32_t x = i + lane * SCAN_IPT;
+#pragma unroll
+        for (int q = 0; q < SCAN_IPT; ++q) {
+            const uint32_t h = cur.h[q], k = cur.k[q];
+            cur.h[q] = run_h;
+            cur.k[q] = run_k;
+            run_h = max(run_h, h);
+            run_k += k;
+        }
+        if (x + SCAN_IPT <= hi) {
+#pragma unroll
+            for (int q = 0; q < SCAN_IPT; q += 4) {
+                *reinterpret_cast<uint4 *>(agg_head + x + q) = make_uint4(cur.h[q], cur.h[q + 1], cur.h[q + 2], cur.h[q + 3]);
+                *reinterpret_cast<uint4 *>(agg_keep + x + q) = make_uint4(cur.k[q], cur.k[q + 1], cur.k[q + 2], cur.k[q + 3]);
+            }
+        } else {
+#pragma unroll
+            for (int q = 0; q < SCAN_IPT; ++q)
+                if (x + q < hi) { agg_head[x + q] = cur.h[q]; agg_keep[x + q] = cur.k[q]; }
+        }
+        ch = max(ch, __shfl_sync(0xffffffffu, ih, 31));
+        ck += step_k;
+        cur = nxt;
+    }
 }
 
+// Rounds that place suffixes (write_sa), and round 0 with ranks for every suffix (scatter_all): per element the SA slot,
+// the suffix id, the rank scatter and -- for survivors -- the compacted triple.  A thread's eight ids and slots come in
+// with 16-byte loads and its eight BWT symbols are read before anything is stored, so the random reads of a thread
+// are in flight together.
 __global__ void __launch_bounds__(SEG_THREADS, 6)
 seg_apply_kernel(const uint16_t *__restrict__ flags, const uint32_t *__restrict__ sidx,
                  const uint32_t *__restrict__ pos /* nullptr = identity */, uint32_t m,
@@ -695,20 +728,7 @@ seg_apply_kernel(const uint16_t *__restrict__ flags, const uint32_t *__restrict_
     __shared__ uint32_t s_h[SEG_THREADS / 32], s_k[SEG_THREADS / 32];
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
     const uint32_t j0 = blockIdx.x * SEG_TILE + tid * SEG_IPT;
-    bool head[SEG_IPT], single[SEG_IPT];
     const uint32_t f = flags[blockIdx.x * SEG_THREADS + tid];      // written by seg_reduce_kernel
-    // round 0 with lazy ranks: a warp whose 256 elements are all singletons (97-99.7 % of them) has nothing to write
-    // and its part of the block scan is known without shuffles: last head = its last element, nothing kept
-    if (!write_sa && !scatter_all && __all_sync(0xffffffffu, ((f >> SEG_IPT) & 0xFFu) == 0xFFu)) {
-        if (lane == 31) { s_h[warp] = j0 + SEG_IPT; s_k[warp] = 0; }
-        __syncthreads();
-        return;
-    }
-#pragma unroll
-    for (int e = 0; e < SEG_IPT; ++e) {
-        head[e] = (f >> e) & 1u;
-        single[e] = (f >> (SEG_IPT + e)) & 1u;
-    }
     // last head and survivors of this thread's eight elements straight from the flag bits
     const uint32_t h8 = f & 0xFFu, s8 = (f >> SEG_IPT) & 0xFFu;
     const uint32_t vm = (j0 + SEG_IPT <= m) ? 0xFFu : (j0 < m ? (1u << (m - j0)) - 1u : 0u);
@@ -732,39 +752,137 @@ seg_apply_kernel(const uint16_t *__restrict__ flags, const uint32_t *__restrict_
     const uint32_t wh = __shfl_sync(0xffffffffu, lasthead, hb ? 31 - __clz(hb) : 0);     // the warp's last head
     if (lane == 31) { s_h[warp] = hb ? wh : 0u; s_k[warp] = wk_total; }
     __syncthreads();
+    if (!vm) return;
     uint32_t ph = carry_head[blockIdx.x], pk = carry_keep[blockIdx.x];
     for (uint32_t w = 0; w < warp; ++w) { ph = max(ph, s_h[w]); pk += s_k[w]; }
-    // round 0 with lazy ranks: a thread whose eight elements are all singletons has nothing to write
-    if (!write_sa && !scatter_all && ((f >> SEG_IPT) & 0xFFu) == 0xFFu) return;
-    uint32_t cur_head = max(ph, eh);   // (index of governing head) + 1 before this thread's first element
+    const uint32_t head_in = max(ph, eh);   // (index of the governing head) + 1 before this thread's first element
+    uint32_t s[SEG_IPT], p[SEG_IPT];
+    if (vm == 0xFFu) {                      // j0 is a multiple of 8: 32-byte aligned
+        const uint4 *vs = reinterpret_cast<const uint4 *>(sidx + j0);
+        const uint4 a = vs[0], b = vs[1];
+        s[0] = a.x; s[1] = a.y; s[2] = a.z; s[3] = a.w; s[4] = b.x; s[5] = b.y; s[6] = b.z; s[7] = b.w;
+        if (pos) {
+            const uint4 *vp = reinterpret_cast<const uint4 *>(pos + j0);
+            const uint4 c = vp[0], d = vp[1];
+            p[0] = c.x; p[1] = c.y; p[2] = c.z; p[3] = c.w; p[4] = d.x; p[5] = d.y; p[6] = d.z; p[7] = d.w;
+        }
+    } else {
+#pragma unroll
+        for (int e = 0; e < SEG_IPT; ++e) {
+            s[e] = (vm >> e) & 1u ? sidx[j0 + e] : 0u;
+            if (pos) p[e] = (vm >> e) & 1u ? pos[j0 + e] : 0u;
+        }
+    }
+    if (!pos) {
+#pragma unroll
+        for (int e = 0; e < SEG_IPT; ++e) p[e] = j0 + e;
+    }
+    // group of the elements before this thread's first head: the slot of a head that lies in an earlier thread
+    uint32_t grp = (h8 & 1u) ? 0u : (pos ? pos[head_in - 1] : head_in - 1);
+    uint8_t c[SEG_IPT];
+    if (write_sa && bwt) {                  // BWT rows carried by round 0: this slot's row follows its suffix
+#pragma unroll
+        for (int e = 0; e < SEG_IPT; ++e) c[e] = (vm >> e) & 1u ? text[s[e] ? s[e] - 1u : n - 1u] : 0;
+    }
     uint32_t slot = pk + ek;
-    uint32_t cur_grp = 0;
-    bool grp_valid = false;
 #pragma unroll
     for (int e = 0; e < SEG_IPT; ++e) {
-        const uint32_t j = j0 + e;
-        if (j >= m) break;
-        if (head[e]) { cur_head = j + 1; grp_valid = false; }
-        if (!grp_valid) {
-            cur_grp = pos ? pos[cur_head - 1] : (cur_head - 1);
-            grp_valid = true;
-        }
-        const uint32_t p = pos ? pos[j] : j;
-        // round 0 with lazy ranks needs the suffix id of survivors only: most of the id stream is never read
-        const bool need_id = write_sa || scatter_all || !single[e];
-        const uint32_t s = need_id ? sidx[j] : 0u;
+        if (!((vm >> e) & 1u)) break;
+        if ((h8 >> e) & 1u) grp = p[e];
+        const bool single = (s8 >> e) & 1u;
         if (write_sa) {
-            sa[p] = s;
-            if (bwt) bwt[p] = text[s ? s - 1u : n - 1u];         // BWT rows carried by round 0: this slot's row follows its suffix
+            sa[p[e]] = s[e];
+            if (bwt) bwt[p[e]] = c[e];
         }
-        if (rank && (scatter_all || !single[e])) rank[s] = cur_grp;
-        if (!single[e]) {
-            cpos[slot] = p;
-            cidx[slot] = s;
-            cgrp[slot] = cur_grp;
+        if (rank && (scatter_all || !single)) rank[s[e]] = grp;
+        if (!single) {
+            cpos[slot] = p[e];
+            cidx[slot] = s[e];
+            cgrp[slot] = grp;
             ++slot;
         }
     }
+}
+
+// Round 0 without rank scatter (lazy ranks; the distributed build's first refinement): only the survivors -- 0.3-3 %
+// of the suffixes -- are written, compacted in order into (cpos, cidx, cgrp).  The flags are the whole input, so a CTA
+// covers C0_TILES scan tiles, 64 elements per thread from one 16-byte flag load; its carry is the scanned aggregate of
+// its first tile, and the prefix inside the CTA comes from the flag bits.  (One CTA per 2048-element tile made this a
+// pass of 330 CTAs per SM, each waiting on two dependent loads to find nothing to do.)
+constexpr int C0_THREADS = 512;
+constexpr int C0_IPT = 64;
+constexpr int C0_TILES = C0_THREADS * C0_IPT / SEG_TILE;
+static_assert(C0_TILES * SEG_TILE == C0_THREADS * C0_IPT && C0_IPT == 8 * SEG_IPT, "a thread reads 8 flag words");
+
+__global__ void __launch_bounds__(C0_THREADS, 3)
+seg_compact0_kernel(const uint16_t *__restrict__ flags, const uint32_t *__restrict__ sidx, uint32_t m,
+                    const uint32_t *__restrict__ carry_head, const uint32_t *__restrict__ carry_keep,
+                    uint32_t *__restrict__ cpos, uint32_t *__restrict__ cidx, uint32_t *__restrict__ cgrp)
+{
+    __shared__ uint32_t s_h[C0_THREADS / 32], s_k[C0_THREADS / 32];
+    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t j0 = blockIdx.x * (uint32_t)(C0_THREADS * C0_IPT) + tid * C0_IPT;
+    // the CTA's carry is loaded with its flags, not after the barrier: the pass is a chain of latencies per CTA
+    const uint32_t t0 = blockIdx.x * (uint32_t)C0_TILES;
+    const uint32_t carry_h = carry_head[t0], carry_k = carry_keep[t0];
+    uint64_t hm = 0, sv = 0;                // head and survivor bits of elements j0 .. j0 + 63
+    if (j0 < m) {
+        const uint4 q = *reinterpret_cast<const uint4 *>(flags + (j0 >> 3));   // 8 flag words: bit e head, 8 + e singleton
+        const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+        uint64_t single = 0;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const uint32_t f = w[i >> 1] >> (16 * (i & 1));
+            hm |= (uint64_t)(f & 0xFFu) << (8 * i);
+            single |= (uint64_t)((f >> 8) & 0xFFu) << (8 * i);
+        }
+        const uint64_t vm = (m - j0 >= (uint32_t)C0_IPT) ? ~0ull : (1ull << (m - j0)) - 1ull;
+        sv = ~single & vm;
+    }
+    const uint32_t lasthead = hm ? j0 + 64u - (uint32_t)__clzll(hm) : 0u;      // (index of the last head) + 1
+    const uint32_t ih = warp_incl_max(lasthead);
+    uint32_t wk_total;
+    const uint32_t ek = warp_excl_sum((uint32_t)__popcll(sv), wk_total);
+    const uint32_t up = __shfl_up_sync(0xffffffffu, ih, 1);
+    const uint32_t eh = lane ? up : 0u;
+    if (lane == 31) { s_h[warp] = ih; s_k[warp] = wk_total; }
+    __syncthreads();
+    if (!sv) return;
+    uint32_t ph = carry_h, pk = carry_k;
+    for (uint32_t w = 0; w < warp; ++w) { ph = max(ph, s_h[w]); pk += s_k[w]; }
+    const uint32_t head_in = max(ph, eh);
+    uint32_t slot = pk + ek;
+    // survivors cluster (repeats): a thread may hold 64 of them, so their ids are read eight at a time, the loads in
+    // flight together -- one by one, each store waited for its load (57 us at C2, most of it in such threads)
+    do {
+        uint32_t e[8], id[8];
+        int cnt = 0;
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            e[q] = sv ? (uint32_t)__ffsll((long long)sv) - 1u : 0u;
+            if (sv) ++cnt;
+            sv &= sv - 1ull;
+        }
+#pragma unroll
+        for (int q = 0; q < 8; ++q) id[q] = q < cnt ? sidx[j0 + e[q]] : 0u;
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            if (q >= cnt) break;
+            const uint64_t hb = hm & (~0ull >> (63u - e[q]));                   // heads at or before element e
+            cpos[slot] = j0 + e[q];
+            cidx[slot] = id[q];
+            cgrp[slot] = hb ? j0 + 63u - (uint32_t)__clzll(hb) : head_in - 1u;
+            ++slot;
+        }
+    } while (sv);
+}
+
+void seg_compact0(const uint16_t *flags, const uint32_t *sidx, uint32_t m, const uint32_t *carry_head,
+                  const uint32_t *carry_keep, uint32_t *cpos, uint32_t *cidx, uint32_t *cgrp, cudaStream_t st)
+{
+    const uint32_t blocks = (uint32_t)(((uint64_t)m + C0_THREADS * C0_IPT - 1) / (C0_THREADS * C0_IPT));
+    if (blocks == 0) return;
+    seg_compact0_kernel<<<blocks, C0_THREADS, 0, st>>>(flags, sidx, m, carry_head, carry_keep, cpos, cidx, cgrp);
 }
 
 // ---------------------------------------------------------------- group-local refinement (no radix sort)
@@ -792,7 +910,7 @@ __device__ __forceinline__ int suffix_cmp_from(const uint8_t *__restrict__ text,
 }
 
 // One group of s <= GS_MAX elements starting at element j, ordered by ONE thread with symbol-by-symbol comparisons
-// (GS_DEPTH deep, end of text exact).  The general case; group_sort_kernel sends here only what its 16-byte windows
+// (GS_DEPTH deep, end of text exact).  The general case; group_sort_kernel sends here only what its 24-byte windows
 // cannot decide.
 template <bool WIDE>
 __device__ __forceinline__ void group_sort_serial(uint32_t *__restrict__ cidx, uint32_t j, uint32_t s, uint32_t g,
@@ -825,29 +943,38 @@ __device__ __forceinline__ void group_sort_serial(uint32_t *__restrict__ cidx, u
     }
 }
 
-// the 16 symbols at text[p .. p + 16) as two big-endian words (integer order = symbol order); three aligned 8-byte
-// loads, all inside [p - 7, p + 24)
-__device__ __forceinline__ void window16_be(const uint8_t *__restrict__ text, uint64_t p, uint64_t &hi, uint64_t &lo)
+// the 8 * WW symbols at text[p .. p + 8 WW) as WW big-endian words (integer order = symbol order); WW + 1 aligned
+// 8-byte loads, all inside [p - 7, p + 8 WW + 8)
+__device__ __forceinline__ uint64_t be64(uint64_t x)
+{
+    return ((uint64_t)__byte_perm((uint32_t)x, 0u, 0x0123) << 32) | __byte_perm((uint32_t)(x >> 32), 0u, 0x0123);
+}
+template <int WW>
+__device__ __forceinline__ void window_be(const uint8_t *__restrict__ text, uint64_t p, uint64_t w[WW])
 {
     const uintptr_t a = reinterpret_cast<uintptr_t>(text) + p;
-    const uint64_t *w = reinterpret_cast<const uint64_t *>(a & ~(uintptr_t)7);
+    const uint64_t *g = reinterpret_cast<const uint64_t *>(a & ~(uintptr_t)7);
     const uint32_t sh = (uint32_t)(a & 7u) * 8u;
-    const uint64_t w0 = __ldg(w), w1 = __ldg(w + 1), w2 = __ldg(w + 2);
-    const uint64_t x0 = sh ? (w0 >> sh) | (w1 << (64u - sh)) : w0;
-    const uint64_t x1 = sh ? (w1 >> sh) | (w2 << (64u - sh)) : w1;
-    hi = ((uint64_t)__byte_perm((uint32_t)x0, 0u, 0x0123) << 32) | __byte_perm((uint32_t)(x0 >> 32), 0u, 0x0123);
-    lo = ((uint64_t)__byte_perm((uint32_t)x1, 0u, 0x0123) << 32) | __byte_perm((uint32_t)(x1 >> 32), 0u, 0x0123);
+    uint64_t x[WW + 1];
+#pragma unroll
+    for (int q = 0; q <= WW; ++q) x[q] = __ldg(g + q);
+#pragma unroll
+    for (int q = 0; q < WW; ++q) w[q] = be64(sh ? (x[q] >> sh) | (x[q + 1] << (64u - sh)) : x[q]);
 }
 
 // One thread per ELEMENT (the one-thread-per-group form left two thirds of the lanes idle behind serial chains of
 // dependent random loads and kept its arrays in local memory: 164 M elements took 8 ms, the distributed build's group
 // round 13-44 ms).  A CTA takes 1008 elements + 16 of look-ahead: (1) group ids into shared memory, every element
 // finds its group's start and size by scanning at most 16 neighbours; a group of 2..16 elements belongs to the CTA
-// holding its first element, larger groups keep one key (g << 32); (2) every member loads its suffix id and the 16
-// symbols beyond the shared depth as two big-endian words -- two dependent random loads per element, all elements in
+// holding its first element, larger groups keep one key (g << 32); (2) every member loads its suffix id and the 8 WW
+// symbols beyond the shared depth as WW big-endian words -- two dependent random loads per element, all elements in
 // flight at once; (3) place in the group = members with a smaller window, key = (g << 32 | that count).  Groups with
-// two equal windows (ties deeper than 16 symbols) or a window reaching the end of the text go to
+// two equal windows (ties deeper than 8 WW symbols) or a window reaching the end of the text go to
 // group_sort_serial on the thread of their first element: the result is that of the serial form in every case.
+// WW = 2 (16 symbols) where the uniform depth is about what equal keys share (per-symbol keys: C3's 9 of ~10); WW = 3
+// for k-gram keys, which guarantee one gram but share ~3 (C2: 6 symbols guaranteed, 18-21 shared): with 16 symbols
+// nearly every group tied and went to the serial form (C2 group round 0.078 ms, 0.060 with 24; on C3, 24 symbols cost
+// more loads than they save: 14.33 -> 14.42 ms per build; B200, 1000 W).
 constexpr int GC_THREADS = 256;
 constexpr int GC_IPT = 4;
 constexpr int GC_SLOTS = GC_THREADS * GC_IPT;        // 1024 elements seen by a CTA
@@ -858,14 +985,14 @@ constexpr uint32_t GC_MARK = 0xFFFFFFFFu;            // low key word of a group'
 constexpr int GC_WORDS = (GC_SLOTS + 2 * GC_HALO) / 32;
 static_assert((GC_SLOTS + 2 * GC_HALO) % 32 == 0 && GC_HALO <= 32, "start bits are read one word back and one ahead");
 
-template <bool WIDE>
+template <bool WIDE, int WW>
 __global__ void __launch_bounds__(GC_THREADS, 6)
 group_sort_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp, uint32_t m,
                   const uint8_t *__restrict__ text, uint64_t n, uint64_t depth, const uint64_t *__restrict__ ids64,
                   uint64_t *__restrict__ keys)
 {
     __shared__ uint32_t s_grp[GC_SLOTS + 2 * GC_HALO];           // element base - GC_HALO + i
-    __shared__ uint64_t s_hi[GC_SLOTS], s_lo[GC_SLOTS];
+    __shared__ uint64_t s_w[WW][GC_SLOTS];                       // the window, most significant word first
     __shared__ uint32_t s_v[GC_SLOTS];
     __shared__ uint16_t s_meta[GC_SLOTS];                        // start slot (10 bits) | size - 1 (4 bits) | member (bit 15)
     __shared__ uint16_t s_x[WIDE ? GC_SLOTS : 1];                // WIDE: the key's extension bits out of the id word
@@ -916,7 +1043,7 @@ group_sort_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp
                     id = w & WIDE_ID_MASK;
                     s_x[slot] = (uint16_t)(w >> WIDE_ID_BITS);
                 }
-                s_lo[slot] = id + depth;                         // where this member's window starts (until the window itself lands here)
+                s_w[0][slot] = id + depth;                       // where this member's window starts (until the window itself lands here)
                 s_v[slot] = v;
                 meta = (uint16_t)(0x8000u | ((size - 1) << 10) | (uint32_t)start);
             }
@@ -924,7 +1051,7 @@ group_sort_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp
         s_meta[slot] = meta;
     }
     __syncthreads();
-    // the window: 16 symbols beyond the shared depth -- for 64-bit ids only where the extension bits of the key
+    // the window: 8 WW symbols beyond the shared depth -- for 64-bit ids only where the extension bits of the key
     // (16 more bits of the code stream, carried in the id word) do not already tell this member from all the others
 #pragma unroll 2
     for (int k = 0; k < GC_IPT; ++k) {
@@ -939,14 +1066,16 @@ group_sort_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp
                 need = false;
                 for (uint32_t i = 0; i < size; ++i) need |= (start + i != slot && s_x[start + i] == x);
             }
-            uint64_t hi = 0, lo = 0;
+            uint64_t w[WW];
+#pragma unroll
+            for (int q = 0; q < WW; ++q) w[q] = 0;
             if (need) {
-                const uint64_t p = s_lo[slot];
-                if (p >= 8 && p + 24 <= n) window16_be(text, p, hi, lo);
+                const uint64_t p = s_w[0][slot];
+                if (p >= 8 && p + 8 * (WW + 1) <= n) window_be<WW>(text, p, w);
                 else hard = 1;
             }
-            s_hi[slot] = hi;
-            s_lo[slot] = lo;
+#pragma unroll
+            for (int q = 0; q < WW; ++q) s_w[q][slot] = w[q];
         }
         s_hard[slot] = hard;
     }
@@ -960,16 +1089,23 @@ group_sort_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict__ cgrp
         place[k] = less[k] = 0;
         if (!(meta & 0x8000u)) continue;
         const uint32_t start = meta & 0x3FFu, size = ((meta >> 10) & 0xFu) + 1;
-        const uint64_t hi = s_hi[slot], lo = s_lo[slot];
+        uint64_t w[WW];
+#pragma unroll
+        for (int q = 0; q < WW; ++q) w[q] = s_w[q][slot];
         const uint32_t x = WIDE ? s_x[slot] : 0u;
         bool tie = false;
         for (uint32_t i = 0; i < size; ++i) {
             const uint32_t o = start + i;
             if (o == slot) continue;
-            const uint64_t oh = s_hi[o], ol = s_lo[o];
             const uint32_t ox = WIDE ? s_x[o] : 0u;
-            const bool eq = ox == x && oh == hi && ol == lo;
-            const bool lt = ox < x || (ox == x && (oh < hi || (oh == hi && ol < lo)));
+            // lexicographic over (extension bits, window words): the first word that differs decides
+            bool eq = ox == x, lt = ox < x;
+#pragma unroll
+            for (int q = 0; q < WW; ++q) {
+                const uint64_t ow = s_w[q][o];
+                lt |= eq && ow < w[q];
+                eq &= ow == w[q];
+            }
             tie |= eq;
             less[k] += lt;
             place[k] += lt || (eq && o < slot);
@@ -1015,16 +1151,17 @@ group_sort_marked_kernel(uint32_t *__restrict__ cidx, const uint32_t *__restrict
 }
 
 cudaError_t group_local_keys(uint32_t *cidx, const uint32_t *cgrp, uint32_t m, const uint8_t *text, uint64_t n,
-                             uint64_t depth, const uint64_t *ids64, uint64_t *keys, cudaStream_t st)
+                             uint64_t depth, bool gram_keys, const uint64_t *ids64, uint64_t *keys, cudaStream_t st)
 {
     if (m == 0) return cudaSuccess;
     const uint32_t blocks = (m + GC_STRIDE - 1) / GC_STRIDE;
     const uint32_t blocks2 = (m + 255) / 256;
     if (ids64) {
-        group_sort_kernel<true><<<blocks, GC_THREADS, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
+        group_sort_kernel<true, 2><<<blocks, GC_THREADS, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
         group_sort_marked_kernel<true><<<blocks2, 256, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
     } else {
-        group_sort_kernel<false><<<blocks, GC_THREADS, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
+        if (gram_keys) group_sort_kernel<false, 3><<<blocks, GC_THREADS, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
+        else group_sort_kernel<false, 2><<<blocks, GC_THREADS, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
         group_sort_marked_kernel<false><<<blocks2, 256, 0, st>>>(cidx, cgrp, m, text, n, depth, ids64, keys);
     }
     count_launch(2);
@@ -1328,11 +1465,16 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
             prof::Scope ps(st, prof::SEG_APPLY, m / 4 + (uint64_t)m_next * 20 +
                                                  ((round != 0 || scatter_all) ? (uint64_t)m * 12 : 0));
             // round 0 with lazy ranks writes no ranks at all: round 1 takes them from the look-up (group start =
-            // lower bound), and round 1's own scatter covers every survivor before round 2 reads the array
-            uint32_t *rank_out = (round == 0 && !scatter_all) ? nullptr : B.rank;
-            seg_apply_kernel<<<tiles, SEG_THREADS, 0, st>>>(B.flags, sidx, pos, m, B.agg_head, B.agg_keep, d_sa, rank_out,
-                                                           cpos, cidx, B.grp, round != 0, scatter_all, d_text, N,
-                                                           carry ? d_bwt : nullptr);
+            // lower bound), and round 1's own scatter covers every survivor before round 2 reads the array.  After
+            // the last round nothing reads the ranks.
+            if (round == 0 && !scatter_all) {
+                seg_compact0(B.flags, sidx, m, B.agg_head, B.agg_keep, cpos, cidx, B.grp, st);
+            } else {
+                seg_apply_kernel<<<tiles, SEG_THREADS, 0, st>>>(B.flags, sidx, pos, m, B.agg_head, B.agg_keep, d_sa,
+                                                               m_next == 0 ? nullptr : B.rank, cpos, cidx, B.grp,
+                                                               round != 0, scatter_all, d_text, N,
+                                                               carry ? d_bwt : nullptr);
+            }
             HK_LAUNCH_CHECK();
         }
         stats.alg_bytes += (uint64_t)m * 8 + m / 2 + (uint64_t)m_next * 20 + ((round != 0 || scatter_all) ? (uint64_t)m * 12 : 0);
@@ -1370,7 +1512,7 @@ static int sa_build_impl(const uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint
             // is ordered by comparing text beyond the k0 symbols its members share.  The depth does not advance
             // (large groups are untouched), every survivor gets its rank scattered by the refinement that follows.
             prof::Scope ps(st, prof::SA_KEYBUILD, (uint64_t)m * 48);
-            HK_CUDA(group_local_keys(vx, B.grp, m, d_text, n, std::min<uint64_t>(h, n), nullptr, kx, st));
+            HK_CUDA(group_local_keys(vx, B.grp, m, d_text, n, std::min<uint64_t>(h, n), gc.tab != nullptr, nullptr, kx, st));
             skey = kx; sidx = vx; vfree = vy;
             stats.round_elems[round] = m;
             stats.round_passes[round] = 0;                      // 0 passes = refined without a radix sort

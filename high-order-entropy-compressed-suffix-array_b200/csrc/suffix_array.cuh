@@ -369,9 +369,11 @@ private:
 constexpr int GS_MAX = 16;       // groups up to this size are ordered by one thread
 constexpr int GS_DEPTH = 64;     // symbols compared beyond the depth the group shares
 // keys[j] = (cgrp[j] << 32 | sub-group) with every group of at most GS_MAX elements reordered in place (cidx) by text
-// comparison from `depth` on; ids64 != nullptr: cidx holds ordinals into ids64 (WIDE_ID_MASK = suffix id, then the key extension bits)
+// comparison from `depth` on (gram_keys: the groups come from k-gram keys, whose members share far more than `depth`
+// symbols -- compared in wider windows); ids64 != nullptr: cidx holds ordinals into ids64 (WIDE_ID_MASK = suffix id,
+// then the key extension bits)
 cudaError_t group_local_keys(uint32_t *cidx, const uint32_t *cgrp, uint32_t m, const uint8_t *text, uint64_t n,
-                             uint64_t depth, const uint64_t *ids64, uint64_t *keys, cudaStream_t st);
+                             uint64_t depth, bool gram_keys, const uint64_t *ids64, uint64_t *keys, cudaStream_t st);
 
 // ---------------------------------------------------------------- segmented rank update (suffix_array.cu)
 // mask = the key bits that were sorted on; carried_out != nullptr: byte j = top byte of sorted key j
@@ -386,5 +388,8 @@ __global__ void __launch_bounds__(SEG_THREADS, 6) seg_apply_kernel(const uint16_
                                  uint32_t *__restrict__ sa, uint32_t *__restrict__ rank, uint32_t *__restrict__ cpos,
                                  uint32_t *__restrict__ cidx, uint32_t *__restrict__ cgrp, bool write_sa, bool scatter_all,
                                  const uint8_t *__restrict__ text, uint32_t n, uint8_t *__restrict__ bwt);
+// the same for round 0 without any rank scatter (pos = identity, nothing placed): the survivors only
+void seg_compact0(const uint16_t *flags, const uint32_t *sidx, uint32_t m, const uint32_t *carry_head,
+                  const uint32_t *carry_keep, uint32_t *cpos, uint32_t *cidx, uint32_t *cgrp, cudaStream_t st);
 
 }  // namespace hkcsa
